@@ -2,6 +2,7 @@
 """bench.py — env-steps/sec of the batched xLSTM recurrent inference step (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--model 48M] [--envs 64]
+                    [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] — "xLSTM 48M recurrent step, 64 synthetic Meta-World envs
 on 1xB200"; for N > 1 every rank runs the same 64 envs-per-GPU shard (weak scaling; env i -> rank i % N as
@@ -21,6 +22,12 @@ per step. A "step" is one env step of all envs: embed + 3 tokens x 12 blocks + h
                reference, online_decision_transformer_model.py:748-758)
   context_prefill  BASELINE.json configs[3] on the side (N = 1): 49 998-token chunkwise prefill of one 206M env, tokens/s
                and the bf16 MMA rate of the whole prefill against the sustained cuBLAS rate (tensor-pipe utilisation)
+
+--dump-outputs DIR: after the timed steps, writes what the last of them returned to its caller as DIR/<name>.npy
+(float32 / float64; the inputs are seeded, so two builds run with the same arguments can be compared file for file):
+action_tokens and action_preds of every env of this rank, and a fixed seeded sample (48 MiB at most) of the recurrent
+state every block carries into the next step, state_block<i>_<C|n|m|conv|slstm>.npy (C in the reference's
+[B, NH, DH, DH] layout, flattened).
 
 --impl reference: times the reference's CPU implementation of the path (the oracle port; the xlstm package is
 absent, see oracle/xlstm_oracle.py header) on the host cores for the same config/metric. Both CPU legs use ONE
@@ -174,10 +181,10 @@ def run_reference(args):
     sd = make_state_dict(cfg, seed=0)
     cores = os.cpu_count() or 1
     # bounded sample (the same definition as the b200 arm's cpu_baseline): cpu_sample(envs) envs, every step one env
-    # step of those envs; K steps unless the time budget (~4 min) ends the run earlier
+    # step of those envs; exactly K timed steps
     b_ref = cpu_sample(args.envs)
     kw = dict(domains=args.domains, discrete=args.discrete)
-    value, ms, timed = time_oracle(cfg, sd, b_ref, args.steps, args.warmup, cores, budget_s=240, **kw)
+    value, ms, timed = time_oracle(cfg, sd, b_ref, args.steps, args.warmup, cores, **kw)
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
         "steps": timed, "warmup": args.warmup, "ms_per_step": statistics.mean(ms), "higher_is_better": True,
@@ -241,6 +248,32 @@ def prefill_leg(peaks, model="206M", tokens=49998, reps=2):
                                "over the WHOLE prefill time, non-GEMM kernels included; peak = sustained cuBLAS bf16"}}
 
 
+DUMP_STATE_BYTES = 48 * 2 ** 20
+
+
+def snapshot_outputs(cfg, out, cache) -> dict:
+    """Device copies of what a policy step returned to its caller (see --dump-outputs), keyed by file name. They stay
+    on the device so that the copy to the host can wait until the clock-sampling window has closed."""
+    from lram_b200 import _lib as L
+    arrays = {"action_tokens": out["action_tokens"].double(),                     # int32 values, exact in float64
+              "action_preds": out["action_preds"].float().clone()}
+    parts = []
+    for i in range(cfg.num_blocks):
+        if cfg.is_slstm(i):
+            parts += [(i, "slstm", L.XL_STATE_SLSTM), (i, "conv", L.XL_STATE_CONV)]
+        else:
+            parts += [(i, "C", None), (i, "n", L.XL_STATE_N), (i, "m", L.XL_STATE_M), (i, "conv", L.XL_STATE_CONV)]
+    cap = DUMP_STATE_BYTES // 4 // len(parts)
+    g = torch.Generator().manual_seed(0)
+    for i, name, part in parts:
+        t = (cache.c_logical(i) if part is None else cache.view(i, part)).reshape(-1)
+        if t.numel() > cap:
+            idx = torch.randint(t.numel(), (cap,), generator=g).sort().values
+            t = t[idx.to(t.device)]
+        arrays[f"state_block{i:02d}_{name}"] = t.float().clone()
+    return arrays
+
+
 def _quiet_stdout():
     """The contract is ONE JSON line on stdout. Libraries write there too (NCCL prints its version banner from C), so
     fd 1 is pointed at stderr for the whole run and the JSON line goes to a duplicate of the original stdout."""
@@ -282,11 +315,15 @@ def main():
                     help="N > 1: all-gather the action tokens of this many env steps in one collective (1 = per step)")
     ap.add_argument("--opt", action="append", default=[], metavar="NAME=VALUE",
                     help="xl_set_option passthrough for A/B runs, e.g. --opt microbatches=1 --opt state_impl=1")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs and a seeded sample of the state as DIR/<name>.npy")
     args = ap.parse_args()
     _quiet_stdout()
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes what the CUDA path computed: not available with --impl reference")
         run_reference(args)
         return
 
@@ -379,6 +416,7 @@ def main():
         tt = torch.tensor([ms_total], device=dev)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         ms_total = tt.item()
+    dumped = snapshot_outputs(cfg, out, cache) if args.dump_outputs and rank == 0 else None
     # A timed region shorter than ~1 s can fall between two nvidia-smi samples: keep the SAME steps running (untimed,
     # same count on every rank: derived from the all-reduced time) until the window under load is ~1.2 s long.
     extra = 0
@@ -559,6 +597,10 @@ def main():
             "gpu_eager_baseline": gpu_eager,
             "context_prefill": prefill,
         }
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumped.items():
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a.cpu().numpy())
         _emit(line)
     eng.close()
     if world > 1:

@@ -284,7 +284,7 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
             .past_key_values, .last_hidden_state — only the LAST timestep is consumed, exactly as
             `compute_inputs` does when the cache is warm (online_decision_transformer_model.py:466-470); on the cold
             first call the reference embeds all T but `handle_inference_cache` trims to the last 3 tokens
-            (decision_xlstm.py:225-229), i.e. to the last timestep as well (pinned by tests/golden/ref_policy_forward.npz).
+            (decision_xlstm.py:225-229), i.e. to the last timestep as well (pinned by tests/golden/ref_policy_forward/).
 
     `state_dict` may be given at construction (then it is loaded straight away) or later through `load_state_dict`,
     the order the reference's agent uses; hot-path keys missing at the first call raise KeyError.

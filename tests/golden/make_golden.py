@@ -3,7 +3,7 @@
     python tests/golden/make_golden.py
 
 Sources of truth:
-  tokenizer_kat.npz   — produced by the REFERENCE'S OWN code imported from /root/reference
+  tokenizer_kat.npz   — produced by the REFERENCE'S OWN code imported from the LRAM_REFERENCE_ROOT checkout
                         (`src/tokenizers_custom/{minmax,mu_law}_tokenizer.py`; they need only torch/numpy).
   hf_mlstm_step.npz   — produced by ``transformers.models.xlstm.modeling_xlstm.mlstm_recurrent_step_native``
                         (transformers 5.5.0 in this image): an independent implementation of the mLSTM
@@ -12,9 +12,9 @@ Sources of truth:
   hf_mlstm_chunkwise.npz — ``mlstm_chunkwise_fw`` (48 tokens, chunk 16, non-zero initial (C, n, m)) and
                         ``xLSTMMultiHeadLayerNorm`` from the same transformers module.
   oracle_toy.npz      — produced by oracle/xlstm_oracle.py itself (regression pin + the vectors the GPU
-                        parity tests re-check on the box, where /root/reference does not exist).
+                        parity tests re-check on the GPU, where no reference checkout is needed).
 
-Nothing at test/bench time reads /root/reference; only this script does.
+Nothing at test/bench time reads the reference checkout; only this script does.
 """
 import importlib.util
 import os
@@ -30,7 +30,10 @@ sys.path.insert(0, ROOT)
 
 
 def _load_reference_tokenizers():
-    base = "/root/reference/src/tokenizers_custom"
+    import ref_stubs
+    if not ref_stubs.reference_available():
+        raise RuntimeError(ref_stubs.SKIP_REASON)
+    base = os.path.join(ref_stubs.REFERENCE_ROOT, "src", "tokenizers_custom")
     pkg = types.ModuleType("ref_tok")
     pkg.__path__ = [base]
     sys.modules["ref_tok"] = pkg

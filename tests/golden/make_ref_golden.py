@@ -2,7 +2,7 @@
 
     python tests/golden/make_ref_golden.py
 
-What runs (unmodified, imported from /root/reference through tests/golden/ref_stubs.py):
+What runs (unmodified, imported from the LRAM_REFERENCE_ROOT checkout through tests/golden/ref_stubs.py):
   * `MultiDomainDiscreteDecisionXLSTMModel.__init__` / `.forward(use_inference_cache=True)`
     (src/algos/models/decision_xlstm.py:175-289, online_decision_transformer_model.py:326-530,588-612,
     discrete_decision_transformer_model.py:236-383, multi_domain_discrete_dt_model.py:12-108),
@@ -20,7 +20,7 @@ Weights: `lram_b200.synth.make_state_dict(cfg, seed)` loaded into the reference 
 (strict=False; the keys it leaves at their init are asserted to be off the hot path). Tests rebuild the same weights from
 the seed, so the fixtures hold inputs' seeds and outputs only.
 
-Files written (tests/golden/): ref_policy_forward.npz, ref_rollout.npz
+Files written (tests/golden/): ref_policy_forward/<case>.npz (one file per case keeps each under 1 MB), ref_rollout.npz
 """
 import os
 import sys
@@ -217,7 +217,11 @@ def main():
     policy_forward_case(fwd, "48M_cont", "48M", seed=16, B=2, n_steps=3, discrete=False, domains="metaworld")
     policy_forward_case(fwd, "110M_disc", "110M", seed=17, B=2, n_steps=3, discrete=True, domains="mixed")
     policy_forward_case(fwd, "206M_cont", "206M", seed=18, B=1, n_steps=2, discrete=False, domains="mimicgen")
-    np.savez_compressed(os.path.join(HERE, "ref_policy_forward.npz"), **fwd)
+    os.makedirs(os.path.join(HERE, "ref_policy_forward"), exist_ok=True)
+    for tag in dict.fromkeys(k.split(".")[0] for k in fwd):
+        f = os.path.join(HERE, "ref_policy_forward", f"{tag}.npz")
+        np.savez_compressed(f, **{k: v for k, v in fwd.items() if k.split(".")[0] == tag})
+        print(os.path.relpath(f, HERE), os.path.getsize(f), "bytes")
     ro = {}
     rollout_case(ro, "toy128_metaworld", "toy128", seed=21, kind="metaworld", n_episodes=3, ep_len=7)
     rollout_case(ro, "toy128_atari", "toy128", seed=22, kind="atari", n_episodes=2, ep_len=5)
@@ -226,8 +230,7 @@ def main():
     rollout_case(ro, "toy128_resetfreq", "toy128", seed=25, kind="metaworld", n_episodes=2, ep_len=9,
                  reset_inf_cache_freq=4)
     np.savez_compressed(os.path.join(HERE, "ref_rollout.npz"), **ro)
-    for f in ("ref_policy_forward.npz", "ref_rollout.npz"):
-        print(f, os.path.getsize(os.path.join(HERE, f)), "bytes")
+    print("ref_rollout.npz", os.path.getsize(os.path.join(HERE, "ref_rollout.npz")), "bytes")
 
 
 if __name__ == "__main__":

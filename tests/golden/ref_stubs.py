@@ -1,7 +1,7 @@
 """Stand-ins for the reference's absent dependencies, so that ITS OWN hot-path code runs unmodified in this container.
 
-Test infrastructure only. /root/reference (read-only) imports `gym`, `stable_baselines3`, `omegaconf`, `dacite`,
-`torchmetrics`, `h5py` and the third-party `xlstm`; none is installed and none can be fetched. `install()`:
+Test infrastructure only. The reference (a read-only checkout of ml-jku/LRAM, named by LRAM_REFERENCE_ROOT) imports
+`gym`, `stable_baselines3`, `omegaconf`, `dacite`, `torchmetrics`, `h5py` and the third-party `xlstm`; none is installed and none can be fetched. `install()`:
   * registers small functional stubs for the handful of symbols the path really executes (gym spaces, SB3's
     `is_image_space` / `get_obs_shape` / `get_action_dim` / `BaseFeaturesExtractor`, `OmegaConf.to_container`,
     `dacite.from_dict`),
@@ -13,8 +13,8 @@ After that `from src.algos.models.decision_xlstm import MultiDomainDiscreteDecis
 `from src.algos.decision_xlstm import DiscreteDecisionXLSTM` and
 `from src.callbacks.evaluation import custom_evaluate_policy` are the reference's real code.
 
-Used by tests/golden/make_ref_golden.py (fixture generator) and by CPU tests that skip when /root/reference is absent
-(it does not exist on the GPU box).
+Used by tests/golden/make_ref_golden.py (fixture generator) and by CPU tests that skip unless LRAM_REFERENCE_ROOT
+names such a checkout (the reference is not part of this repository).
 """
 from __future__ import annotations
 
@@ -30,7 +30,8 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-REFERENCE_ROOT = os.environ.get("LRAM_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("LRAM_REFERENCE_ROOT", "")
+SKIP_REASON = "needs a checkout of the reference (ml-jku/LRAM): set LRAM_REFERENCE_ROOT"
 
 # third-party packages that are absent here
 _STUB_TOPLEVEL = ("gym", "stable_baselines3", "omegaconf", "dacite", "torchmetrics", "h5py", "xlstm", "wandb_stub")
@@ -45,7 +46,7 @@ _REAL_SRC = ("src.buffers.buffer_utils", "src.envs.env_utils")
 
 
 def reference_available() -> bool:
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "src", "algos", "models"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "src", "algos", "models"))
 
 
 class _AutoStub(types.ModuleType):
@@ -182,12 +183,12 @@ _installed = False
 
 
 def install() -> None:
-    """Idempotent. Puts the stubs in sys.modules / sys.meta_path and /root/reference on sys.path."""
+    """Idempotent. Puts the stubs in sys.modules / sys.meta_path and the reference checkout on sys.path."""
     global _installed
     if _installed:
         return
     if not reference_available():
-        raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT}")
+        raise RuntimeError(f"reference tree not found at LRAM_REFERENCE_ROOT={REFERENCE_ROOT!r}")
     repo_root = os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
     for p in (repo_root, REFERENCE_ROOT):
         if p not in sys.path:

@@ -152,10 +152,53 @@ def test_bench_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert len(lines) == 1, p.stdout
     d = json.loads(lines[0])
     assert d["impl"] == "reference" and d["unit"] == "env-steps/s" and d["higher_is_better"] is True
-    assert d["value"] > 0 and d["n_gpus"] == 1 and d["gpu_launches"] == 0
+    assert d["value"] > 0 and d["n_gpus"] == 1 and d["gpu_launches"] == 0 and d["steps"] == 2
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["config"]["workload"] and "model" in d["config"]
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs_equal_an_independent_run(tmp_path):
+    """`bench.py --dump-outputs DIR` on a toy workload writes exactly what an engine stepped warmup + steps times over the
+    same seeded stream holds after its last step (float32 / float64, under 64 MB), and one more step changes it."""
+    import json
+    import bench
+    from lram_b200.engine import XLSTMEngine
+    W, K, B = 3, 5, 4
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--model", "toy128", "--envs", str(B),
+                        "--steps", str(K), "--warmup", str(W), "--no-cpu-baseline", "--profile-steps", "0",
+                        "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    assert json.loads(p.stdout.strip().splitlines()[-1])["steps"] == K
+    got = {f.stem: np.load(f) for f in sorted(tmp_path.glob("*.npy"))}
+    assert all(v.dtype in (np.float32, np.float64) for v in got.values())
+    assert sum(v.nbytes for v in got.values()) <= 64 * 2 ** 20
+
+    cfg = preset("toy128")
+    states, rtg, _ = make_stream(cfg, range(B), W + K, domains="metaworld")
+    eng = XLSTMEngine(cfg, make_state_dict(cfg, seed=0), max_batch=B)
+    cache = eng.new_state(B)
+    s_in, r_in = torch.empty(B, cfg.state_dim, device="cuda"), torch.empty(B, device="cuda")
+    out = {"action_tokens": torch.zeros(B, cfg.act_dim, dtype=torch.int32, device="cuda"),
+           "action_preds": torch.zeros(B, cfg.act_dim, dtype=torch.float32, device="cuda")}
+
+    def step(t):
+        s_in.copy_(torch.from_numpy(states[t % (W + K)]))
+        r_in.copy_(torch.from_numpy(rtg[t % (W + K)]))
+        eng.policy_step(cache, s_in, r_in, mode=L.XL_MODE_FUSED, flags=L.XL_FLAG_GRAPH, out=out)
+
+    for t in range(W + K):
+        step(t)
+    want = {k: v.cpu().numpy() for k, v in bench.snapshot_outputs(cfg, out, cache).items()}
+    assert got.keys() == want.keys() and {"action_tokens", "action_preds", "state_block00_C"} <= set(got)
+    for k in want:
+        assert np.array_equal(got[k], want[k]), k
+    assert got["action_tokens"].any() and got["state_block00_C"].any()
+    step(W + K)
+    later = bench.snapshot_outputs(cfg, out, cache)
+    assert not np.array_equal(got["state_block00_C"], later["state_block00_C"].cpu().numpy())
+    eng.close()
 
 
 def test_every_option_of_the_library_is_documented_in_the_header():

@@ -189,9 +189,11 @@ def test_reset_rows_equals_none_state():
         pkv = pol.step(torch.from_numpy(states[t]), torch.from_numpy(rtg[t]), past_key_values=pkv)["past_key_values"]
     mask = torch.tensor([False, True, False])
     o = pol.step(torch.from_numpy(states[2]), torch.from_numpy(rtg[2]), past_key_values=O.reset_state_rows(pkv, mask))
-    fresh = pol.step(torch.from_numpy(states[2, 1:2]), torch.from_numpy(rtg[2, 1:2]), past_key_values=None)
-    assert torch.equal(o["action_tokens"][1], fresh["action_tokens"][0])
-    assert (o["last_hidden_state"][1] - fresh["last_hidden_state"][0]).abs().max() < 1e-6
+    # a fresh batch of the same size: CPU BLAS picks its GEMM kernels by shape and host ISA, so a batch of another size
+    # may round differently (batch-size independence is test_batched_equals_single_env's pin)
+    fresh = pol.step(torch.from_numpy(states[2]), torch.from_numpy(rtg[2]), past_key_values=None)
+    assert torch.equal(o["action_tokens"][1], fresh["action_tokens"][1])
+    assert (o["last_hidden_state"][1] - fresh["last_hidden_state"][1]).abs().max() < 1e-6
 
 
 def test_discrete_head_branch():

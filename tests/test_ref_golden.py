@@ -1,11 +1,11 @@
 """Parity against vectors produced by the REFERENCE'S OWN model / agent / rollout code
-(tests/golden/ref_policy_forward.npz, ref_rollout.npz; generator tests/golden/make_ref_golden.py runs
-/root/reference's `MultiDomainDiscreteDecisionXLSTMModel.forward`, `DiscreteDecisionXLSTM.predict` and
+(tests/golden/ref_policy_forward/<case>.npz, ref_rollout.npz; generator tests/golden/make_ref_golden.py runs the
+reference's `MultiDomainDiscreteDecisionXLSTMModel.forward`, `DiscreteDecisionXLSTM.predict` and
 `custom_evaluate_policy` through stub packages, with the absent `xlstm` package stood in by oracle/xlstm_shim.py).
 
 CPU (`-m "not gpu"`): the oracle's LRAM-side restatement (embed, token layout, cache trim, head slice, argmax,
-inv_tokenize, rollout bookkeeping) == the reference's code; and, when /root/reference is present, the fixtures
-regenerate bit-identically from the reference.
+inv_tokenize, rollout bookkeeping) == the reference's code; and, when LRAM_REFERENCE_ROOT points at a checkout of the
+reference, the fixtures regenerate bit-identically from it.
 GPU (`-m gpu`): the CUDA path through the host mirror == the reference's outputs: action tokens / argmax actions
 bit-exact, hidden states / logits / recurrent state within REL_TOL = 1e-3 (north_star's tolerance).
 """
@@ -33,7 +33,12 @@ gpu = pytest.mark.gpu
 
 @pytest.fixture(scope="module")
 def fwd(golden_dir):
-    return np.load(os.path.join(golden_dir, "ref_policy_forward.npz"))
+    d = os.path.join(golden_dir, "ref_policy_forward")
+    out = {}
+    for tag in FWD_TAGS:
+        with np.load(os.path.join(d, f"{tag}.npz")) as z:
+            out.update({k: z[k] for k in z.files})
+    return out
 
 
 @pytest.fixture(scope="module")
@@ -144,11 +149,11 @@ def _ref_stubs():
 
 
 def test_fixtures_regenerate_from_the_reference(fwd, rollouts):
-    """Only where /root/reference exists (the build container): the committed fixtures are what the reference's own
+    """Only with a checkout of the reference (LRAM_REFERENCE_ROOT): the committed fixtures are what the reference's own
     code produces today."""
     ref_stubs = _ref_stubs()
     if not ref_stubs.reference_available():
-        pytest.skip("reference tree not present (GPU box)")
+        pytest.skip(ref_stubs.SKIP_REASON)
     import make_ref_golden as G
     out = {}
     G.policy_forward_case(out, "toy128_cont", "toy128", seed=11, B=5, n_steps=6, discrete=False)
