@@ -177,6 +177,52 @@ int xl_state_reset(xl_handle* h, void* state, const uint8_t* env_mask, int B, vo
  * `stream`); a different ring drops the cached graphs. B must stay the same between arming and gathering. */
 int xl_set_token_ring(xl_handle* h, int32_t* ring, int slots, int next_slot, void* stream);
 
+/* Stochastic action selection on the device: the reference's `a_sample_kwargs` (sample_from_logits,
+ * src/algos/models/model_utils.py:7-32, called once per env at discrete_decision_transformer_sb3.py:62-63) with a
+ * counter-based random stream. While armed, every xl_policy_step* picks its tokens by this contract instead of the
+ * argmax; steps that xl_policy_prefill runs internally still take the argmax and do not count as steps here.
+ *
+ * For env b and action row j, take the row l[0..n) of logits, n = num_actions (discrete: the env's logits; continuous:
+ * row j of its [act_dim, num_actions] block). In fp64:
+ *  1. top_p > 0: percentile = torch.quantile(l, top_p): rank = (double)top_p * (n - 1), lo = floor(rank),
+ *     hi = ceil(rank), w = rank - lo, with v = sorted(l): w < 0.5 ? v[lo] + w (v[hi] - v[lo])
+ *     : v[hi] - (v[hi] - v[lo]) (1 - w). If percentile != max for EVERY row of the env, max taken over the env's
+ *     whole logit block (a NaN anywhere in the block makes it NaN), every l_i <= percentile becomes -inf.
+ *  2. top_k > 0: the k largest of the resulting row stay candidates, ties at the boundary to the lowest indices;
+ *     -inf positions among them have weight 0.
+ *  3. w_i = exp(temperature * (l_i - l_max)) over the candidates, Z = sum w_i (index order). u in [0, 1) from
+ *     Philox4x32-10 with counter (step, global_env_id, j, 0) and key (seed & 0xffffffff, seed >> 32):
+ *     u = ((x0 >> 5) * 2^26 + (x1 >> 6)) * 2^-53. The token is the first candidate, in index order, whose running sum
+ *     exceeds u * Z.
+ *  4. global_env_id = env_id_base + b * env_id_stride (b counts the envs of the call). With envs sharded as
+ *     env i -> rank i mod N, base = rank and stride = N give every env the draws it gets on one GPU running all envs.
+ *  5. step: a device counter, set to step0 here and advanced once per policy step on the device (inside a captured
+ *     graph too); a step draws with the value it finds, so the first step after arming uses step0.
+ *  6. A row containing NaN, or with no finite maximum among its candidates (everything cut, all -inf, or +inf), yields
+ *     the argmax token (first index of the max of the first discrete_actions logits when discrete, of all num_actions
+ *     otherwise; NaN counts as the max), where the reference would raise.
+ * tokens / actions / token ring then hold the sampled tokens exactly as they hold the argmax ones (discrete: actions =
+ * (float)token; continuous: max(token - discrete_actions, 0) * bin_width + min_val).
+ * Rejected with XL_ERR_INVALID_ARG: temperature <= 0 or not finite, top_p outside [0, 1], top_k < 0 or > num_actions,
+ * env_id_base < 0, env_id_stride < 1; XL_ERR_UNSUPPORTED: num_actions > 512 or act_dim > 8. */
+typedef struct {
+  float temperature;     /* 1.0 (the reference multiplies the logits by it)  */
+  float top_p;           /* 0.5; 0 = no quantile cut                          */
+  int32_t top_k;         /* 0 = no top-k cut                                  */
+  int32_t env_id_base;   /* global id of the call's env 0                     */
+  int32_t env_id_stride; /* global id step between consecutive envs           */
+  uint64_t seed;
+} xl_sampling;
+/* params == NULL disarms: steps go back to the argmax. step0 = counter value of the next step. The parameters and the
+ * counter are written on `stream` into the handle's device memory, so changing them needs no graph re-capture; arming
+ * or disarming changes the step's kernels and drops the cached graphs. */
+int xl_set_sampling(xl_handle* h, const xl_sampling* params, uint32_t step0, void* stream);
+/* Unit-parity entry: sample B rows of given logits (discrete: [B, num_actions]; continuous: [B, act_dim*num_actions])
+ * at an explicit step; tokens [B, act_dim] / actions [B, act_dim] as xl_policy_step writes them. Leaves the armed
+ * sampler and its counter alone. */
+int xl_sample_actions(xl_handle* h, const float* logits, int B, unsigned flags, const xl_sampling* params,
+                      uint32_t step, int32_t* tokens, float* actions, void* stream);
+
 /* xLSTMEncoder.forward(inputs_embeds=x_in, past_key_values=state, use_cache=True)
  * (src/algos/models/decision_xlstm.py:138-169) == T x xLSTMBlockStack.step + post_blocks_norm.
  * x_in, x_out: fp32 [B, T, d] (may alias). State updated in place. 1 <= T <= 4. */
@@ -202,7 +248,8 @@ int xl_mlstm_cell_step(xl_handle* h, float* C, float* n, float* m, const float* 
  *                                or fp32 [B, d] state embeddings with XL_FLAG_STATE_EMBEDS
  *   rtg     fp32 [B]             returns-to-go of this timestep
  *   rewards fp32 [B] or NULL     reward token input; NULL = 0 (what the reference feeds, evaluation.py:132)
- *   tokens  int32 [B, act_dim]   argmax action tokens (continuous) / [B] first column (discrete)
+ *   tokens  int32 [B, act_dim]   argmax (or, armed, sampled: xl_set_sampling) action tokens (continuous) / first
+ *                                column (discrete)
  *   actions fp32 [B, act_dim]    inv_tokenized actions (continuous) / token as float (discrete)
  *   logits  fp32 [B, act_dim*num_actions] or NULL;  hidden fp32 [B, T, d] or NULL (last_hidden_state) */
 int xl_policy_step(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,

@@ -49,6 +49,12 @@ class XLConfig(C.Structure):
     ]
 
 
+class XLSampling(C.Structure):
+    """xl_sampling: parameters of the device sampler (xl_set_sampling)."""
+    _fields_ = [("temperature", C.c_float), ("top_p", C.c_float), ("top_k", C.c_int32), ("env_id_base", C.c_int32),
+                ("env_id_stride", C.c_int32), ("seed", C.c_uint64)]
+
+
 class XLError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"xlstm_b200 error {code}: {msg}")
@@ -115,6 +121,10 @@ def load():
     lib.xl_linear.restype = i32
     lib.xl_set_token_ring.argtypes = [vp, vp, i32, i32, vp]
     lib.xl_set_token_ring.restype = i32
+    lib.xl_set_sampling.argtypes = [vp, C.POINTER(XLSampling), u32, vp]
+    lib.xl_set_sampling.restype = i32
+    lib.xl_sample_actions.argtypes = [vp, vp, i32, u32, C.POINTER(XLSampling), u32, vp, vp, vp]
+    lib.xl_sample_actions.restype = i32
     lib.xl_set_option.argtypes = [vp, C.c_char_p, i32]
     lib.xl_set_option.restype = i32
     lib.xl_profile_begin.argtypes = [vp]

@@ -5,6 +5,7 @@
 #include <cuda_runtime.h>
 
 #include <algorithm>
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
@@ -54,6 +55,9 @@ struct GraphCacheEntry {
 
 }  // namespace
 
+// words of the handle's counters area: [0] token ring step, [1] sampler step, [2] step word of xl_sample_actions;
+// xl_sampling copies (32 B, 8-B aligned) of the armed sampler and of xl_sample_actions at kCntArmed / kCntUnit
+constexpr int kCntRing = 0, kCntSample = 1, kCntUnitStep = 2, kCntArmed = 8, kCntUnit = 16;
 constexpr int kMaxMicro = 8;   // env micro-batches pipelined on side streams
 constexpr int kSplitMax = 8;   // split-K planes of the skinny projections
 constexpr size_t kSplitRows = 1024;   // split-K only pays (and has plane storage) up to this many rows
@@ -153,6 +157,9 @@ struct xl_handle {
   std::vector<std::pair<const void*, void*>> host_map;   // host pointer -> device alias (nullptr: not mapped)
   int32_t* tok_ring = nullptr;
   int tok_slots = 0;
+  // sampler (xl_set_sampling): while armed, policy_back launches the sampling kernel instead of the argmax one; its
+  // parameters and step counter live in the counters area (kCnt* below), written on the caller's stream
+  bool sampling = false;
   bool profiling = false;
   std::vector<cudaEvent_t> prof_state;  // start/stop pairs around state-step launches
   std::vector<cudaEvent_t> prof_step;   // start/stop pairs around policy steps
@@ -657,7 +664,8 @@ int run_encoder(xl_handle* h, void* state, const Slice& sl, const float* x_in, f
 constexpr unsigned kFlagLn0Done = 1u << 29;     // internal: the embed kernel already ran block 0's pre-norm (operands in place)
 constexpr unsigned kFlagHeadOnly = 1u << 28;    // internal: nobody reads the hidden states: post_blocks_norm only on the
                                                 // action-token rows, fused with the head's operand split (policy_back)
-constexpr unsigned kFlagNoRing = 1u << 30;      // internal: steps run on behalf of xl_policy_prefill leave the token ring alone
+constexpr unsigned kFlagNoRing = 1u << 30;      // internal: steps run on behalf of xl_policy_prefill leave the token ring
+                                                // and the sampler alone (argmax, no step counted)
 
 // Arguments of one policy step (device pointers for the WHOLE batch of B envs).
 struct StepArgs {
@@ -706,7 +714,8 @@ int policy_front(xl_handle* h, const StepArgs& a, const Slice& sl, float* xt) {
                           (const float*)PW(XL_W_EMBED_RETURN_W), (const float*)PW(XL_W_EMBED_RETURN_B),
                           (const float*)PW(XL_W_EMBED_REWARD_W), (const float*)PW(XL_W_EMBED_REWARD_B),
                           (const float*)PW(XL_W_EMBED_LN_W), (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, xt,
-                          sl.Bk, d, (h->tok_ring && sl.b0 == 0 && !(a.flags & kFlagNoRing)) ? h->counters : nullptr,
+                          sl.Bk, d, (h->tok_ring && sl.b0 == 0 && !(a.flags & kFlagNoRing)) ? h->counters + kCntRing : nullptr,
+                          (h->sampling && sl.b0 == 0 && !(a.flags & kFlagNoRing)) ? h->counters + kCntSample : nullptr,
                           ln0_w, c.ln_eps, xn0, hi0, lo0, sl.s);
   h->launches += 1;
   return XL_OK;
@@ -744,6 +753,8 @@ int policy_back(xl_handle* h, const StepArgs& a, const Slice& sl, const float* h
   int rc;
   int32_t* ring = (h->tok_ring && !(a.flags & kFlagNoRing)) ? h->tok_ring + (size_t)sl.b0 * c.act_dim : nullptr;
   const int64_t ring_stride = (int64_t)a.B * c.act_dim;
+  const bool sample = h->sampling && !(a.flags & kFlagNoRing);
+  const float bw = (c.tok_max_val - c.tok_min_val) / (float)c.action_channels;
   if (discrete) {
     rc = linear(h, ws, xa, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, ws.logits, Bk, n_out, d, impl, s,
                 head_only);
@@ -751,15 +762,24 @@ int policy_back(xl_handle* h, const StepArgs& a, const Slice& sl, const float* h
     if (logits) {
       XL_CUDA(cudaMemcpyAsync(logits, ws.logits, sizeof(float) * (size_t)Bk * n_out, cudaMemcpyDeviceToDevice, s));
     }
-    xl::launch_argmax_tokens(ws.logits, n_out, Bk, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, tokens,
-                             actions, ring, h->counters, h->tok_slots, ring_stride, s);
+    if (sample)
+      xl::launch_sample_tokens(ws.logits, n_out, Bk, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, tokens, actions,
+                               ring, h->counters + kCntRing, h->tok_slots, ring_stride, h->counters + kCntArmed,
+                               h->counters + kCntSample, sl.b0, s);
+    else
+      xl::launch_argmax_tokens(ws.logits, n_out, Bk, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, tokens,
+                               actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride, s);
   } else {
     float* lg = logits ? logits : ws.logits;
     rc = linear(h, ws, xa, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, lg, Bk, n_out, d, impl, s, head_only);
     if (rc) return rc;
-    const float bw = (c.tok_max_val - c.tok_min_val) / (float)c.action_channels;
-    xl::launch_argmax_tokens(lg, h->head_out, Bk, c.act_dim, h->num_actions, c.discrete_actions, 0, bw,
-                             c.tok_min_val, tokens, actions, ring, h->counters, h->tok_slots, ring_stride, s);
+    if (sample)
+      xl::launch_sample_tokens(lg, h->head_out, Bk, c.act_dim, h->num_actions, c.discrete_actions, 0, bw, c.tok_min_val,
+                               tokens, actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride,
+                               h->counters + kCntArmed, h->counters + kCntSample, sl.b0, s);
+    else
+      xl::launch_argmax_tokens(lg, h->head_out, Bk, c.act_dim, h->num_actions, c.discrete_actions, 0, bw,
+                               c.tok_min_val, tokens, actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride, s);
   }
   h->launches += 1;
   return XL_OK;
@@ -1638,8 +1658,8 @@ int xl_policy_prefill(xl_handle* h, void* state, const float* states, const floa
       xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
                               (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
                               (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
-                              (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, 0.f,
-                              nullptr, nullptr, nullptr, s);
+                              (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
+                              0.f, nullptr, nullptr, nullptr, s);
       h->launches += 1;
       rc = prefill_blocks(h, state, B, Tc * T, flags, s);
       if (rc) return rc;
@@ -1687,9 +1707,66 @@ int xl_set_token_ring(xl_handle* h, int32_t* ring, int slots, int next_slot, voi
     h->tok_slots = ring ? slots : 0;
   }
   if (ring) {
-    xl::launch_set_u32(h->counters, (unsigned)next_slot, (cudaStream_t)stream);
+    xl::launch_set_u32(h->counters + kCntRing, (unsigned)next_slot, (cudaStream_t)stream);
     XL_CUDA(cudaGetLastError());
   }
+  return XL_OK;
+}
+
+static int check_sampling(const xl_handle* h, const xl_sampling* p) {
+  if (!(p->temperature > 0.f) || !std::isfinite(p->temperature))
+    return fail(XL_ERR_INVALID_ARG, "sampling: temperature %g must be finite and > 0", (double)p->temperature);
+  if (!(p->top_p >= 0.f && p->top_p <= 1.f)) return fail(XL_ERR_INVALID_ARG, "sampling: top_p %g outside [0, 1]", (double)p->top_p);
+  if (p->top_k < 0 || p->top_k > h->num_actions)
+    return fail(XL_ERR_INVALID_ARG, "sampling: top_k %d outside [0, num_actions=%d]", p->top_k, h->num_actions);
+  if (p->env_id_base < 0 || p->env_id_stride < 1)
+    return fail(XL_ERR_INVALID_ARG, "sampling: env_id_base %d must be >= 0 and env_id_stride %d >= 1", p->env_id_base,
+                p->env_id_stride);
+  if (h->num_actions > xl::kSampleMaxActions || h->cfg.act_dim > xl::kSampleMaxRows)
+    return fail(XL_ERR_UNSUPPORTED, "sampling: num_actions %d > %d or act_dim %d > %d", h->num_actions,
+                xl::kSampleMaxActions, h->cfg.act_dim, xl::kSampleMaxRows);
+  return XL_OK;
+}
+
+int xl_set_sampling(xl_handle* h, const xl_sampling* params, uint32_t step0, void* stream) {
+  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+  if (params) {
+    int rc = check_sampling(h, params);
+    if (rc) return rc;
+  }
+  if (h->sampling != (params != nullptr)) {
+    // the sampling kernel and the counter advance are baked into captured graphs; the parameters are not
+    for (auto& g : h->graphs)
+      if (g.exec) cudaGraphExecDestroy(g.exec);
+    h->graphs.clear();
+    h->sampling = params != nullptr;
+  }
+  if (params) {
+    xl::launch_set_sampling(h->counters + kCntArmed, params, h->counters + kCntSample, step0, (cudaStream_t)stream);
+    XL_CUDA(cudaGetLastError());
+  }
+  return XL_OK;
+}
+
+int xl_sample_actions(xl_handle* h, const float* logits, int B, unsigned flags, const xl_sampling* params,
+                      uint32_t step, int32_t* tokens, float* actions, void* stream) {
+  int rc = check_batch(h, B);
+  if (rc) return rc;
+  if (!logits || !params || !tokens || !actions) return fail(XL_ERR_INVALID_ARG, "null argument");
+  rc = check_sampling(h, params);
+  if (rc) return rc;
+  const xl_config& c = h->cfg;
+  cudaStream_t s = (cudaStream_t)stream;
+  const bool discrete = (flags & XL_FLAG_DISCRETE) != 0;
+  // the kernel draws for (*counter - 1)
+  xl::launch_set_sampling(h->counters + kCntUnit, params, h->counters + kCntUnitStep, step + 1u, s);
+  const float bw = (c.tok_max_val - c.tok_min_val) / (float)c.action_channels;
+  xl::launch_sample_tokens(logits, discrete ? h->num_actions : h->head_out, B, c.act_dim, h->num_actions,
+                           c.discrete_actions, discrete ? 1 : 0, discrete ? 0.f : bw, discrete ? 0.f : c.tok_min_val,
+                           tokens, actions, nullptr, nullptr, 1, 0, h->counters + kCntUnit, h->counters + kCntUnitStep, 0,
+                           s);
+  h->launches += 2;
+  XL_CUDA(cudaGetLastError());
   return XL_OK;
 }
 

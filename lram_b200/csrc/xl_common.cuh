@@ -133,4 +133,36 @@ __device__ __forceinline__ float ld_cg(const float* p) { return __ldcg(p); }
 
 __device__ __forceinline__ float bf16_bits_to_float(uint16_t b) { return __uint_as_float(((uint32_t)b) << 16); }
 
+// torch.argmax of lg[0..n) by one warp (result valid in every lane): first index of the maximum; NaN counts as the
+// maximum (first NaN wins). Used by the argmax action kernel and as the sampler's fallback, which must agree.
+__device__ __forceinline__ int warp_argmax(const float* __restrict__ lg, int n, int lane) {
+  float best = -INFINITY;
+  int bi = 0x7fffffff;
+  bool best_nan = false;
+  for (int i = lane; i < n; i += 32) {
+    const float v = lg[i];
+    const bool vn = (v != v);
+    bool take;
+    if (best_nan) take = false;                       // earlier NaN in this lane wins (smaller index)
+    else if (vn) take = true;
+    else take = (bi == 0x7fffffff) || (v > best);
+    if (take) { best = v; bi = i; best_nan = vn; }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
+    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+    const int on = __shfl_xor_sync(0xffffffffu, (int)best_nan, o);
+    bool take;
+    if (oi == 0x7fffffff) take = false;
+    else if (bi == 0x7fffffff) take = true;
+    else if (best_nan && on) take = oi < bi;
+    else if (on) take = true;
+    else if (best_nan) take = false;
+    else take = (ov > best) || (ov == best && oi < bi);
+    if (take) { best = ov; bi = oi; best_nan = (on != 0); }
+  }
+  return bi;
+}
+
 }  // namespace xl

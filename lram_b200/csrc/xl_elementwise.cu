@@ -201,6 +201,7 @@ __global__ void __launch_bounds__(256) embed_tokens_kernel(
     const float* __restrict__ w_ret, const float* __restrict__ b_ret, const float* __restrict__ w_rew,
     const float* __restrict__ b_rew, const float* __restrict__ ln_w, const float* __restrict__ ln_b,
     float eps, float* __restrict__ x, int B, int d, unsigned* __restrict__ step_counter,
+    unsigned* __restrict__ sample_counter,
     const float* __restrict__ ln0_w, float ln0_eps, float* __restrict__ xn0, __nv_bfloat16* __restrict__ a_hi,
     __nv_bfloat16* __restrict__ a_lo) {
   const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -209,6 +210,8 @@ __global__ void __launch_bounds__(256) embed_tokens_kernel(
   // token ring (xl_set_token_ring): this is the first kernel of an env step that every step runs -> it advances the
   // step counter the argmax kernel at the end of the step derives its ring slot from
   if (step_counter && blockIdx.x == 0 && threadIdx.x == 0) *step_counter = *step_counter + 1;
+  // the sampler's step (xl_set_sampling) advances here for the same reason
+  if (sample_counter && blockIdx.x == 0 && threadIdx.x == 0) *sample_counter = *sample_counter + 1;
   pdl_trigger();
   if (row >= 3 * B) return;
   const int b = row / 3, tok = row - 3 * b;
@@ -262,6 +265,7 @@ __global__ void __launch_bounds__(1024) embed_tokens_cta_kernel(
     const float* __restrict__ w_ret, const float* __restrict__ b_ret, const float* __restrict__ w_rew,
     const float* __restrict__ b_rew, const float* __restrict__ ln_w, const float* __restrict__ ln_b,
     float eps, float* __restrict__ x, int B, int d, unsigned* __restrict__ step_counter,
+    unsigned* __restrict__ sample_counter,
     const float* __restrict__ ln0_w, float ln0_eps, float* __restrict__ xn0, __nv_bfloat16* __restrict__ a_hi,
     __nv_bfloat16* __restrict__ a_lo) {
   __shared__ float red[32];
@@ -281,6 +285,7 @@ __global__ void __launch_bounds__(1024) embed_tokens_cta_kernel(
   }
   pdl_wait();
   if (step_counter && blockIdx.x == 0 && threadIdx.x == 0) *step_counter = *step_counter + 1;   // token ring slot
+  if (sample_counter && blockIdx.x == 0 && threadIdx.x == 0) *sample_counter = *sample_counter + 1;   // sampler step
   pdl_trigger();
   float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
   if (ok) {
@@ -320,17 +325,18 @@ __global__ void __launch_bounds__(1024) embed_tokens_cta_kernel(
 void launch_embed_tokens(const float* s_emb, const float* rtg, const float* rew, const float* w_ret,
                          const float* b_ret, const float* w_rew, const float* b_rew, const float* ln_w,
                          const float* ln_b, float eps, float* x, int B, int d, unsigned* step_counter,
-                         const float* ln0_w, float ln0_eps, float* xn0, void* a_hi, void* a_lo, cudaStream_t s) {
+                         unsigned* sample_counter, const float* ln0_w, float ln0_eps, float* xn0, void* a_hi,
+                         void* a_lo, cudaStream_t s) {
   const int rows = 3 * B;
   if (d <= 4096 && (d & 3) == 0) {
     const int threads = (((d >> 2) + 31) / 32) * 32;
     launch_k(embed_tokens_cta_kernel, dim3(rows), dim3(threads), 0, s, s_emb, rtg, rew, w_ret, b_ret, w_rew, b_rew, ln_w,
-             ln_b, eps, x, B, d, step_counter, ln0_w, ln0_eps, xn0, (__nv_bfloat16*)a_hi, (__nv_bfloat16*)a_lo);
+             ln_b, eps, x, B, d, step_counter, sample_counter, ln0_w, ln0_eps, xn0, (__nv_bfloat16*)a_hi, (__nv_bfloat16*)a_lo);
     return;
   }
   dim3 grid((rows + 7) / 8);
   launch_k(embed_tokens_kernel, grid, dim3(256), 0, s, s_emb, rtg, rew, w_ret, b_ret, w_rew, b_rew, ln_w, ln_b, eps,
-           x, B, d, step_counter, ln0_w, ln0_eps, xn0, (__nv_bfloat16*)a_hi, (__nv_bfloat16*)a_lo);
+           x, B, d, step_counter, sample_counter, ln0_w, ln0_eps, xn0, (__nv_bfloat16*)a_hi, (__nv_bfloat16*)a_lo);
 }
 
 // zero-pad states [rows, K] -> bf16 hi/lo operand planes [rows, Kpad] of the embed_state GEMM (pad + split in one)
@@ -974,33 +980,7 @@ __global__ void __launch_bounds__(256) argmax_tokens_kernel(const float* __restr
   const int b = discrete ? w : w / act_dim;
   const int j = discrete ? 0 : w - b * act_dim;
   const float* lg = logits + (int64_t)b * row_pitch + (int64_t)j * num_actions;
-  const int n = discrete ? discrete_actions : num_actions;
-  float best = -INFINITY;
-  int bi = 0x7fffffff;
-  bool best_nan = false;
-  for (int i = lane; i < n; i += 32) {
-    const float v = lg[i];
-    const bool vn = (v != v);
-    bool take;
-    if (best_nan) take = false;                       // earlier NaN in this lane wins (smaller index)
-    else if (vn) take = true;
-    else take = (bi == 0x7fffffff) || (v > best);
-    if (take) { best = v; bi = i; best_nan = vn; }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float ov = __shfl_xor_sync(0xffffffffu, best, o);
-    const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
-    const int on = __shfl_xor_sync(0xffffffffu, (int)best_nan, o);
-    bool take;
-    if (oi == 0x7fffffff) take = false;
-    else if (bi == 0x7fffffff) take = true;
-    else if (best_nan && on) take = oi < bi;
-    else if (on) take = true;
-    else if (best_nan) take = false;
-    else take = (ov > best) || (ov == best && oi < bi);
-    if (take) { best = ov; bi = oi; best_nan = (on != 0); }
-  }
+  const int bi = warp_argmax(lg, discrete ? discrete_actions : num_actions, lane);
   if (lane == 0) {
     // token ring: the step's tokens also land in slot (step - 1) % slots of the caller's ring, from where the
     // multi-GPU result gather picks them up without a copy between graph replays

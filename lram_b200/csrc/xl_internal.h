@@ -27,8 +27,10 @@ void launch_ln_rows_reduce(float* x, const float* part, int splits, int64_t part
 void launch_embed_tokens(const float* s_emb, const float* rtg, const float* rew, const float* w_ret,
                          const float* b_ret, const float* w_rew, const float* b_rew, const float* ln_w,
                          const float* ln_b, float eps, float* x, int B, int d, unsigned* step_counter,
-                         const float* ln0_w, float ln0_eps, float* xn0, void* a_hi, void* a_lo, cudaStream_t s);
+                         unsigned* sample_counter, const float* ln0_w, float ln0_eps, float* xn0, void* a_hi,
+                         void* a_lo, cudaStream_t s);
 // ln0_w != nullptr: also the first block's pre-norm of the produced rows -> xn0 (fp32) and/or bf16 hi/lo planes
+// step_counter / sample_counter (nullable): incremented once per launch (token ring slot / sampler step)
 void launch_pad_split(const float* in, int K, void* hi, void* lo, int Kpad, int rows, cudaStream_t s);
 void launch_ln_rows_gather(const float* x, const float* part, int splits, int64_t part_stride, const float* w,
                            float eps, int rows, int d, int row_mul, int row_off, void* a_hi, void* a_lo,
@@ -72,6 +74,21 @@ void launch_argmax_tokens(const float* logits, int64_t row_pitch, int B, int act
                           int32_t* tokens, float* actions, int32_t* ring, const unsigned* step_counter,
                           int ring_slots, int64_t ring_slot_stride, cudaStream_t s);
 void launch_set_u32(unsigned* p, unsigned v, cudaStream_t s);
+
+// ---- xl_sample.cu --------------------------------------------------------------------------------
+// Stochastic action selection (xl_set_sampling; contract in include/xlstm_b200.h): drop-in for launch_argmax_tokens
+// with the same layouts. prm points at a device copy of the parameters; the step drawn for is *step_counter - 1;
+// env b's global id is prm->env_id_base + (env_offset + b) * prm->env_id_stride. num_actions <= kSampleMaxActions,
+// act_dim <= kSampleMaxRows.
+constexpr int kSampleMaxActions = 512;
+constexpr int kSampleMaxRows = 8;
+void launch_sample_tokens(const float* logits, int64_t row_pitch, int B, int act_dim, int num_actions,
+                          int discrete_actions, int discrete, float bin_width, float min_val, int32_t* tokens,
+                          float* actions, int32_t* ring, const unsigned* ring_counter, int ring_slots,
+                          int64_t ring_slot_stride, const void* prm, const unsigned* step_counter, int env_offset,
+                          cudaStream_t s);
+// stream-ordered write of the parameters (an xl_sampling) to dst and of `counter_value` to *counter
+void launch_set_sampling(void* dst, const void* params, unsigned* counter, unsigned counter_value, cudaStream_t s);
 
 void launch_state_reset(float* C, float* n, float* m, float* conv, const uint8_t* mask, int B,
                         int64_t c_per_env, int64_t n_per_env, int64_t m_per_env, int64_t conv_per_env,

@@ -24,6 +24,7 @@ from __future__ import annotations
 
 import dataclasses
 import math
+import weakref
 from typing import Any, Dict, Optional
 
 import torch
@@ -397,6 +398,13 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
                 self.embed_image.to(self._engine.device)
         return self._engine
 
+    def engine_for(self, B: int) -> XLSTMEngine:
+        """The engine, rebuilt with room for B envs when it has less."""
+        if B > self.engine.max_batch:
+            self.max_batch = self.encoder.max_batch = B
+            self.invalidate_engine()
+        return self.engine
+
     @property
     def device(self):
         return self.engine.device
@@ -429,13 +437,9 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
         if prompt is not None or context_trjs is not None:
             raise NotImplementedError("prompts / retrieval contexts are out of scope")
         cfg = self.cfg
-        engine = self.engine
-        dev = engine.device
         B = states.shape[0]
-        if B > engine.max_batch:
-            self.max_batch = self.encoder.max_batch = B
-            self.invalidate_engine()
-            engine = self.engine
+        engine = self.engine_for(B)
+        dev = engine.device
         state_embeds = False
         if states.dim() == 5:
             # image observations [B, T, C, H, W], raw 0..255 whatever the dtype: /255 (unconditionally, as embed_inputs
@@ -521,12 +525,20 @@ class DiscreteDecisionXLSTM:
     (src/callbacks/evaluation.py:134-139), plus `predict_batch`, the same computation for B envs at once (used by
     `lram_b200.rollout.custom_evaluate_policy`). Carries what the loop reads from the agent: `past_key_values`,
     `use_inference_cache`, `eval_context_len`, `persist_context`, `compute_target_return_val`,
-    `get_reward_scale_for_env`."""
+    `get_reward_scale_for_env`.
+
+    `a_sample_kwargs` samples the actions as the reference does (`sample_from_logits` on the step's logits, torch's
+    global RNG). Setting `a_sample_seed` as well moves the draw onto the device: the policy's engine is armed with
+    those kwargs (`XLSTMEngine.set_sampling`, a Philox stream keyed on the seed) and `predict` / `predict_batch` return
+    the step's sampled action tokens, with the shape and dtype of the torch path. The two paths differ in one place:
+    the torch path's top-p guard (`percentile != max`, all rows) spans the whole batch of `predict_batch`, the device
+    path takes it per env, as the reference's one call per env does."""
 
     def __init__(self, policy: MultiDomainDiscreteDecisionXLSTMModel, use_inference_cache: bool = True,
                  state_mean=None, state_std=None, reset_inf_cache_freq: Optional[int] = None,
                  target_return: float = 1.0, reward_scale: float = 1.0, persist_context: bool = False,
-                 eval_context_len: int = 5, a_sample_kwargs: Optional[dict] = None):
+                 eval_context_len: int = 5, a_sample_kwargs: Optional[dict] = None,
+                 a_sample_seed: Optional[int] = None):
         self.policy = policy
         self.device = policy.device
         self.use_inference_cache = use_inference_cache
@@ -540,6 +552,8 @@ class DiscreteDecisionXLSTM:
         self.persist_context = persist_context
         self.eval_context_len = eval_context_len
         self.a_sample_kwargs = a_sample_kwargs
+        self.a_sample_seed = a_sample_seed
+        self._sampler_engine = None                 # weakref to the engine armed with the device sampler
         self.s_proj_raw = False
         self.ddp_kwargs: Dict[str, Any] = {}
 
@@ -594,11 +608,14 @@ class DiscreteDecisionXLSTM:
     def get_action_pred(self, policy, states, actions, rewards, returns_to_go, timesteps, attention_mask,
                         deterministic, prompt, is_eval=False, task_id=None, env_act_dim=None):
         """discrete_decision_transformer_sb3.py:13-72, shared-action-head branch (:60-68)."""
+        device_sampling = self._arm_device_sampler(policy, states.shape[0])
         out = policy(states=states, actions=actions, rewards=rewards, returns_to_go=returns_to_go,
                      timesteps=timesteps, attention_mask=attention_mask, return_dict=True,
                      deterministic=deterministic, prompt=prompt, task_id=task_id, ddp_kwargs=self.ddp_kwargs,
                      use_inference_cache=self.use_inference_cache, past_key_values=self.past_key_values)
-        if self.a_sample_kwargs is not None:
+        if device_sampling:
+            action = out.action_tokens[0, :out.action_logits.shape[-2]]
+        elif self.a_sample_kwargs is not None:
             action = sample_from_logits(out.action_logits[0, -1], **self.a_sample_kwargs)   # :62-63
         else:
             action = out.action_preds[0, -1]
@@ -607,6 +624,16 @@ class DiscreteDecisionXLSTM:
         if env_act_dim is not None:
             action = action[:env_act_dim]
         return action, action
+
+    def _arm_device_sampler(self, policy, B: int) -> bool:
+        """True when actions are drawn on the device; arms the engine that will run a batch of B envs once."""
+        if self.a_sample_kwargs is None or self.a_sample_seed is None:
+            return False
+        engine = policy.engine_for(B)
+        if self._sampler_engine is None or self._sampler_engine() is not engine:
+            engine.set_sampling(**self.a_sample_kwargs, seed=self.a_sample_seed)
+            self._sampler_engine = weakref.ref(engine)
+        return True
 
     @torch.no_grad()
     def predict_batch(self, policy, observations: torch.Tensor, returns_to_go: torch.Tensor, action_dim: int,
@@ -622,12 +649,15 @@ class DiscreteDecisionXLSTM:
         states, actions, rtg, timesteps, _, rewards = self.pad_inputs(states, actions, rtg, timesteps, rewards=rewards)
         if self.state_mean is not None and self.state_std is not None:
             states = (states - self.state_mean) / self.state_std
+        device_sampling = self._arm_device_sampler(policy, B)
         out = policy(states=states, actions=actions, rewards=rewards, returns_to_go=rtg, timesteps=timesteps,
                      attention_mask=torch.ones(B, 1, dtype=torch.long, device=self.device), return_dict=True,
                      deterministic=True, prompt=None, task_id=None, ddp_kwargs=self.ddp_kwargs,
                      use_inference_cache=True, past_key_values=self.past_key_values)
         self.past_key_values = out.past_key_values
-        if self.a_sample_kwargs is not None:
+        if device_sampling:
+            act = out.action_tokens[:, :out.action_logits.shape[-2]]
+        elif self.a_sample_kwargs is not None:
             act = sample_from_logits(out.action_logits[:, -1], **self.a_sample_kwargs)
         else:
             act = out.action_preds[:, -1]

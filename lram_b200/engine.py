@@ -13,6 +13,7 @@ from __future__ import annotations
 
 import ctypes as C
 import functools
+import math
 from typing import Dict, Optional
 
 import torch
@@ -161,6 +162,24 @@ class StateCache:
             self.view(i, L.XL_STATE_N).copy_(n.to(self.buf.device, torch.float32).reshape(self.B, -1, n.shape[2]))
             self.view(i, L.XL_STATE_M).copy_(m.to(self.buf.device, torch.float32).reshape(self.B, -1))
             self.view(i, L.XL_STATE_CONV).copy_(st["conv_state"][0].to(self.buf.device, torch.float32))
+
+
+def sampling_params(cfg: XLSTMPolicyConfig, temperature: float = 1.0, top_k: int = 0, top_p: float = 0.5,
+                    seed: int = 0, env_id_base: int = 0, env_id_stride: int = 1) -> L.XLSampling:
+    """Checked `xl_sampling` for the device sampler; raises ValueError on what the library would reject."""
+    temperature, top_p = float(temperature), float(top_p)
+    if not (math.isfinite(temperature) and temperature > 0.0):
+        raise ValueError(f"temperature={temperature} must be finite and > 0")
+    if not 0.0 <= top_p <= 1.0:
+        raise ValueError(f"top_p={top_p} outside [0, 1]")
+    if not 0 <= int(top_k) <= cfg.num_actions:
+        raise ValueError(f"top_k={top_k} outside [0, num_actions={cfg.num_actions}]")
+    if int(env_id_base) < 0 or int(env_id_stride) < 1:
+        raise ValueError(f"env_id_base={env_id_base} must be >= 0 and env_id_stride={env_id_stride} >= 1")
+    if not 0 <= int(seed) < 2 ** 64:
+        raise ValueError(f"seed={seed} outside [0, 2^64)")
+    return L.XLSampling(temperature=temperature, top_p=top_p, top_k=int(top_k), env_id_base=int(env_id_base),
+                        env_id_stride=int(env_id_stride), seed=int(seed))
 
 
 def _on_device(fn):
@@ -382,6 +401,40 @@ class XLSTMEngine:
         self._token_ring = ring                       # keep it alive
         L.check(self.lib.xl_set_token_ring(self.handle, _ptr(ring), 0 if ring is None else ring.shape[0],
                                            int(next_slot), self._stream()))
+
+    def set_sampling(self, temperature: Optional[float] = 1.0, top_k: int = 0, top_p: float = 0.5, seed: int = 0,
+                     env_id_base: int = 0, env_id_stride: int = 1, step0: int = 0):
+        """Arm the device sampler (`set_sampling(None)` disarms): every policy step then draws its action tokens by the
+        `sample_from_logits` rule (defaults are its defaults) from a Philox stream keyed on (seed, step, global env id,
+        action row) instead of taking the argmax; contract at xl_set_sampling in include/xlstm_b200.h. The first step
+        after arming draws for step `step0`. Env b of this engine has global id env_id_base + b * env_id_stride (a shard
+        of envs i -> rank i mod N: base = rank, stride = N). Parameters are checked before anything reaches the GPU."""
+        p = None if temperature is None else sampling_params(self.cfg, temperature, top_k, top_p, seed, env_id_base,
+                                                             env_id_stride)
+        if not 0 <= int(step0) < 2 ** 32:
+            raise ValueError(f"step0={step0} outside [0, 2^32)")
+        with torch.cuda.device(self.device):
+            L.check(self.lib.xl_set_sampling(self.handle, None if p is None else C.byref(p), int(step0), self._stream()))
+
+    @_on_device
+    def sample_actions(self, logits: torch.Tensor, step: int, temperature: float = 1.0, top_k: int = 0,
+                       top_p: float = 0.5, seed: int = 0, env_id_base: int = 0, env_id_stride: int = 1,
+                       discrete: bool = False):
+        """The sampler alone on given logits (discrete [B, num_actions], continuous [B, act_dim * num_actions]) at an
+        explicit step: -> (tokens int32 [B, act_dim], actions fp32 [B, act_dim]) as `policy_step` returns them
+        (discrete: first column). Leaves the armed sampler alone."""
+        cfg = self.cfg
+        p = sampling_params(cfg, temperature, top_k, top_p, seed, env_id_base, env_id_stride)
+        n = cfg.num_actions if discrete else cfg.head_out
+        assert logits.is_cuda and logits.dtype == torch.float32 and logits.dim() == 2 and logits.shape[1] == n
+        logits = logits.contiguous()
+        B = logits.shape[0]
+        tokens = torch.zeros(B, cfg.act_dim, dtype=torch.int32, device=self.device)
+        actions = torch.zeros(B, cfg.act_dim, dtype=torch.float32, device=self.device)
+        L.check(self.lib.xl_sample_actions(self.handle, _ptr(logits), B, L.XL_FLAG_DISCRETE if discrete else 0,
+                                           C.byref(p), int(step) & 0xFFFFFFFF, _ptr(tokens), _ptr(actions),
+                                           self._stream()))
+        return tokens, actions
 
     @_on_device
     def set_option(self, name: str, value: int):

@@ -158,10 +158,20 @@ class OverlappedTokenGather:
 
 class BatchedRollout:
     """Drives B envs of a `SyntheticEnvBatch`-like object (reset() -> obs[B,204]; step(a) -> obs, reward, done)
-    through the CUDA policy, one library call per env step with pinned host buffers."""
+    through the CUDA policy, one library call per env step with pinned host buffers.
 
-    def __init__(self, engine: XLSTMEngine, envs, mode: int = L.XL_MODE_FUSED, use_graph: bool = True):
+    `sample_kwargs` (the reference's `a_sample_kwargs`: temperature, top_k, top_p; env_id_base / env_id_stride for a
+    shard of a multi-GPU run) arms the engine's device sampler, so a sampled rollout is still one call per step. Draws
+    come from a counter-based stream keyed on `seed` (None: one drawn from torch's global RNG); every `run()` without
+    `keep_state` restarts it at step 0, so equal seeds give equal rollouts. The engine stays armed afterwards."""
+
+    def __init__(self, engine: XLSTMEngine, envs, mode: int = L.XL_MODE_FUSED, use_graph: bool = True,
+                 sample_kwargs: Optional[Dict[str, Any]] = None, seed: Optional[int] = None):
         self.engine, self.envs = engine, envs
+        self.sample_kwargs = dict(sample_kwargs) if sample_kwargs is not None else None
+        if self.sample_kwargs is not None:
+            self.seed = int(torch.randint(0, 2 ** 62, ()).item()) if seed is None else int(seed)
+            engine.set_sampling(**self.sample_kwargs, seed=self.seed, step0=0)
         self.B = envs.B
         cfg = engine.cfg
         self.mode = mode
@@ -192,6 +202,8 @@ class BatchedRollout:
         rtg = self.rtg0.copy()
         if not keep_state:
             self.engine.reset(self.state)
+            if self.sample_kwargs is not None:
+                self.engine.set_sampling(**self.sample_kwargs, seed=self.seed, step0=0)
         ep_ret = np.zeros(B, dtype=np.float64)
         returns: List[List[float]] = [[] for _ in range(B)]
         toks = [] if record else None
