@@ -279,6 +279,28 @@ int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B
 int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
                       int Tn, unsigned flags, void* stream);
 
+/* Ragged context prefill: a context length per env. lengths is a HOST int32 [B] array (tokens for xl_prefill_ragged,
+ * timesteps for xl_policy_prefill_ragged); the buffers keep the shapes above ([B, S, d]; [B, Tn, state_dim], [B, Tn]).
+ *  - Env b's state ends exactly where lengths[b] recurrent steps over its first lengths[b] tokens (timesteps) would
+ *    leave it, the promise xl_prefill makes, per env. lengths[b] == 0 leaves every byte of env b's state unchanged.
+ *  - Inputs at positions >= lengths[b] are never read (they may hold NaN).
+ *  - y_out (nullable): row t < lengths[b] holds that token's last_hidden_state; every other row is written as 0.
+ *  - Every length == S (Tn): this IS xl_prefill / xl_policy_prefill (bit-identical). Every length 0: the state is left
+ *    alone, y_out zeroed, XL_OK.
+ *  - XL_ERR_INVALID_ARG before any device work: lengths NULL, a length < 0 or > S (Tn), and the checks of the uniform
+ *    calls. XL_ERR_UNSUPPORTED (state untouched) for lengths that are neither all S nor all 0 when the shape has no
+ *    sequence path (conv_kernel != 4, or a head dim without a cell plan); no shipped preset is affected.
+ *  - The policy form's work never advances the sampler's step counter or the token ring slot (as xl_policy_prefill).
+ * Work goes to the envs that have tokens: the active envs are sorted by length (descending, stable) and each chunk runs
+ * on the prefix of them that still has tokens, an env's end padded up to the chunk with identity tokens (forget gate 1,
+ * input gate 0, conv window and sLSTM state kept). When the active envs are not already envs 0..B'-1 in that order, their
+ * state slots are gathered into a library-owned compact state of xl_state_bytes(h, B') bytes (grow-only, freed by
+ * xl_destroy; growing it synchronises the device) and scattered back at the end. Not graph-capturable. */
+int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out, const int32_t* lengths, int B, int S,
+                      unsigned flags, void* stream);
+int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
+                             const int32_t* lengths, int B, int Tn, unsigned flags, void* stream);
+
 /* out[M,N] = A[M,K] @ W[N,K]^T (+ bias[N]) (+ residual[M,N]); A fp32, W bf16, fp32 accumulate.
  * The nn.Linear of proj_up / proj_down / embed_state / action_net. impl: 0 auto, 1 CUDA-core, 2 tcgen05. */
 int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bias, const float* residual,

@@ -117,6 +117,10 @@ def load():
     lib.xl_prefill.restype = i32
     lib.xl_policy_prefill.argtypes = [vp, vp, vp, vp, vp, i32, i32, u32, vp]
     lib.xl_policy_prefill.restype = i32
+    lib.xl_prefill_ragged.argtypes = [vp, vp, vp, vp, vp, i32, i32, u32, vp]
+    lib.xl_prefill_ragged.restype = i32
+    lib.xl_policy_prefill_ragged.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, u32, vp]
+    lib.xl_policy_prefill_ragged.restype = i32
     lib.xl_linear.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
     lib.xl_linear.restype = i32
     lib.xl_set_token_ring.argtypes = [vp, vp, i32, i32, vp]

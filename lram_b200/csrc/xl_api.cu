@@ -138,6 +138,12 @@ struct xl_handle {
         *pf_semb = nullptr, *pf_spad = nullptr, *pf_sin = nullptr, *pf_rtg = nullptr, *pf_rew = nullptr, *pf_gsc = nullptr;
   __nv_bfloat16 *pf_hi = nullptr, *pf_lo = nullptr;
   uint8_t *pf_pc = nullptr, *pf_pv = nullptr;   // prepared operands of the chunkwise tensor-core cell
+  // ragged prefill (xl_prefill_ragged / xl_policy_prefill_ragged): compact state of the active envs (grow-only,
+  // xl_state_bytes(h, active envs)) and the call's [perm | token lengths] index (host staging and device copy)
+  char* rg_state = nullptr;
+  size_t rg_state_bytes = 0;
+  int32_t* rg_idx = nullptr;                    // device, 2 * max_batch
+  std::vector<int32_t> rg_host;
   int prefill_gemm_2cta = 0;                    // A/B: shallow-ring Linear tiles, two CTAs per SM        ("prefill_gemm_2cta")
   int prefill_rows = 16384;                     // rows (envs x tokens) per prefill chunk                  ("prefill_rows")
   char* pf_tc = nullptr;                        // workspace of the tcgen05 chunkwise cell (grow-only)
@@ -525,8 +531,9 @@ int block_post(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigne
 // [b0, b0+Bk) of a state holding Btot envs. pend_sp > 1: the previous mLSTM block left that many split-K
 // proj_down planes, folded into x by this block's first LayerNorm. Workspace reuse: xn = LN(x), act = swish(conv),
 // u = gate pre-activations [M,4,d], gated = y [M,d], qkv = feed-forward up projection [M,2ff].
+// len / pos (ragged prefill, b0 == 0): env b of the slice has clamp(len[b] - pos, 0, T) real tokens, pads after them
 int slstm_block(xl_handle* h, void* state, const Ws& ws, int Btot, int b0, int Bk, int i, int T, unsigned flags,
-                int pend_sp, cudaStream_t s) {
+                int pend_sp, cudaStream_t s, const int32_t* len = nullptr, int pos = 0) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim, NH = c.num_heads, ff = c.ffn_dim, KS = c.conv_kernel, M = Bk * T;
   const StateLayout L = state_layout(h, Btot);
@@ -543,12 +550,12 @@ int slstm_block(xl_handle* h, void* state, const Ws& ws, int Btot, int b0, int B
                               d, nullptr, nullptr, s);
   else
     xl::launch_ln_rows(ws.x, d, ws.xn, d, F(XL_W_XLSTM_NORM), nullptr, 1, c.ln_eps, M, d, nullptr, nullptr, s);
-  if (!xl::launch_slstm_conv(ws.xn, conv, F(XL_W_CONV_W), F(XL_W_CONV_B), ws.act, Bk, T, d, KS, s))
+  if (!xl::launch_slstm_conv(ws.xn, conv, F(XL_W_CONV_W), F(XL_W_CONV_B), ws.act, Bk, T, d, KS, s, len, pos))
     return fail(XL_ERR_UNSUPPORTED, "sLSTM conv kernel not instantiated for KS=%d", KS);
   xl::launch_slstm_gates(ws.act, ws.xn, F(XL_W_S_GATE_I), F(XL_W_S_GATE_F), F(XL_W_S_GATE_Z), F(XL_W_S_GATE_O),
                          F(XL_W_S_BIAS), ws.u, M, d, NH, s);
   for (int t = 0; t < T; ++t)
-    XL_CUDA(xl::launch_slstm_cell(ws.u, F(XL_W_S_RECURRENT), st, ws.gated, Bk, Btot, T, t, d, NH, s));
+    XL_CUDA(xl::launch_slstm_cell(ws.u, F(XL_W_S_RECURRENT), st, ws.gated, Bk, Btot, T, t, d, NH, s, len, pos));
   xl::launch_slstm_out(ws.gated, F(XL_W_S_GROUP_NORM), ws.x, st, M, T, d, NH, c.ln_eps, s);
   xl::launch_ln_rows(ws.x, d, tc_up ? nullptr : ws.xn, d, F(XL_W_FFN_NORM), nullptr, 1, c.ln_eps, M, d,
                      tc_up ? ws.a_hi : nullptr, tc_up ? ws.a_lo : nullptr, s);
@@ -950,11 +957,15 @@ int prefill_chunk_tokens(const xl_handle* h, int B) {
 }
 
 // The block stack over the chunk held in pf_x [B*Sc, d] (rows [env][token]), in place; state advanced by Sc tokens.
-int prefill_blocks(xl_handle* h, void* state, int B, int Sc, unsigned flags, cudaStream_t s) {
+// The state holds Btot >= B envs; the chunk belongs to its first B. Ragged prefill (len != nullptr, a device array of B
+// token counts; the chunk starts at token pos of the context): env b advances by its clamp(len[b] - pos, 0, Sc) real
+// tokens only, every env of the chunk having at least one.
+int prefill_blocks(xl_handle* h, void* state, int Btot, int B, int Sc, unsigned flags, cudaStream_t s,
+                   const int32_t* len = nullptr, int pos = 0) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim, inner = c.inner_dim, NH = c.num_heads, DH = h->DH;
   const int M = B * Sc;
-  const StateLayout L = state_layout(h, B);
+  const StateLayout L = state_layout(h, Btot);
   const Ws ws = prefill_ws(h);
   const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
   const bool tc_up = impl != 1 && xl::gemm_tc_supported(M, 2 * inner, d) && (size_t)M * d <= ws.a_cap;
@@ -963,7 +974,7 @@ int prefill_blocks(xl_handle* h, void* state, int B, int Sc, unsigned flags, cud
     if (is_slstm(h, i)) {
       // no parallel form exists for the sLSTM: its cell runs token by token (Sc launches of a tiny kernel), the
       // rest of the block (conv, gate projections, GroupNorm, feed-forward) over the whole chunk
-      int rcs = slstm_block(h, state, ws, B, 0, B, i, Sc, flags, 1, s);
+      int rcs = slstm_block(h, state, ws, Btot, 0, B, i, Sc, flags, 1, s, len, pos);
       if (rcs) return rcs;
       continue;
     }
@@ -995,11 +1006,12 @@ int prefill_blocks(xl_handle* h, void* state, int B, int Sc, unsigned flags, cud
     cp.gate_part = ws.gate_part;
     cp.B = B; cp.T = Sc; cp.inner = inner; cp.NH = NH; cp.KS = c.conv_kernel; cp.NCH = h->NCH;
     cp.impl = 0;
-    if (!xl::launch_conv_qkv_gates_seq(cp, Sc, s))
+    if (!xl::launch_conv_qkv_gates_seq(cp, Sc, s, len, pos))
       return fail(XL_ERR_UNSUPPORTED, "sequence conv/qkv kernel not instantiated for KS=%d NH=%d", cp.KS, cp.NH);
     XL_CUDA(cudaGetLastError());
     xl::launch_gate_scan_seq(ws.gate_part, (const float*)w.w[XL_W_IGATE_B], (const float*)w.w[XL_W_FGATE_B],
-                             (float*)(base + L.m_off), h->pf_f, h->pf_i, h->pf_m, h->pf_gsc, B, Sc, NH, h->NCH, s);
+                             (float*)(base + L.m_off), h->pf_f, h->pf_i, h->pf_m, h->pf_gsc, B, Sc, NH, h->NCH, s,
+                             len, pos);
     XL_CUDA(cudaGetLastError());
     // tcgen05 cell: whole 128-token chunks per (env, head) -- short runs of many envs (Sc < 64: more than half of every
     // chunk would be padding) or a workspace beyond 8 GiB fall through to the 16-token mma.sync cell
@@ -1036,6 +1048,121 @@ int prefill_blocks(xl_handle* h, void* state, int B, int Sc, unsigned flags, cud
 
 bool prefill_fast_path(const xl_handle* h) {
   return xl::prefill_cell_supported(h->DH) && h->cfg.conv_kernel == 4;
+}
+
+// ---- ragged prefill ----------------------------------------------------------------------------------------------
+// The active envs (length > 0) sorted by length, descending and stable: compact env k is caller env perm[k]. Once sorted,
+// the envs that still have tokens at position pos are a prefix Bk of the compact batch, so every chunk runs the
+// sequence kernels on that prefix (same base pointers, smaller B) and pads each env's end up to the chunk's length with
+// identity tokens. If the active envs already are envs 0..Bc-1 in that order, the chunks work on the caller's state in
+// place; otherwise the state is gathered into a compact one of Bc envs and scattered back at the end.
+struct RaggedPlan {
+  std::vector<int32_t> perm, len;     // len: in the caller's units (tokens or timesteps)
+  bool in_place = false;
+  void* st = nullptr;                 // the state the chunks advance
+  int Btot = 0;                       // envs of its layout
+  const int32_t *d_perm = nullptr, *d_len = nullptr;   // device copies; d_len in tokens
+};
+struct RaggedChunk {
+  int pos, Bk, n;                     // units [pos, pos + n) of the first Bk compact envs
+};
+
+int check_lengths(const int32_t* lengths, int B, int S, const char* what) {
+  if (!lengths) return fail(XL_ERR_INVALID_ARG, "null lengths");
+  for (int b = 0; b < B; ++b)
+    if (lengths[b] < 0 || lengths[b] > S)
+      return fail(XL_ERR_INVALID_ARG, "lengths[%d]=%d outside [0, %s=%d]", b, lengths[b], what, S);
+  return XL_OK;
+}
+
+xl::StateCopyGeom state_copy_geom(const xl_handle* h, int B, int Bc) {
+  const xl_config& c = h->cfg;
+  xl::StateCopyGeom g;
+  g.slstm_mask = h->slstm_mask;
+  g.num_blocks = c.num_blocks;
+  const int Bs[2] = {B, Bc};
+  for (int j = 0; j < 2; ++j) {
+    const StateLayout L = state_layout(h, Bs[j]);
+    g.B[j] = Bs[j];
+    g.layer_bytes[j] = L.layer_bytes; g.slayer_bytes[j] = L.slayer_bytes;
+    g.c_off[j] = L.c_off; g.n_off[j] = L.n_off; g.m_off[j] = L.m_off; g.conv_off[j] = L.conv_off;
+    g.s_off[j] = L.s_off; g.sconv_off[j] = L.sconv_off;
+  }
+  const size_t f = sizeof(float), NH = c.num_heads, DH = h->DH, KS = c.conv_kernel;
+  g.c_env = f * NH * DH * DH; g.n_env = f * NH * DH; g.m_env = f * NH; g.conv_env = f * KS * c.inner_dim;
+  g.s_env = f * c.embedding_dim; g.sconv_env = f * KS * c.embedding_dim;
+  return g;
+}
+
+// Sort, upload the index, and gather the state when the active envs are not a sorted prefix. tok = tokens per unit.
+int ragged_begin(xl_handle* h, void* state, const int32_t* lengths, int B, int tok, RaggedPlan& p, cudaStream_t s) {
+  for (int b = 0; b < B; ++b)
+    if (lengths[b] > 0) p.perm.push_back(b);
+  std::stable_sort(p.perm.begin(), p.perm.end(), [&](int a, int b) { return lengths[a] > lengths[b]; });
+  const int Bc = (int)p.perm.size();
+  p.in_place = true;
+  for (int k = 0; k < Bc; ++k) {
+    p.len.push_back(lengths[p.perm[k]]);
+    p.in_place = p.in_place && p.perm[k] == k;
+  }
+  if (!h->rg_idx) XL_CUDA(cudaMalloc((void**)&h->rg_idx, sizeof(int32_t) * 2 * (size_t)h->cfg.max_batch));
+  h->rg_host.assign(2 * (size_t)Bc, 0);
+  for (int k = 0; k < Bc; ++k) {
+    h->rg_host[k] = p.perm[k];
+    h->rg_host[Bc + k] = p.len[k] * tok;
+  }
+  XL_CUDA(cudaMemcpyAsync(h->rg_idx, h->rg_host.data(), sizeof(int32_t) * 2 * (size_t)Bc, cudaMemcpyHostToDevice, s));
+  p.d_perm = h->rg_idx;
+  p.d_len = h->rg_idx + Bc;
+  if (p.in_place) {
+    p.st = state;
+    p.Btot = B;
+    return XL_OK;
+  }
+  const size_t need = xl_state_bytes(h, Bc);
+  if (need > h->rg_state_bytes) {
+    XL_CUDA(cudaDeviceSynchronize());          // nothing may still be using the old buffer
+    if (h->rg_state) cudaFree(h->rg_state);
+    h->rg_state = nullptr;
+    h->rg_state_bytes = 0;
+    cudaError_t e = cudaMalloc((void**)&h->rg_state, need);
+    if (e != cudaSuccess)
+      return fail(XL_ERR_CUDA, "cudaMalloc(ragged prefill state %zu B) failed: %s", need, cudaGetErrorString(e));
+    h->rg_state_bytes = need;
+  }
+  xl::launch_state_permute(state, h->rg_state, p.d_perm, Bc, state_copy_geom(h, B, Bc), 0, s);
+  h->launches += 1;
+  XL_CUDA(cudaGetLastError());
+  p.st = h->rg_state;
+  p.Btot = Bc;
+  return XL_OK;
+}
+
+int ragged_end(xl_handle* h, void* state, int B, const RaggedPlan& p, cudaStream_t s) {
+  if (p.in_place) return XL_OK;
+  const int Bc = (int)p.perm.size();
+  xl::launch_state_permute(state, h->rg_state, p.d_perm, Bc, state_copy_geom(h, B, Bc), 1, s);
+  h->launches += 1;
+  XL_CUDA(cudaGetLastError());
+  return XL_OK;
+}
+
+// Chunks of the shrinking active prefix, in units of T tokens (1: encoder tokens; tokens_per_step: timesteps): today's
+// chunk length for Bk envs (prefill_chunk_tokens), cut to the longest remaining context rounded up to 8 units (16 where
+// the chunkwise cells run: whole 16-token chunks of the mma.sync cell). Grows the prefill workspace to the largest.
+int ragged_chunks(xl_handle* h, const std::vector<int32_t>& len, int T, std::vector<RaggedChunk>& out) {
+  const int gran = (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(h->DH)) ? 16 : 8;
+  int pos = 0, Bk = (int)len.size(), rows = 0;
+  while (pos < len[0]) {
+    while (len[Bk - 1] <= pos) --Bk;
+    const int cmax = prefill_chunk_tokens(h, Bk) / T;
+    const int n = std::min(cmax, (len[0] - pos + gran - 1) / gran * gran);
+    out.push_back({pos, Bk, n});
+    // >= 48 tokens per env: room for the gate-scan maps of short chunks (ensure_prefill_ws sizes them for that)
+    rows = std::max(rows, Bk * std::max(n * T, 48));
+    pos += n;
+  }
+  return ensure_prefill_ws(h, rows);
 }
 
 }  // namespace
@@ -1174,6 +1301,8 @@ void xl_destroy(xl_handle* h) {
   if (h->ws) cudaFree(h->ws);
   if (h->pf_tc) cudaFree(h->pf_tc);
   if (h->pf_buf) cudaFree(h->pf_buf);
+  if (h->rg_state) cudaFree(h->rg_state);
+  if (h->rg_idx) cudaFree(h->rg_idx);
   if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
   for (int k = 0; k < kMaxMicro - 1; ++k) {
     if (h->side[k]) cudaStreamDestroy(h->side[k]);
@@ -1588,7 +1717,7 @@ int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B
       XL_CUDA(cudaMemcpy2DAsync(h->pf_x, sizeof(float) * (size_t)Sc * d, x_in + (size_t)pos * d,
                                 sizeof(float) * (size_t)S * d, sizeof(float) * (size_t)Sc * d, B,
                                 cudaMemcpyDeviceToDevice, s));
-      rc = prefill_blocks(h, state, B, Sc, flags, s);
+      rc = prefill_blocks(h, state, B, B, Sc, flags, s);
       if (rc) return rc;
       if (y_out) {
         xl::launch_ln_rows(h->pf_x, d, h->pf_xn, d, post_w, nullptr, 1, c.ln_eps, B * Sc, d, nullptr, nullptr, s);
@@ -1661,7 +1790,7 @@ int xl_policy_prefill(xl_handle* h, void* state, const float* states, const floa
                               (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
                               0.f, nullptr, nullptr, nullptr, s);
       h->launches += 1;
-      rc = prefill_blocks(h, state, B, Tc * T, flags, s);
+      rc = prefill_blocks(h, state, B, B, Tc * T, flags, s);
       if (rc) return rc;
       pos += Tc;
     }
@@ -1683,6 +1812,93 @@ int xl_policy_prefill(xl_handle* h, void* state, const float* states, const floa
     if (rc) return rc;
   }
   return XL_OK;
+}
+
+int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out, const int32_t* lengths, int B, int S,
+                      unsigned flags, void* stream) {
+  int rc = check_batch(h, B);
+  if (rc) return rc;
+  if (!state || !x_in) return fail(XL_ERR_INVALID_ARG, "null argument");
+  if (S <= 0) return fail(XL_ERR_INVALID_ARG, "S=%d must be positive", S);
+  if ((rc = check_lengths(lengths, B, S, "S"))) return rc;
+  rc = weights_ready(h, true);
+  if (rc) return rc;
+  const int nfull = (int)std::count(lengths, lengths + B, S), nzero = (int)std::count(lengths, lengths + B, 0);
+  if (nfull == B) return xl_prefill(h, state, x_in, y_out, B, S, flags, stream);
+  if (nzero < B && !prefill_fast_path(h))
+    return fail(XL_ERR_UNSUPPORTED, "ragged prefill needs the sequence path (conv_kernel 4, a cell plan for DH=%d)", h->DH);
+  cudaStream_t s = (cudaStream_t)stream;
+  const xl_config& c = h->cfg;
+  const int d = c.embedding_dim;
+  if (y_out) XL_CUDA(cudaMemsetAsync(y_out, 0, sizeof(float) * (size_t)B * S * d, s));
+  if (nzero == B) return XL_OK;
+  const float* post_w = (const float*)h->pw[XL_W_POST_NORM - XL_W_POST_NORM];
+  RaggedPlan p;
+  std::vector<RaggedChunk> chunks;
+  if ((rc = ragged_begin(h, state, lengths, B, 1, p, s))) return rc;
+  if ((rc = ragged_chunks(h, p.len, 1, chunks))) return rc;
+  for (const RaggedChunk& ch : chunks) {
+    xl::launch_ragged_rows(const_cast<float*>(x_in), h->pf_x, p.d_perm, p.d_len, 1, ch.Bk, S, ch.n, ch.pos, d, 0, s);
+    h->launches += 1;
+    rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, ch.n, flags, s, p.d_len, ch.pos);
+    if (rc) return rc;
+    if (y_out) {
+      xl::launch_ln_rows(h->pf_x, d, h->pf_xn, d, post_w, nullptr, 1, c.ln_eps, ch.Bk * ch.n, d, nullptr, nullptr, s);
+      xl::launch_ragged_rows(y_out, h->pf_xn, p.d_perm, p.d_len, 1, ch.Bk, S, ch.n, ch.pos, d, 1, s);
+      h->launches += 2;
+    }
+    XL_CUDA(cudaGetLastError());
+  }
+  return ragged_end(h, state, B, p, s);
+}
+
+int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
+                             const int32_t* lengths, int B, int Tn, unsigned flags, void* stream) {
+  int rc = check_batch(h, B);
+  if (rc) return rc;
+  if (!state || !states || !rtg) return fail(XL_ERR_INVALID_ARG, "null argument");
+  if (Tn <= 0) return fail(XL_ERR_INVALID_ARG, "Tn=%d must be positive", Tn);
+  if ((rc = check_lengths(lengths, B, Tn, "Tn"))) return rc;
+  rc = xl_weights_ready(h);
+  if (rc) return rc;
+  const int nfull = (int)std::count(lengths, lengths + B, Tn), nzero = (int)std::count(lengths, lengths + B, 0);
+  if (nfull == B) return xl_policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream);
+  if (nzero == B) return XL_OK;
+  if (!prefill_fast_path(h))
+    return fail(XL_ERR_UNSUPPORTED, "ragged prefill needs the sequence path (conv_kernel 4, a cell plan for DH=%d)", h->DH);
+  cudaStream_t s = (cudaStream_t)stream;
+  const xl_config& c = h->cfg;
+  const int d = c.embedding_dim, sd = c.state_dim, T = c.tokens_per_step;
+  const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
+  auto PW = [&](int id) { return h->pw[id - XL_W_POST_NORM]; };
+  RaggedPlan p;
+  std::vector<RaggedChunk> chunks;
+  if ((rc = ragged_begin(h, state, lengths, B, T, p, s))) return rc;
+  if ((rc = ragged_chunks(h, p.len, T, chunks))) return rc;
+  for (const RaggedChunk& ch : chunks) {
+    const int Tc = ch.n, rows = ch.Bk * Tc;
+    const Ws ws = prefill_ws(h);
+    // the chunk's timesteps of the prefix envs, pads zero-filled: [Bk, Tc, sd], [Bk, Tc]
+    xl::launch_ragged_rows(const_cast<float*>(states), h->pf_sin, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, sd, 0, s);
+    xl::launch_ragged_rows(const_cast<float*>(rtg), h->pf_rtg, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
+    if (rewards)
+      xl::launch_ragged_rows(const_cast<float*>(rewards), h->pf_rew, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
+    xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
+    h->launches += rewards ? 4 : 3;
+    rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
+                rows, d, h->Kpad, impl, s);
+    if (rc) return rc;
+    xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
+                            (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
+                            (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
+                            (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
+                            0.f, nullptr, nullptr, nullptr, s);
+    h->launches += 1;
+    rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, Tc * T, flags, s, p.d_len, ch.pos * T);
+    if (rc) return rc;
+    XL_CUDA(cudaGetLastError());
+  }
+  return ragged_end(h, state, B, p, s);
 }
 
 int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bias, const float* residual,

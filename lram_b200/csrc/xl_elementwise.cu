@@ -4,6 +4,8 @@
 // each kernel.
 #include <cuda_bf16.h>
 
+#include <algorithm>
+
 #include "xl_common.cuh"
 #include "xl_internal.h"
 
@@ -1038,6 +1040,97 @@ void launch_state_reset(float* C, float* n, float* m, float* conv, const uint8_t
   dim3 grid(32, B);
   state_reset_kernel<<<grid, 256, 0, s>>>(C, n, m, conv, mask, B, c_per_env, n_per_env, m_per_env,
                                           conv_per_env);
+}
+
+// ---- ragged prefill: env permutation of the state and chunk rows ----------------------------------------
+// grid = (CTAs per env, Bc compact envs, blocks). Every part is env-major with a fixed per-env size, so one part of one
+// env is a contiguous run of bytes on both sides; runs whose size is a multiple of 16 B (all but m when NH < 4) go as
+// 128-bit words. HBM-bound.
+__device__ __forceinline__ void copy_run(const char* __restrict__ src, char* __restrict__ dst, size_t bytes, int64_t t0,
+                                         int64_t stride) {
+  if (bytes % 16 == 0) {
+    const uint4* s4 = reinterpret_cast<const uint4*>(src);
+    uint4* d4 = reinterpret_cast<uint4*>(dst);
+    for (int64_t i = t0; i < (int64_t)(bytes / 16); i += stride) d4[i] = s4[i];
+  } else {
+    const float* s1 = reinterpret_cast<const float*>(src);
+    float* d1 = reinterpret_cast<float*>(dst);
+    for (int64_t i = t0; i < (int64_t)(bytes / 4); i += stride) d1[i] = s1[i];
+  }
+}
+
+__global__ void __launch_bounds__(256) state_permute_kernel(char* caller, char* compact, const int32_t* __restrict__ perm,
+                                                            StateCopyGeom g, int to_caller) {
+  const int k = blockIdx.y, blk = blockIdx.z;
+  const int64_t t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
+  pdl_wait();
+  pdl_trigger();
+  const int env[2] = {perm[k], k};
+  const uint64_t below = blk >= 64 ? ~0ull : ((1ull << blk) - 1ull);
+  const int ns = __popcll(g.slstm_mask & below);
+  char* base[2];
+#pragma unroll
+  for (int j = 0; j < 2; ++j)
+    base[j] = (j ? compact : caller) + (size_t)(blk - ns) * g.layer_bytes[j] + (size_t)ns * g.slayer_bytes[j];
+  const int from = to_caller ? 1 : 0, to = 1 - from;
+  auto run = [&](const size_t* off, size_t env_bytes, size_t plane) {
+    // plane: bytes between the planes of one part per env of the batch (sLSTM (y, c, n, m)); 0 = one plane
+    for (int p = 0; p < (plane ? 4 : 1); ++p)
+      copy_run(base[from] + off[from] + p * plane * g.B[from] + env[from] * env_bytes,
+               base[to] + off[to] + p * plane * g.B[to] + env[to] * env_bytes, env_bytes, t0, stride);
+  };
+  if ((g.slstm_mask >> blk) & 1ull) {
+    run(g.s_off, g.s_env, g.s_env);
+    run(g.sconv_off, g.sconv_env, 0);
+  } else {
+    run(g.c_off, g.c_env, 0);
+    run(g.n_off, g.n_env, 0);
+    run(g.m_off, g.m_env, 0);
+    run(g.conv_off, g.conv_env, 0);
+  }
+}
+
+void launch_state_permute(void* caller, void* compact, const int32_t* perm, int Bc, const StateCopyGeom& g,
+                          int to_caller, cudaStream_t s) {
+  // ~8 KiB of C per thread row of a CTA: enough CTAs in flight for HBM at a few envs, no more than 64 per (env, block)
+  const size_t words = std::max(g.c_env, g.s_env * 4) / 16;
+  const unsigned per = (unsigned)std::min<size_t>(64, std::max<size_t>(1, words / (256 * 32)));
+  launch_k(state_permute_kernel, dim3(per, Bc, g.num_blocks), dim3(256), 0, s, (char*)caller, (char*)compact, perm, g,
+           to_caller);
+}
+
+__global__ void __launch_bounds__(256) ragged_rows_kernel(float* caller, float* compact, const int32_t* __restrict__ perm,
+                                                          const int32_t* __restrict__ len, int len_div, int S, int Sc,
+                                                          int pos, int width, int to_caller) {
+  const int k = blockIdx.y;
+  pdl_wait();
+  pdl_trigger();
+  const int nk = min(max(len[k] / len_div - pos, 0), Sc);
+  const int rows = to_caller ? nk : Sc;                       // the scatter writes valid rows only
+  float* crow = compact + (int64_t)k * Sc * width;
+  float* urow = caller + ((int64_t)perm[k] * S + pos) * width;
+  const int64_t n = (int64_t)rows * width, valid = (int64_t)nk * width;
+  const int64_t t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, stride = (int64_t)gridDim.x * blockDim.x;
+  if (width % 4 == 0) {
+    for (int64_t i = t0; i < n / 4; i += stride) {
+      if (to_caller) reinterpret_cast<float4*>(urow)[i] = reinterpret_cast<const float4*>(crow)[i];
+      else reinterpret_cast<float4*>(crow)[i] = 4 * i < valid ? reinterpret_cast<const float4*>(urow)[i]
+                                                              : make_float4(0.f, 0.f, 0.f, 0.f);
+    }
+  } else {
+    for (int64_t i = t0; i < n; i += stride) {
+      if (to_caller) urow[i] = crow[i];
+      else crow[i] = i < valid ? urow[i] : 0.f;
+    }
+  }
+}
+
+void launch_ragged_rows(float* caller, float* compact, const int32_t* perm, const int32_t* len, int len_div, int Bk,
+                        int S, int Sc, int pos, int width, int to_caller, cudaStream_t s) {
+  const int64_t words = ((int64_t)Sc * width + 3) / 4;
+  const unsigned per = (unsigned)std::min<int64_t>(64, std::max<int64_t>(1, (words + 255) / 256));
+  launch_k(ragged_rows_kernel, dim3(per, Bk), dim3(256), 0, s, caller, compact, perm, len, len_div, S, Sc, pos, width,
+           to_caller);
 }
 
 

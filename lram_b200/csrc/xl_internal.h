@@ -94,6 +94,29 @@ void launch_state_reset(float* C, float* n, float* m, float* conv, const uint8_t
                         int64_t c_per_env, int64_t n_per_env, int64_t m_per_env, int64_t conv_per_env,
                         cudaStream_t s);
 
+// Geometry of two state buffers of the same handle for the ragged prefill: [0] = the caller's state (B[0] envs),
+// [1] = the compact state (B[1] envs). Offsets are bytes within a block's slot (state_layout of xl_api.cu); *_env are
+// bytes per env of each part (s_env: per plane of the sLSTM's [4, B, d] planes).
+struct StateCopyGeom {
+  uint64_t slstm_mask;
+  int num_blocks;
+  int B[2];
+  size_t layer_bytes[2], slayer_bytes[2];
+  size_t c_off[2], n_off[2], m_off[2], conv_off[2], s_off[2], sconv_off[2];
+  size_t c_env, n_env, m_env, conv_env, s_env, sconv_env;
+};
+// Every part of every block of env perm[k] of the caller's state <-> env k of the compact state, k < Bc.
+// to_caller = 0: gather (caller -> compact); 1: scatter (compact -> caller). One launch, 128-bit accesses where a part's
+// per-env size allows them.
+void launch_state_permute(void* caller, void* compact, const int32_t* perm, int Bc, const StateCopyGeom& g,
+                          int to_caller, cudaStream_t s);
+// Ragged prefill row gather / scatter of one chunk. Compact row (k, t), k < Bk, t < Sc, <-> caller row
+// (perm[k], pos + t) of a [*, S, width] buffer; n_k = clamp(len[k] / len_div - pos, 0, Sc) rows of env k are valid.
+// to_caller = 0: compact[k, t] = t < n_k ? caller[perm[k], pos + t] : 0 (pad rows zero-filled, the caller's never read);
+// 1: caller[perm[k], pos + t] = compact[k, t] for t < n_k only.
+void launch_ragged_rows(float* caller, float* compact, const int32_t* perm, const int32_t* len, int len_div, int Bk,
+                        int S, int Sc, int pos, int width, int to_caller, cudaStream_t s);
+
 // bulk L2 prefetch of [base, base+bytes) (side stream, plain launch; see xl_elementwise.cu)
 void launch_l2_prefetch(const void* base, size_t bytes, int num_sms, int evict_last, cudaStream_t s);
 
@@ -144,17 +167,20 @@ void launch_repack_qkv(const float* qkv, float* qk, float* v, int M, int inner, 
 
 // ---- xl_slstm.cu ---------------------------------------------------------------------------------
 // sLSTM block (xLSTM[a:b] stacks). Rows ordered [env][token], T tokens per env; DHs = d / NH.
+// Ragged prefill (len != nullptr): env b of the launch has n_b = clamp(len[b] - pos, 0, T) real tokens; the tokens
+// after them are identity pads that change no state (len == nullptr: all T tokens are real).
 // conv step over the T tokens + swish: xc [M,d]; conv_state [B,KS,d] in/out. false: KS not instantiated
 bool launch_slstm_conv(const float* xn, float* conv_state, const float* cw, const float* cb, float* xc, int B,
-                       int T, int d, int KS, cudaStream_t s);
+                       int T, int d, int KS, cudaStream_t s, const int32_t* len = nullptr, int pos = 0);
 // pre [M,4,d] (gate-major i,f,z,o) = bias + headwise projections (i,f from xc; z,o from xn); W_* [NH,DHs,DHs],
 // bias [NH,4,DHs]
 void launch_slstm_gates(const float* xc, const float* xn, const float* w_i, const float* w_f, const float* w_z,
                         const float* w_o, const float* bias, float* pre, int M, int d, int NH, cudaStream_t s);
 // token t of every env: raw = pre + R y_{t-1}, pointwise update of (c,n,m) in st [4,stB,d] (st points at the
-// slice's first env, B envs processed); y -> y_out [M,d]
+// slice's first env, B envs processed); y -> y_out [M,d]. A pad token (t >= n_b) leaves (c,n,m) alone and carries
+// y_{t-1} into its y_out row, so that slstm_out stores the y of the env's last real token.
 cudaError_t launch_slstm_cell(const float* pre, const float* R, float* st, float* y_out, int B, int stB, int T, int t,
-                              int d, int NH, cudaStream_t s);
+                              int d, int NH, cudaStream_t s, const int32_t* len = nullptr, int pos = 0);
 // x += MultiHeadLayerNorm(y_out) (gamma = 1 + w); st_y [B,d] <- y of each env's last token
 void launch_slstm_out(const float* y_out, const float* gn_w, float* x, float* st_y, int M, int T, int d, int NH,
                       float eps, cudaStream_t s);
@@ -164,15 +190,20 @@ void launch_ffn_gate(const float* up, float* out, void* hi, void* lo, int M, int
 // ---- xl_prefill.cu -------------------------------------------------------------------------------
 // Sequence (context prefill) versions of the per-block kernels; rows are ordered [env][token] with S tokens
 // per env. S % 8 == 0.
+// Ragged prefill (len != nullptr, the chunk starting at token pos of the context): env b has n_b = clamp(len[b] - pos,
+// 0, S) real tokens, then identity pads (lf = 0, i~ = -inf: f = 1, i = 0, m carried, so every cell leaves C and n as
+// they are). Every env of such a launch has n_b >= 1. len == nullptr: all S tokens are real, results as before.
 bool prefill_cell_supported(int DH);
-// conv + SiLU + q/k/v + gate partials over the chunk, then conv_state <- last KS inputs. p.qk receives the q
-// plane [M, inner] followed by the k plane [M, inner] (M = B*S). false: no instantiation
-bool launch_conv_qkv_gates_seq(const ConvQkvParams& p, int S, cudaStream_t s);
+// conv + SiLU + q/k/v + gate partials over the chunk, then conv_state <- last KS inputs (ragged: the last KS rows of
+// the old window followed by the env's n_b inputs). p.qk receives the q plane [M, inner] followed by the k plane
+// [M, inner] (M = B*S). false: no instantiation
+bool launch_conv_qkv_gates_seq(const ConvQkvParams& p, int S, cudaStream_t s, const int32_t* len = nullptr,
+                               int pos = 0);
 // m/f/i per token ([B*NH][S] each) from the gate partials; m_state [B*NH] in/out; scratch: gate_scan_seq_scratch_floats()
 size_t gate_scan_seq_scratch_floats(int B, int S, int NH);
 void launch_gate_scan_seq(const float* gate_part, const float* igate_b, const float* fgate_b, float* m_state,
                           float* fseq, float* iseq, float* mseq, float* scratch, int B, int S, int NH, int NCH,
-                          cudaStream_t s);
+                          cudaStream_t s, const int32_t* len = nullptr, int pos = 0);
 // C / n advanced over the S tokens on chip; num [B*S, inner] = q^T C, qn [B*S, NH] = q.n per token
 cudaError_t launch_cell_seq(float* C, float* n, const float* q, const float* k, const float* v, const float* fseq,
                             const float* iseq, float* num, float* qn, int B, int S, int NH, int DH, int inner,

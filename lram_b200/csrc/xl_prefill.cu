@@ -527,11 +527,35 @@ __global__ void __launch_bounds__(64 * kConvRuns, 2) conv_qkv_gates_seq2_kernel(
 }
 
 // new conv_state = the last KS x_m rows of the chunk (S >= KS): separate kernel, because the first token run of
-// the conv kernel still reads the old window while its last run would overwrite it
+// the conv kernel still reads the old window while its last run would overwrite it.
+// Ragged (len != nullptr): one thread per (env, 4-channel group) takes the last KS rows of (old window ++ the env's n_b
+// valid rows) -- old rows still count when n_b < KS -- and reads all of them before it writes.
 __global__ void __launch_bounds__(256) conv_state_seq_kernel(const float* __restrict__ u, float* __restrict__ conv_state,
-                                                             int B, int S, int KS, int inner) {
+                                                             int B, int S, int KS, int inner,
+                                                             const int32_t* __restrict__ len, int pos) {
   pdl_wait();
   pdl_trigger();
+  if (len) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (int64_t)B * (inner >> 2)) return;
+    const int c4 = (int)(i % (inner >> 2));
+    const int b = (int)(i / (inner >> 2));
+    const int nb = min(max(len[b] - pos, 0), S);
+    float4 w[4];                                           // KS <= 4
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+      if (r >= KS) break;
+      const int idx = nb - KS + r;                         // chunk row, or (< 0) row KS + idx of the old window
+      w[r] = idx >= 0 ? reinterpret_cast<const float4*>(u + ((int64_t)b * S + idx) * 2 * inner)[c4]
+                      : reinterpret_cast<const float4*>(conv_state + ((int64_t)b * KS + KS + idx) * inner)[c4];
+    }
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {
+      if (r >= KS) break;
+      reinterpret_cast<float4*>(conv_state + ((int64_t)b * KS + r) * inner)[c4] = w[r];
+    }
+    return;
+  }
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t n4 = (int64_t)B * KS * (inner >> 2);
   if (i >= n4) return;
@@ -587,7 +611,7 @@ __global__ void __launch_bounds__(kScanThreads) gate_pre_seq_kernel(const float*
                                                                     const float* __restrict__ m_state,
                                                                     float* __restrict__ fseq, float* __restrict__ iseq,
                                                                     float* __restrict__ scratch, int B, int S, int NH,
-                                                                    int NCH) {
+                                                                    int NCH, const int32_t* __restrict__ len, int pos) {
   __shared__ float s_ig[kSuper + 32], s_lf[kSuper + 32];
   pdl_wait();
   pdl_trigger();
@@ -597,6 +621,7 @@ __global__ void __launch_bounds__(kScanThreads) gate_pre_seq_kernel(const float*
   const float bi = igate_b ? igate_b[hd] : 0.f, bf = fgate_b ? fgate_b[hd] : 0.f;
   const int s0 = sp * kSuper;
   const int cnt = min(kSuper, S - s0);
+  const int nreal = len ? len[b] - pos - s0 : cnt;   // tokens u >= nreal of the super-chunk are identity pads
   for (int u = tid; u < cnt; u += kScanThreads) {
     const float* gp = gate_part + ((int64_t)b * S + s0 + u) * NCH * 2 * NH + hd;
     float si = 0.f, sf = 0.f;
@@ -604,7 +629,11 @@ __global__ void __launch_bounds__(kScanThreads) gate_pre_seq_kernel(const float*
       si += gp[c * 2 * NH];
       sf += gp[c * 2 * NH + NH];
     }
-    const float ig = si + bi, lf = log_sigmoid(sf + bf);
+    float ig = si + bi, lf = log_sigmoid(sf + bf);
+    if (u >= nreal) {                           // m' = max(m, -inf) = m, f = exp(0) = 1, i = exp(-inf) = 0 exactly
+      ig = -INFINITY;
+      lf = 0.f;
+    }
     s_ig[u] = ig;
     s_lf[u] = lf;
     const int64_t o = (int64_t)bh * S + s0 + u;
@@ -1056,7 +1085,7 @@ static bool launch_conv_seq2(const ConvQkvParams& p, int S, int run, dim3 grid, 
   return launch_k(pf::conv_qkv_gates_seq2_kernel<NH, false>, grid, block, smem, s, p, S, run) == cudaSuccess;
 }
 
-bool launch_conv_qkv_gates_seq(const ConvQkvParams& p, int S, cudaStream_t s) {
+bool launch_conv_qkv_gates_seq(const ConvQkvParams& p, int S, cudaStream_t s, const int32_t* len, int pos) {
   const int nblk = p.inner / 4;
   const int per_chunk = (nblk + p.NCH - 1) / p.NCH;
   const int threads = ((per_chunk + 31) / 32) * 32;
@@ -1083,9 +1112,9 @@ bool launch_conv_qkv_gates_seq(const ConvQkvParams& p, int S, cudaStream_t s) {
   } else {
     return false;
   }
-  const int64_t n4 = (int64_t)p.B * p.KS * (p.inner / 4);
+  const int64_t n4 = (int64_t)p.B * (len ? 1 : p.KS) * (p.inner / 4);
   launch_k(pf::conv_state_seq_kernel, dim3((unsigned)((n4 + 255) / 256)), dim3(256), 0, s, p.u, p.conv_state, p.B, S,
-           p.KS, p.inner);
+           p.KS, p.inner, len, pos);
   return true;
 }
 
@@ -1095,10 +1124,10 @@ size_t gate_scan_seq_scratch_floats(int B, int S, int NH) {
 
 void launch_gate_scan_seq(const float* gate_part, const float* igate_b, const float* fgate_b, float* m_state,
                           float* fseq, float* iseq, float* mseq, float* scratch, int B, int S, int NH, int NCH,
-                          cudaStream_t s) {
+                          cudaStream_t s, const int32_t* len, int pos) {
   const dim3 grid(B * NH, (S + pf::kSuper - 1) / pf::kSuper);
   launch_k(pf::gate_pre_seq_kernel, grid, dim3(pf::kScanThreads), 0, s, gate_part, igate_b, fgate_b,
-           (const float*)m_state, fseq, iseq, scratch, B, S, NH, NCH);
+           (const float*)m_state, fseq, iseq, scratch, B, S, NH, NCH, len, pos);
   launch_k(pf::gate_scan_seq_kernel, grid, dim3(pf::kScanThreads), 0, s, m_state, fseq, iseq, mseq,
            (const float*)scratch, B, S, NH);
 }

@@ -16,7 +16,8 @@ namespace xl {
 template <int KS>
 __global__ void slstm_conv_kernel(const float* __restrict__ xn, float* __restrict__ conv_state,
                                   const float* __restrict__ cw, const float* __restrict__ cb,
-                                  float* __restrict__ xc, int B, int T, int d) {
+                                  float* __restrict__ xc, int B, int T, int d, const int32_t* __restrict__ len,
+                                  int pos) {
   pdl_wait();
   pdl_trigger();
   const int c = blockIdx.x * blockDim.x + threadIdx.x;
@@ -29,7 +30,9 @@ __global__ void slstm_conv_kernel(const float* __restrict__ xn, float* __restric
     win[k] = conv_state[((size_t)b * KS + k) * d + c];
   }
   const float bias = cb[c];
-  for (int t = 0; t < T; ++t) {
+  const int nb = len ? min(max(len[b] - pos, 0), T) : T;   // ragged prefill: tokens t >= nb are pads (window kept)
+  for (int t = nb; t < T; ++t) xc[((size_t)b * T + t) * d + c] = 0.f;
+  for (int t = 0; t < nb; ++t) {
 #pragma unroll
     for (int k = 0; k + 1 < KS; ++k) win[k] = win[k + 1];
     win[KS - 1] = xn[((size_t)b * T + t) * d + c];
@@ -44,12 +47,12 @@ __global__ void slstm_conv_kernel(const float* __restrict__ xn, float* __restric
 }
 
 bool launch_slstm_conv(const float* xn, float* conv_state, const float* cw, const float* cb, float* xc, int B,
-                       int T, int d, int KS, cudaStream_t s) {
+                       int T, int d, int KS, cudaStream_t s, const int32_t* len, int pos) {
   dim3 grid((d + 127) / 128, B), block(128);
   switch (KS) {
-    case 2: launch_k(slstm_conv_kernel<2>, grid, block, 0, s, xn, conv_state, cw, cb, xc, B, T, d); break;
-    case 3: launch_k(slstm_conv_kernel<3>, grid, block, 0, s, xn, conv_state, cw, cb, xc, B, T, d); break;
-    case 4: launch_k(slstm_conv_kernel<4>, grid, block, 0, s, xn, conv_state, cw, cb, xc, B, T, d); break;
+    case 2: launch_k(slstm_conv_kernel<2>, grid, block, 0, s, xn, conv_state, cw, cb, xc, B, T, d, len, pos); break;
+    case 3: launch_k(slstm_conv_kernel<3>, grid, block, 0, s, xn, conv_state, cw, cb, xc, B, T, d, len, pos); break;
+    case 4: launch_k(slstm_conv_kernel<4>, grid, block, 0, s, xn, conv_state, cw, cb, xc, B, T, d, len, pos); break;
     default: return false;
   }
   return true;
@@ -126,7 +129,8 @@ void launch_slstm_gates(const float* xc, const float* xn, const float* w_i, cons
 constexpr int kCO = 32, kCE = 8, kCS = 8;
 __global__ void __launch_bounds__(256) slstm_cell_kernel(const float* __restrict__ pre, const float* __restrict__ R,
                                                          float* __restrict__ st, float* __restrict__ y_out,
-                                                         int B, int stB, int T, int t, int d, int NH, int DH) {
+                                                         int B, int stB, int T, int t, int d, int NH, int DH,
+                                                         const int32_t* __restrict__ len, int pos) {
   extern __shared__ float smem[];
   float* sy = smem;                         // [kCE][DH]
   float* red = smem + kCE * DH;             // [kCS][kCE][4][kCO]
@@ -169,8 +173,12 @@ __global__ void __launch_bounds__(256) slstm_cell_kernel(const float* __restrict
   // thread (e = ds, o): fixed-order sum over the 8 slices, then the pointwise update of element (b, h*DH + o0 + o)
   const int e = ds, b = b0 + e;
   if (b >= B || !o_ok) return;
-  float raw[4];
   const int ch = h * DH + o0 + o;
+  if (len && t >= len[b] - pos) {               // ragged prefill pad: state kept, y_{t-1} carried forward
+    y_out[((size_t)b * T + t) * d + ch] = sy[e * DH + o0 + o];
+    return;
+  }
+  float raw[4];
 #pragma unroll
   for (int g = 0; g < 4; ++g) {
     float s = 0.f;
@@ -195,12 +203,12 @@ __global__ void __launch_bounds__(256) slstm_cell_kernel(const float* __restrict
 }
 
 cudaError_t launch_slstm_cell(const float* pre, const float* R, float* st, float* y_out, int B, int stB, int T, int t,
-                              int d, int NH, cudaStream_t s) {
+                              int d, int NH, cudaStream_t s, const int32_t* len, int pos) {
   const int DH = d / NH;
   const size_t smem = sizeof(float) * ((size_t)kCE * DH + (size_t)kCS * kCE * 4 * kCO);
   if (cudaError_t e = ensure_dyn_smem<&slstm_cell_kernel>(smem); e != cudaSuccess) return e;
   dim3 grid((DH + kCO - 1) / kCO, NH, (B + kCE - 1) / kCE);
-  return launch_k(slstm_cell_kernel, grid, dim3(256), smem, s, pre, R, st, y_out, B, stB, T, t, d, NH, DH);
+  return launch_k(slstm_cell_kernel, grid, dim3(256), smem, s, pre, R, st, y_out, B, stB, T, t, d, NH, DH, len, pos);
 }
 
 // ---- MultiHeadLayerNorm(y) -> residual add; carries y of the last token into the state -----------

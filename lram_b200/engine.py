@@ -16,6 +16,7 @@ import functools
 import math
 from typing import Dict, Optional
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -182,6 +183,25 @@ def sampling_params(cfg: XLSTMPolicyConfig, temperature: float = 1.0, top_k: int
                         env_id_stride=int(env_id_stride), seed=int(seed))
 
 
+def check_lengths(lengths, B: int, S: int, what: str = "S") -> np.ndarray:
+    """Per-env context lengths of a ragged prefill as the library takes them (a host int32 [B] array): a sequence, an
+    ndarray or a CPU integer tensor of B values in [0, S]. Raises ValueError otherwise."""
+    if isinstance(lengths, torch.Tensor):
+        if lengths.device.type != "cpu":
+            raise ValueError(f"lengths must be on the host, got a tensor on {lengths.device}")
+        if lengths.dtype.is_floating_point or lengths.dtype.is_complex or lengths.dtype == torch.bool:
+            raise ValueError(f"lengths must be integers, got {lengths.dtype}")
+        lengths = lengths.numpy()
+    arr = np.asarray(lengths)
+    if arr.ndim != 1 or arr.shape[0] != B:
+        raise ValueError(f"lengths must hold one value per env ({B}), got shape {arr.shape}")
+    if arr.dtype == np.bool_ or not np.issubdtype(arr.dtype, np.integer):
+        raise ValueError(f"lengths must be integers, got dtype {arr.dtype}")
+    if (arr < 0).any() or (arr > S).any():
+        raise ValueError(f"lengths must lie in [0, {what}={S}], got min {arr.min()} max {arr.max()}")
+    return np.ascontiguousarray(arr, dtype=np.int32)
+
+
 def _on_device(fn):
     """Run an engine method with the engine's GPU as the current CUDA device: the handle, its workspace, its streams
     and the per-device kernel attributes all belong to `self.device`, whatever device the caller has current."""
@@ -295,22 +315,40 @@ class XLSTMEngine:
                                          mode, flags, self._stream()))
         return out
 
-    @_on_device
-    def prefill(self, state: StateCache, x: torch.Tensor, want_hidden: bool = True, flags: int = 0):
+    def prefill(self, state: StateCache, x: torch.Tensor, want_hidden: bool = True, flags: int = 0, lengths=None):
         """Context prefill of the encoder: x [B,S,d] fp32 cuda (embedded tokens) -> last_hidden_state [B,S,d]
-        (or None); state advanced by S tokens, exactly as S recurrent steps would (xl_prefill)."""
+        (or None); state advanced by S tokens, exactly as S recurrent steps would (xl_prefill).
+        `lengths` (B ints in [0, S]: sequence, ndarray or CPU tensor): env b advances by its first lengths[b] tokens
+        only, an env with 0 keeps its state, rows from lengths[b] on are never read and come back as 0
+        (xl_prefill_ragged). Checked before anything reaches the library."""
+        lens = None if lengths is None else check_lengths(lengths, state.B, x.shape[1], "S")
+        return self._prefill(state, x, want_hidden, flags, lens)
+
+    @_on_device
+    def _prefill(self, state, x, want_hidden, flags, lens):
         assert x.is_cuda and x.dtype == torch.float32 and x.dim() == 3 and x.shape[0] == state.B
         x = x.contiguous()
         out = torch.empty_like(x) if want_hidden else None
-        L.check(self.lib.xl_prefill(self.handle, _ptr(state.buf), _ptr(x), _ptr(out), x.shape[0], x.shape[1], flags,
-                                    self._stream()))
+        if lens is None:
+            L.check(self.lib.xl_prefill(self.handle, _ptr(state.buf), _ptr(x), _ptr(out), x.shape[0], x.shape[1],
+                                        flags, self._stream()))
+        else:
+            L.check(self.lib.xl_prefill_ragged(self.handle, _ptr(state.buf), _ptr(x), _ptr(out),
+                                               lens.ctypes.data_as(C.c_void_p), x.shape[0], x.shape[1], flags,
+                                               self._stream()))
         return out
 
-    @_on_device
     def policy_prefill(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,
-                       rewards: Optional[torch.Tensor] = None, flags: int = 0):
+                       rewards: Optional[torch.Tensor] = None, flags: int = 0, lengths=None):
         """Warm the recurrent state with Tn timesteps of context per env: states [B,Tn,state_dim], rtg [B,Tn],
-        rewards [B,Tn] or None (= the 0 placeholder the rollout feeds). No action outputs (xl_policy_prefill)."""
+        rewards [B,Tn] or None (= the 0 placeholder the rollout feeds). No action outputs (xl_policy_prefill).
+        `lengths` (B ints in [0, Tn]): env b takes its first lengths[b] timesteps only, an env with 0 keeps its state
+        (xl_policy_prefill_ragged). Checked before anything reaches the library."""
+        lens = None if lengths is None else check_lengths(lengths, state.B, states.shape[1], "Tn")
+        return self._policy_prefill(state, states, rtg, rewards, flags, lens)
+
+    @_on_device
+    def _policy_prefill(self, state, states, rtg, rewards, flags, lens):
         cfg = self.cfg
         B, Tn = state.B, states.shape[1]
         assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == (B, Tn, cfg.state_dim)
@@ -319,8 +357,13 @@ class XLSTMEngine:
         if rewards is not None:
             rewards = rewards.to(self.device, torch.float32).contiguous()
             assert rewards.numel() == B * Tn
-        L.check(self.lib.xl_policy_prefill(self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards), B, Tn,
-                                           flags, self._stream()))
+        if lens is None:
+            L.check(self.lib.xl_policy_prefill(self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards), B,
+                                               Tn, flags, self._stream()))
+        else:
+            L.check(self.lib.xl_policy_prefill_ragged(self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg),
+                                                      _ptr(rewards), lens.ctypes.data_as(C.c_void_p), B, Tn, flags,
+                                                      self._stream()))
 
     @_on_device
     def policy_step(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,

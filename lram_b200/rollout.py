@@ -21,7 +21,7 @@ import numpy as np
 import torch
 
 from . import _lib as L
-from .engine import XLSTMEngine
+from .engine import XLSTMEngine, check_lengths
 
 
 def shard_env_ids(n_envs: int, rank: int, world_size: int) -> List[int]:
@@ -185,16 +185,28 @@ class BatchedRollout:
         self.rtg0 = np.asarray(envs.rtg0, dtype=np.float32)
         self.scale = np.asarray(envs.reward_scale, dtype=np.float32)
 
-    def prefill_context(self, states, rtg, rewards=None) -> None:
-        """Warm the recurrent state of every env with a context of Tn earlier timesteps before the rollout starts —
-        the batched counterpart of `persist_context` (src/callbacks/evaluation.py:213-237), where the reference keeps
-        the previous episodes' tokens in front of the new episode: states [B, Tn, state_dim], rtg [B, Tn], rewards
-        [B, Tn] or None (the 0 placeholder the rollout feeds). One chunkwise-parallel pass (`xl_policy_prefill`) leaves
-        the state exactly where Tn recurrent env steps would. Follow with `run(..., keep_state=True)`."""
+    def prefill_context(self, states, rtg, rewards=None, lengths=None) -> None:
+        """Warm the recurrent state with a context of earlier timesteps before the rollout starts — the batched
+        counterpart of `persist_context` (src/callbacks/evaluation.py:213-237), where the reference keeps the previous
+        episodes' tokens in front of the new episode: states [B, Tn, state_dim], rtg [B, Tn], rewards [B, Tn] or None
+        (the 0 placeholder the rollout feeds). Follow with `run(..., keep_state=True)`.
+
+        lengths=None: every env is reset and takes all Tn timesteps; one chunkwise-parallel pass (`xl_policy_prefill`)
+        leaves the state exactly where Tn recurrent env steps would. lengths (B ints in [0, Tn]; histories of different
+        lengths, e.g. episodes that ended at different times): only the envs with lengths[b] > 0 are reset, each then
+        takes its own first lengths[b] timesteps (`xl_policy_prefill_ragged`); envs with 0 keep their state, so a few
+        envs of a running batch can be re-primed without touching the others."""
+        lens = None
+        if lengths is not None:
+            Tn = (states.shape if hasattr(states, "shape") else np.shape(states))[1]
+            lens = check_lengths(lengths, self.B, Tn, "Tn")
         dev = self.engine.device
         to = lambda a: None if a is None else torch.as_tensor(np.ascontiguousarray(a), dtype=torch.float32).to(dev)  # noqa: E731
-        self.engine.reset(self.state)
-        self.engine.policy_prefill(self.state, to(states), to(rtg), to(rewards))
+        if lens is None:
+            self.engine.reset(self.state)
+        else:
+            self.engine.reset(self.state, torch.from_numpy((lens > 0).astype(np.uint8)))
+        self.engine.policy_prefill(self.state, to(states), to(rtg), to(rewards), lengths=lens)
 
     def run(self, n_steps: int, record: bool = False, keep_state: bool = False) -> Dict[str, object]:
         envs, B = self.envs, self.B
