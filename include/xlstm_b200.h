@@ -275,7 +275,8 @@ int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B
 /* Same for the whole policy: Tn timesteps of context per env, states fp32 [B, Tn, state_dim], rtg fp32 [B, Tn],
  * rewards fp32 [B, Tn] or NULL (= 0). Embeds every timestep into its (s, rtg, r) tokens
  * (online_decision_transformer_model.py:522-530,588-612) and prefills the 3*Tn tokens; no action outputs
- * (a context only warms the state: src/callbacks/evaluation.py:213-237 `persist_context`). */
+ * (a context only warms the state: src/callbacks/evaluation.py:213-237 `persist_context`; xl_policy_forward below
+ * returns them). */
 int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
                       int Tn, unsigned flags, void* stream);
 
@@ -300,6 +301,47 @@ int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out
                       unsigned flags, void* stream);
 int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
                              const int32_t* lengths, int B, int Tn, unsigned flags, void* stream);
+
+/* Outputs of xl_policy_forward. Every pointer is device memory and nullable (NULL = not wanted). */
+typedef struct {
+  int32_t* tokens;          /* [B, Tn, act_dim]  argmax action tokens per timestep, as xl_policy_step's tokens      */
+  float* actions;           /* [B, Tn, act_dim]  as xl_policy_step's actions                                       */
+  float* logits;            /* [B, Tn, n_out]    n_out = act_dim * num_actions (discrete: num_actions)             */
+  const int32_t* targets;   /* [B, Tn, act_dim]  action tokens to score                                            */
+  float* logprobs;          /* [B, Tn, act_dim]  log-probability of targets; needs targets                         */
+} xl_seq_outputs;
+
+/* Sequence forward of the policy: the per-timestep action outputs of whole trajectories in one chunkwise pass. This is
+ * MultiDomainDiscreteDecisionXLSTMModel.forward(use_inference_cache=False) over [B, Tn] timesteps, every timestep read
+ * at its rtg token (SURVEY.md a10/a11), with the state advanced as xl_policy_prefill advances it.
+ *  - Inputs: those of xl_policy_prefill: states fp32 [B, Tn, state_dim], rtg fp32 [B, Tn], rewards fp32 [B, Tn] or NULL
+ *    (= 0). lengths NULL: every env has Tn timesteps; otherwise a HOST int32 [B] array of values in [0, Tn], as for
+ *    xl_policy_prefill_ragged.
+ *  - Outputs at (b, t), t < lengths[b]: what xl_policy_step returns at that timestep (sampler disarmed) when env b is
+ *    stepped from `state` over its timesteps 0..t. The logits agree to the error of the chunkwise prefill against
+ *    recurrent steps; tokens are equal except where the top two logits of a row are closer than that error. Timesteps
+ *    that run as eager steps (see below) are bit-identical to xl_policy_step.
+ *  - State after the call: bit-identical to xl_policy_prefill (lengths NULL) or xl_policy_prefill_ragged (lengths) on the
+ *    same arguments: the same kernels and chunks run, and the head only reads the residual stream.
+ *  - logprobs[b,t,j] = log_softmax(row)[targets[b,t,j]], in fp32 with the row maximum subtracted. The row is the one the
+ *    sampler draws from: row j of the [act_dim, num_actions] logit block (discrete: all num_actions logits of the env,
+ *    not only the discrete_actions the argmax reads; column 0 only). A target < 0 gives 0 (padded action dims past an env's own act_dim); a target >= num_actions gives NaN.
+ *  - XL_FLAG_DISCRETE: the token rule and column meaning of xl_policy_step (argmax over the first discrete_actions logits,
+ *    actions = (float)token) in column 0; columns >= 1 of tokens / actions / logprobs hold -1 / 0 / 0.
+ *  - Past an env's length (t >= lengths[b]): tokens -1, actions, logits and logprobs 0. Inputs there are never read. An
+ *    env with length 0 keeps every byte of its state slot.
+ *  - Always the argmax: the armed sampler is not used, and neither its step counter nor the token ring slot advances
+ *    (as xl_policy_prefill).
+ *  - Chunk flow: per chunk of the prefill, post_blocks_norm of the rtg-token rows only (as the head's bf16 operand
+ *    planes), the action head as one tcgen05 Linear over the chunk's timesteps into a library-owned logits workspace
+ *    (grow-only, chunk timesteps x n_out floats, freed by xl_destroy; growing it synchronises the device), then one
+ *    reduction kernel per chunk: argmax, inv_tokenize, log-sum-exp and the scatter to [B, Tn, ...]. The last
+ *    Tn mod 8 timesteps of a uniform call (all of them on shapes without the sequence path) run as eager policy steps.
+ *  - XL_ERR_INVALID_ARG: out NULL, logprobs without targets, and the checks of xl_policy_prefill(_ragged).
+ *    XL_ERR_UNSUPPORTED: XL_FLAG_STATE_EMBEDS; lengths that are neither all Tn nor all 0 on shapes without the sequence
+ *    path (as xl_policy_prefill_ragged; state and outputs untouched). Not graph-capturable. */
+int xl_policy_forward(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
+                      const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out, unsigned flags, void* stream);
 
 /* out[M,N] = A[M,K] @ W[N,K]^T (+ bias[N]) (+ residual[M,N]); A fp32, W bf16, fp32 accumulate.
  * The nn.Linear of proj_up / proj_down / embed_state / action_net. impl: 0 auto, 1 CUDA-core, 2 tcgen05. */

@@ -55,6 +55,12 @@ class XLSampling(C.Structure):
                 ("env_id_stride", C.c_int32), ("seed", C.c_uint64)]
 
 
+class XLSeqOutputs(C.Structure):
+    """xl_seq_outputs: device buffers of xl_policy_forward (each nullable)."""
+    _fields_ = [("tokens", C.c_void_p), ("actions", C.c_void_p), ("logits", C.c_void_p), ("targets", C.c_void_p),
+                ("logprobs", C.c_void_p)]
+
+
 class XLError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"xlstm_b200 error {code}: {msg}")
@@ -121,6 +127,8 @@ def load():
     lib.xl_prefill_ragged.restype = i32
     lib.xl_policy_prefill_ragged.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, u32, vp]
     lib.xl_policy_prefill_ragged.restype = i32
+    lib.xl_policy_forward.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, C.POINTER(XLSeqOutputs), u32, vp]
+    lib.xl_policy_forward.restype = i32
     lib.xl_linear.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
     lib.xl_linear.restype = i32
     lib.xl_set_token_ring.argtypes = [vp, vp, i32, i32, vp]

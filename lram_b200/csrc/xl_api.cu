@@ -144,6 +144,9 @@ struct xl_handle {
   size_t rg_state_bytes = 0;
   int32_t* rg_idx = nullptr;                    // device, 2 * max_batch
   std::vector<int32_t> rg_host;
+  // sequence forward (xl_policy_forward): logits of one chunk's timesteps [rows, n_out] (grow-only)
+  float* sq_logits = nullptr;
+  size_t sq_logits_floats = 0;
   int prefill_gemm_2cta = 0;                    // A/B: shallow-ring Linear tiles, two CTAs per SM        ("prefill_gemm_2cta")
   int prefill_rows = 16384;                     // rows (envs x tokens) per prefill chunk                  ("prefill_rows")
   char* pf_tc = nullptr;                        // workspace of the tcgen05 chunkwise cell (grow-only)
@@ -1165,6 +1168,84 @@ int ragged_chunks(xl_handle* h, const std::vector<int32_t>& len, int T, std::vec
   return ensure_prefill_ws(h, rows);
 }
 
+// ---- sequence forward: the head hook of the policy-prefill loops --------------------------------------------------
+// With a hook, the loops also emit the action outputs of every timestep (xl_policy_forward); without one they are
+// xl_policy_prefill / xl_policy_prefill_ragged unchanged. The hook only reads what the loops leave behind.
+struct SeqHead {
+  xl_seq_outputs out;
+  int discrete, n_out, Tn;
+};
+
+int ensure_seq_logits(xl_handle* h, size_t floats) {
+  if (floats <= h->sq_logits_floats) return XL_OK;
+  XL_CUDA(cudaDeviceSynchronize());            // nothing may still be using the old workspace
+  if (h->sq_logits) cudaFree(h->sq_logits);
+  h->sq_logits = nullptr;
+  h->sq_logits_floats = 0;
+  cudaError_t e = cudaMalloc((void**)&h->sq_logits, sizeof(float) * floats);
+  if (e != cudaSuccess)
+    return fail(XL_ERR_CUDA, "cudaMalloc(sequence logits %zu B) failed: %s", sizeof(float) * floats, cudaGetErrorString(e));
+  h->sq_logits_floats = floats;
+  return XL_OK;
+}
+
+// tokens / actions / logprobs / logits of `rows` timesteps whose logits sit in sq_logits (see xl::SeqHeadParams)
+void seq_head_reduce(xl_handle* h, const SeqHead& hd, int rows, int Tc, int pos, const int32_t* perm,
+                     const int32_t* len, cudaStream_t s) {
+  const xl_config& c = h->cfg;
+  xl::SeqHeadParams p;
+  p.logits = h->sq_logits;
+  p.rows = rows; p.Tc = Tc; p.pos = pos; p.Tn = hd.Tn;
+  p.n_out = hd.n_out; p.act_dim = c.act_dim; p.num_actions = h->num_actions; p.discrete_actions = c.discrete_actions;
+  p.discrete = hd.discrete;
+  p.bin_width = hd.discrete ? 0.f : (c.tok_max_val - c.tok_min_val) / (float)c.action_channels;
+  p.min_val = hd.discrete ? 0.f : c.tok_min_val;
+  p.perm = perm; p.len = len; p.len_div = c.tokens_per_step;
+  p.tokens = hd.out.tokens; p.actions = hd.out.actions; p.out_logits = hd.out.logits;
+  p.targets = hd.out.targets; p.logprobs = hd.out.logprobs;
+  xl::launch_seq_head(p, s);
+  h->launches += 1;
+}
+
+// Head of one prefill chunk of Bk envs x Tc timesteps, after prefill_blocks: post_blocks_norm of the rtg-token rows of
+// pf_x only (complete there: the prefill's proj_down leaves no split-K planes), emitted as the head's bf16 operand planes
+// where the tcgen05 Linear runs; the head Linear over the chunk's Bk*Tc timesteps into sq_logits; the reduction.
+int seq_head_chunk(xl_handle* h, const SeqHead& hd, int Bk, int Tc, int pos, const int32_t* perm, const int32_t* len,
+                   unsigned flags, cudaStream_t s) {
+  const xl_config& c = h->cfg;
+  const int d = c.embedding_dim, T = c.tokens_per_step, rows = Bk * Tc;
+  const Ws ws = prefill_ws(h);
+  const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
+  auto PW = [&](int id) { return h->pw[id - XL_W_POST_NORM]; };
+  const float* post_w = (const float*)PW(XL_W_POST_NORM);
+  int rc = ensure_seq_logits(h, (size_t)rows * hd.n_out);
+  if (rc) return rc;
+  const bool tc = impl != 1 && xl::gemm_tc_supported(rows, hd.n_out, d) && (size_t)rows * d <= ws.a_cap && d <= 4096;
+  if (tc)
+    xl::launch_ln_rows_gather(ws.x, nullptr, 1, 0, post_w, c.ln_eps, rows, d, T, c.action_token_pos, ws.a_hi, ws.a_lo, s);
+  else
+    xl::launch_ln_rows(ws.x + (size_t)c.action_token_pos * d, (int64_t)T * d, ws.xn, d, post_w, nullptr, 1, c.ln_eps,
+                       rows, d, nullptr, nullptr, s);
+  h->launches += 1;
+  rc = linear(h, ws, ws.xn, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, h->sq_logits, rows, hd.n_out, d,
+              impl, s, /*presplit=*/tc);
+  if (rc) return rc;
+  seq_head_reduce(h, hd, rows, Tc, pos, perm, len, s);
+  XL_CUDA(cudaGetLastError());
+  return XL_OK;
+}
+
+// Every output position of the call set to its past-the-length value (tokens -1, the rest 0): the ragged forward then
+// writes only the timesteps its envs have.
+int seq_clear_outputs(const xl_handle* h, const SeqHead& hd, int B, cudaStream_t s) {
+  const size_t pos = (size_t)B * hd.Tn, A = h->cfg.act_dim;
+  if (hd.out.tokens) XL_CUDA(cudaMemsetAsync(hd.out.tokens, 0xff, sizeof(int32_t) * pos * A, s));
+  if (hd.out.actions) XL_CUDA(cudaMemsetAsync(hd.out.actions, 0, sizeof(float) * pos * A, s));
+  if (hd.out.logprobs) XL_CUDA(cudaMemsetAsync(hd.out.logprobs, 0, sizeof(float) * pos * A, s));
+  if (hd.out.logits) XL_CUDA(cudaMemsetAsync(hd.out.logits, 0, sizeof(float) * pos * hd.n_out, s));
+  return XL_OK;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1303,6 +1384,7 @@ void xl_destroy(xl_handle* h) {
   if (h->pf_buf) cudaFree(h->pf_buf);
   if (h->rg_state) cudaFree(h->rg_state);
   if (h->rg_idx) cudaFree(h->rg_idx);
+  if (h->sq_logits) cudaFree(h->sq_logits);
   if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
   for (int k = 0; k < kMaxMicro - 1; ++k) {
     if (h->side[k]) cudaStreamDestroy(h->side[k]);
@@ -1745,8 +1827,9 @@ int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B
   return XL_OK;
 }
 
-int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
-                      int Tn, unsigned flags, void* stream) {
+// xl_policy_prefill; with a head hook (xl_policy_forward) also the action outputs of every timestep
+static int policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
+                          int Tn, unsigned flags, void* stream, const SeqHead* head) {
   int rc = check_batch(h, B);
   if (rc) return rc;
   if (!state || !states || !rtg) return fail(XL_ERR_INVALID_ARG, "null argument");
@@ -1792,10 +1875,13 @@ int xl_policy_prefill(xl_handle* h, void* state, const float* states, const floa
       h->launches += 1;
       rc = prefill_blocks(h, state, B, B, Tc * T, flags, s);
       if (rc) return rc;
+      if (head && (rc = seq_head_chunk(h, *head, B, Tc, pos, nullptr, nullptr, flags, s))) return rc;
       pos += Tc;
     }
   }
-  // remaining timesteps: ordinary fused policy steps, outputs discarded
+  // remaining timesteps: ordinary fused policy steps, outputs discarded (head hook: their logits are reduced as a chunk
+  // of one timestep)
+  if (head && pos < Tn && (rc = ensure_seq_logits(h, (size_t)B * head->n_out))) return rc;
   for (; pos < Tn; ++pos) {
     XL_CUDA(cudaMemcpy2DAsync(h->d_states, sizeof(float) * (size_t)sd, states + (size_t)pos * sd,
                               sizeof(float) * (size_t)Tn * sd, sizeof(float) * (size_t)sd, B, cudaMemcpyDeviceToDevice, s));
@@ -1806,12 +1892,18 @@ int xl_policy_prefill(xl_handle* h, void* state, const float* states, const floa
                                 cudaMemcpyDeviceToDevice, s));
     StepArgs a;
     a.state = state; a.states = h->d_states; a.rtg = h->d_rtg; a.rewards = rewards ? h->d_rew : nullptr;
-    a.tokens = h->d_tokens; a.actions = h->d_actions; a.logits = nullptr; a.hidden = nullptr;
+    a.tokens = h->d_tokens; a.actions = h->d_actions; a.logits = head ? h->sq_logits : nullptr; a.hidden = nullptr;
     a.B = B; a.mode = XL_MODE_FUSED; a.flags = (flags & ~(unsigned)XL_FLAG_GRAPH) | kFlagNoRing;
     rc = run_policy(h, a, s);
     if (rc) return rc;
+    if (head) seq_head_reduce(h, *head, B, 1, pos, nullptr, nullptr, s);
   }
   return XL_OK;
+}
+
+int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
+                      int Tn, unsigned flags, void* stream) {
+  return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, nullptr);
 }
 
 int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out, const int32_t* lengths, int B, int S,
@@ -1852,8 +1944,10 @@ int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out
   return ragged_end(h, state, B, p, s);
 }
 
-int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
-                             const int32_t* lengths, int B, int Tn, unsigned flags, void* stream) {
+// xl_policy_prefill_ragged; with a head hook (xl_policy_forward) also the action outputs of every timestep
+static int policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
+                                 const int32_t* lengths, int B, int Tn, unsigned flags, void* stream,
+                                 const SeqHead* head) {
   int rc = check_batch(h, B);
   if (rc) return rc;
   if (!state || !states || !rtg) return fail(XL_ERR_INVALID_ARG, "null argument");
@@ -1862,11 +1956,12 @@ int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, con
   rc = xl_weights_ready(h);
   if (rc) return rc;
   const int nfull = (int)std::count(lengths, lengths + B, Tn), nzero = (int)std::count(lengths, lengths + B, 0);
-  if (nfull == B) return xl_policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream);
-  if (nzero == B) return XL_OK;
-  if (!prefill_fast_path(h))
+  if (nfull == B) return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, head);
+  if (nzero < B && !prefill_fast_path(h))
     return fail(XL_ERR_UNSUPPORTED, "ragged prefill needs the sequence path (conv_kernel 4, a cell plan for DH=%d)", h->DH);
   cudaStream_t s = (cudaStream_t)stream;
+  if (head && (rc = seq_clear_outputs(h, *head, B, s))) return rc;
+  if (nzero == B) return XL_OK;
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim, sd = c.state_dim, T = c.tokens_per_step;
   const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
@@ -1896,9 +1991,31 @@ int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, con
     h->launches += 1;
     rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, Tc * T, flags, s, p.d_len, ch.pos * T);
     if (rc) return rc;
+    if (head && (rc = seq_head_chunk(h, *head, ch.Bk, Tc, ch.pos, p.d_perm, p.d_len, flags, s))) return rc;
     XL_CUDA(cudaGetLastError());
   }
   return ragged_end(h, state, B, p, s);
+}
+
+int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
+                             const int32_t* lengths, int B, int Tn, unsigned flags, void* stream) {
+  return policy_prefill_ragged(h, state, states, rtg, rewards, lengths, B, Tn, flags, stream, nullptr);
+}
+
+int xl_policy_forward(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
+                      const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out, unsigned flags, void* stream) {
+  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+  if (!out) return fail(XL_ERR_INVALID_ARG, "null outputs");
+  if (out->logprobs && !out->targets) return fail(XL_ERR_INVALID_ARG, "logprobs need targets");
+  if (flags & XL_FLAG_STATE_EMBEDS)
+    return fail(XL_ERR_UNSUPPORTED, "xl_policy_forward takes raw states (no state embeddings)");
+  SeqHead hd;
+  hd.out = *out;
+  hd.discrete = (flags & XL_FLAG_DISCRETE) ? 1 : 0;
+  hd.n_out = hd.discrete ? h->num_actions : h->head_out;
+  hd.Tn = Tn;
+  if (!lengths) return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, &hd);
+  return policy_prefill_ragged(h, state, states, rtg, rewards, lengths, B, Tn, flags, stream, &hd);
 }
 
 int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bias, const float* residual,

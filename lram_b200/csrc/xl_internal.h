@@ -117,6 +117,25 @@ void launch_state_permute(void* caller, void* compact, const int32_t* perm, int 
 void launch_ragged_rows(float* caller, float* compact, const int32_t* perm, const int32_t* len, int len_div, int Bk,
                         int S, int Sc, int pos, int width, int to_caller, cudaStream_t s);
 
+// ---- xl_seq_head.cu ------------------------------------------------------------------------------
+// Per-timestep head reduction of xl_policy_forward over the logits of one chunk: argmax token (warp_argmax), action,
+// log-probability of the target and a copy of the logit row, each written to its [B, Tn, ...] position.
+struct SeqHeadParams {
+  const float* logits;          // [rows, n_out] chunk rows: row r = timestep pos + r % Tc of compact env r / Tc
+  int rows, Tc, pos, Tn;
+  int n_out, act_dim, num_actions, discrete_actions, discrete;
+  float bin_width, min_val;
+  const int32_t* perm;          // compact env k -> caller env perm[k]; nullptr = identity
+  const int32_t* len;           // ragged: env k's valid timesteps are t < len[k] / len_div (others skipped); nullptr = all
+  int len_div;
+  int32_t* tokens;              // [B, Tn, act_dim] (nullable, as every output below)
+  float* actions;               // [B, Tn, act_dim]
+  float* out_logits;            // [B, Tn, n_out]
+  const int32_t* targets;       // [B, Tn, act_dim] (needed with logprobs)
+  float* logprobs;              // [B, Tn, act_dim]
+};
+void launch_seq_head(const SeqHeadParams& p, cudaStream_t s);
+
 // bulk L2 prefetch of [base, base+bytes) (side stream, plain launch; see xl_elementwise.cu)
 void launch_l2_prefetch(const void* base, size_t bytes, int num_sms, int evict_last, cudaStream_t s);
 

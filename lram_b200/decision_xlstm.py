@@ -128,7 +128,10 @@ def config_from_reference(hf_config, **policy_kwargs) -> XLSTMPolicyConfig:
 
 class FusedXLSTMEncoder(nn.Module):
     """Drop-in for `xLSTMEncoder` on the `use_cache=True` path: `forward(inputs_embeds=..., past_key_values=...,
-    use_cache=True)` returns `last_hidden_state` [B, n_tok, d] and the (opaque) `past_key_values`.
+    use_cache=True)` returns `last_hidden_state` [B, n_tok, d] and the (opaque) `past_key_values`. With
+    `use_cache=False` it returns the hidden states of every token from a zero state and `past_key_values=None` (the
+    reference's non-cache branch; `past_key_values` is not read there). Inputs that require grad with grad enabled raise
+    NotImplementedError: there is no training path.
 
     Construct it like the reference constructs its encoder, `FusedXLSTMEncoder(config=config)` with the policy's
     `xLSTMConfig` (or an `XLSTMPolicyConfig`): the parameters `layers.blocks.{i}....` / `layers.post_blocks_norm.weight`
@@ -229,14 +232,19 @@ class FusedXLSTMEncoder(nn.Module):
                 return_dict=None):
         if inputs_embeds is None:
             raise ValueError("xLSTM encoder consumes already embedded inputs (inputs_embeds)")
-        if not use_cache:
-            raise NotImplementedError("parallel (training) form is out of scope of the recurrent-inference path")
+        if not use_cache and torch.is_grad_enabled() and inputs_embeds.requires_grad:
+            raise NotImplementedError("training (autograd through the encoder) is out of scope of the inference path")
         engine = self.engine
         B = inputs_embeds.shape[0]
         if B > engine.max_batch and self._owns_engine and self._engine_provider is None:   # grow the workspace
             self.max_batch = B
             self.invalidate_engine()
             engine = self.engine
+        if not use_cache:
+            # the non-cache branch (decision_xlstm.py:166-167, xLSTMBlockStack.forward(x)): every token from a zero
+            # state, no cache kept or read; computed by the chunkwise prefill, which equals the parallel form
+            hs = engine.prefill(engine.new_state(B), inputs_embeds.detach().to(engine.device, torch.float32))
+            return _Output(last_hidden_state=hs, past_key_values=None, hidden_states=None, attentions=None)
         if past_key_values is None:
             cache = engine.new_state(B)                        # zeros == state None (m starts at 0)
         elif isinstance(past_key_values, StateCache):
@@ -286,6 +294,8 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
             `compute_inputs` does when the cache is warm (online_decision_transformer_model.py:466-470); on the cold
             first call the reference embeds all T but `handle_inference_cache` trims to the last 3 tokens
             (decision_xlstm.py:225-229), i.e. to the last timestep as well (pinned by tests/golden/ref_policy_forward/).
+    forward(..., use_inference_cache=False) is the reference's ordinary forward: outputs for all T timesteps from a zero
+            state, computed in one chunkwise pass (`_forward_sequence`).
 
     `state_dict` may be given at construction (then it is loaded straight away) or later through `load_state_dict`,
     the order the reference's agent uses; hot-path keys missing at the first call raise KeyError.
@@ -432,10 +442,10 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
                 attention_mask=None, output_hidden_states=None, output_attentions=None, return_dict=None,
                 deterministic=True, with_log_probs=False, prompt=None, task_id=None, ddp_kwargs=None,
                 context_trjs=None, inference_params=None, past_key_values=None, use_inference_cache=False):
-        if not use_inference_cache:
-            raise NotImplementedError("only the inference-cache (recurrent) path is implemented")
         if prompt is not None or context_trjs is not None:
             raise NotImplementedError("prompts / retrieval contexts are out of scope")
+        if not use_inference_cache:
+            return self._forward_sequence(states, actions, rewards, returns_to_go)
         cfg = self.cfg
         B = states.shape[0]
         engine = self.engine_for(B)
@@ -492,6 +502,39 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
                        action_logits=logits, action_tokens=tokens, past_key_values=cache,
                        state_preds=None, return_preds=None, reward_preds=None, action_log_probs=None,
                        hidden_states=None, attentions=None, entropy=None, prompt_infos=None, cross_attentions=None)
+
+    def _forward_sequence(self, states, actions, rewards, returns_to_go):
+        """`forward(use_inference_cache=False)`: the reference's ordinary forward over all T timesteps, each read at its
+        rtg token (SURVEY.md a10/a11), from a fresh zero state; no cache is kept (`past_key_values=None`). Runs as one
+        `XLSTMEngine.policy_forward`. Returns action_preds [B,T,A] (discrete [B,T,1]), action_logits [B,T,A,num_actions]
+        (discrete [B,T,1,num_actions]) and action_tokens. `last_hidden_state` is None: the sequence forward returns no
+        hidden states. `attention_mask` is not read, as the reference's encoder does not read it. Rewards None = 0."""
+        cfg = self.cfg
+        if states.dim() == 5 or (states.dim() == 3 and self.img_is_encoded and states.shape[-1] == cfg.d):
+            raise NotImplementedError("image observations are not implemented on the sequence forward")
+        if states.dim() != 3:
+            raise ValueError(f"states must be [B,T,{cfg.state_dim}], got {tuple(states.shape)}")
+        if states.shape[-1] != cfg.state_dim:
+            raise ValueError(f"states must be padded to {cfg.state_dim} (DecisionXLSTM.pad_inputs)")
+        B, T = states.shape[:2]
+        engine = self.engine_for(B)
+        dev = engine.device
+        discrete = bool(self.is_discrete and actions is not None and actions.shape[-1] == 1)
+        st = states.to(dev, torch.float32).contiguous()
+        rtg = returns_to_go.to(dev, torch.float32).reshape(B, T).contiguous()
+        rew = None if rewards is None else rewards.to(dev, torch.float32).reshape(B, T).contiguous()
+        out = engine.policy_forward(engine.new_state(B), st, rtg, rew, discrete=discrete, want_logits=True)
+        tokens = out["action_tokens"].to(torch.long)
+        if discrete:
+            action_preds = tokens[:, :, :1]
+            logits = out["action_logits"].view(B, T, 1, cfg.num_actions)
+        else:
+            action_preds = out["action_preds"]
+            logits = out["action_logits"].view(B, T, cfg.act_dim, cfg.num_actions)
+        return _Output(last_hidden_state=None, action_preds=action_preds, action_logits=logits, action_tokens=tokens,
+                       past_key_values=None, state_preds=None, return_preds=None, reward_preds=None,
+                       action_log_probs=None, hidden_states=None, attentions=None, entropy=None, prompt_infos=None,
+                       cross_attentions=None)
 
 
 def sample_from_logits(logits: torch.Tensor, temperature: float = 1.0, top_k: int = 0, top_p: float = 0.5):

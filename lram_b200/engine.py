@@ -365,6 +365,65 @@ class XLSTMEngine:
                                                       _ptr(rewards), lens.ctypes.data_as(C.c_void_p), B, Tn, flags,
                                                       self._stream()))
 
+    def policy_forward(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,
+                       rewards: Optional[torch.Tensor] = None, lengths=None, discrete: bool = False,
+                       targets: Optional[torch.Tensor] = None, want_logits: bool = False) -> dict:
+        """Action outputs of every timestep of whole trajectories in one chunkwise pass (xl_policy_forward): what
+        `policy_step` would return at each timestep when stepped from `state` over states [B,Tn,state_dim], rtg [B,Tn],
+        rewards [B,Tn] or None (= 0). The state ends where `policy_prefill` on the same arguments leaves it.
+        Returns "action_tokens" (int32) and "action_preds" [B,Tn,act_dim] (argmax, never sampled; discrete: column 0,
+        the other columns -1 / 0), with `want_logits` "action_logits" [B,Tn,n_out] (n_out = num_actions when discrete,
+        act_dim * num_actions otherwise), and with `targets` (an integer tensor [B,Tn,act_dim] on this engine's device,
+        values in [-1, num_actions); -1 = a padded action dim, scored 0) "action_logprobs" [B,Tn,act_dim]: the log-softmax
+        of each action row's logits at the target (discrete: column 0). `lengths` (B ints in [0, Tn]) gives env b its
+        first lengths[b] timesteps only; outputs past them are -1 / 0 and an env with 0 keeps its state.
+        Lengths and targets are checked before anything reaches the library; the range check of `targets` costs one
+        device reduction and a synchronisation."""
+        cfg = self.cfg
+        B, Tn = state.B, states.shape[1]
+        lens = None if lengths is None else check_lengths(lengths, B, Tn, "Tn")
+        if targets is not None:
+            if not isinstance(targets, torch.Tensor):
+                raise ValueError(f"targets must be a tensor, got {type(targets).__name__}")
+            if targets.dtype.is_floating_point or targets.dtype.is_complex or targets.dtype == torch.bool:
+                raise ValueError(f"targets must be integers, got {targets.dtype}")
+            if tuple(targets.shape) != (B, Tn, cfg.act_dim):
+                raise ValueError(f"targets must have shape {(B, Tn, cfg.act_dim)}, got {tuple(targets.shape)}")
+            if targets.device != self.device:
+                raise ValueError(f"targets must be on {self.device}, got {targets.device}")
+            if targets.numel():
+                lo, hi = (int(v) for v in torch.aminmax(targets))
+                if lo < -1 or hi >= cfg.num_actions:
+                    raise ValueError(f"targets must lie in [-1, num_actions={cfg.num_actions}), got min {lo} max {hi}")
+        return self._policy_forward(state, states, rtg, rewards, lens, discrete, targets, want_logits)
+
+    @_on_device
+    def _policy_forward(self, state, states, rtg, rewards, lens, discrete, targets, want_logits):
+        cfg = self.cfg
+        B, Tn = state.B, states.shape[1]
+        assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == (B, Tn, cfg.state_dim)
+        assert rtg.is_cuda and rtg.dtype == torch.float32 and rtg.numel() == B * Tn
+        states, rtg = states.contiguous(), rtg.contiguous()
+        if rewards is not None:
+            rewards = rewards.to(self.device, torch.float32).contiguous()
+            assert rewards.numel() == B * Tn
+        out = {"action_tokens": torch.empty(B, Tn, cfg.act_dim, dtype=torch.int32, device=self.device),
+               "action_preds": torch.empty(B, Tn, cfg.act_dim, dtype=torch.float32, device=self.device)}
+        if want_logits:
+            n = cfg.num_actions if discrete else cfg.head_out
+            out["action_logits"] = torch.empty(B, Tn, n, dtype=torch.float32, device=self.device)
+        if targets is not None:
+            targets = targets.to(torch.int32).contiguous()
+            out["action_logprobs"] = torch.empty(B, Tn, cfg.act_dim, dtype=torch.float32, device=self.device)
+        so = L.XLSeqOutputs(tokens=out["action_tokens"].data_ptr(), actions=out["action_preds"].data_ptr(),
+                            logits=_ptr(out.get("action_logits")).value, targets=_ptr(targets).value,
+                            logprobs=_ptr(out.get("action_logprobs")).value)
+        L.check(self.lib.xl_policy_forward(
+            self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards),
+            None if lens is None else lens.ctypes.data_as(C.c_void_p), B, Tn, C.byref(so),
+            L.XL_FLAG_DISCRETE if discrete else 0, self._stream()))
+        return out
+
     @_on_device
     def policy_step(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,
                     rewards: Optional[torch.Tensor] = None, mode: int = L.XL_MODE_FUSED, flags: int = 0,
