@@ -136,7 +136,8 @@ typedef enum { XL_STATE_C = 0, XL_STATE_N = 1, XL_STATE_M = 2, XL_STATE_CONV = 3
 #define XL_FLAG_STATE_EMBEDS 8u /* xl_policy_step: `states` is fp32 [B, d] = state-token embeddings already
                                  * computed by the caller (image observations: embed_image / ImpalaCNN,
                                  * discrete_decision_transformer_model.py:187-203, image_encoders.py:10-66, stays in
-                                 * PyTorch/cuDNN); the embed_state Linear is skipped                          */
+                                 * PyTorch/cuDNN); the embed_state Linear is skipped. The sequence calls take
+                                 * embeddings through xl_policy_prefill_embeds / xl_policy_forward_embeds       */
 
 int xl_abi_version(void);
 const char* xl_last_error(void);
@@ -276,7 +277,7 @@ int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B
  * rewards fp32 [B, Tn] or NULL (= 0). Embeds every timestep into its (s, rtg, r) tokens
  * (online_decision_transformer_model.py:522-530,588-612) and prefills the 3*Tn tokens; no action outputs
  * (a context only warms the state: src/callbacks/evaluation.py:213-237 `persist_context`; xl_policy_forward below
- * returns them). */
+ * returns them). XL_FLAG_STATE_EMBEDS: XL_ERR_UNSUPPORTED, state untouched (embeddings: xl_policy_prefill_embeds). */
 int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
                       int Tn, unsigned flags, void* stream);
 
@@ -291,7 +292,8 @@ int xl_policy_prefill(xl_handle* h, void* state, const float* states, const floa
  *  - XL_ERR_INVALID_ARG before any device work: lengths NULL, a length < 0 or > S (Tn), and the checks of the uniform
  *    calls. XL_ERR_UNSUPPORTED (state untouched) for lengths that are neither all S nor all 0 when the shape has no
  *    sequence path (conv_kernel != 4, or a head dim without a cell plan); no shipped preset is affected.
- *  - The policy form's work never advances the sampler's step counter or the token ring slot (as xl_policy_prefill).
+ *  - The policy form's work never advances the sampler's step counter or the token ring slot (as xl_policy_prefill),
+ *    and it rejects XL_FLAG_STATE_EMBEDS as xl_policy_prefill does.
  * Work goes to the envs that have tokens: the active envs are sorted by length (descending, stable) and each chunk runs
  * on the prefix of them that still has tokens, an env's end padded up to the chunk with identity tokens (forget gate 1,
  * input gate 0, conv window and sLSTM state kept). When the active envs are not already envs 0..B'-1 in that order, their
@@ -339,9 +341,40 @@ typedef struct {
  *    Tn mod 8 timesteps of a uniform call (all of them on shapes without the sequence path) run as eager policy steps.
  *  - XL_ERR_INVALID_ARG: out NULL, logprobs without targets, and the checks of xl_policy_prefill(_ragged).
  *    XL_ERR_UNSUPPORTED: XL_FLAG_STATE_EMBEDS; lengths that are neither all Tn nor all 0 on shapes without the sequence
- *    path (as xl_policy_prefill_ragged; state and outputs untouched). Not graph-capturable. */
+ *    path (as xl_policy_prefill_ragged; state and outputs untouched). Not graph-capturable. State embeddings:
+ *    xl_policy_forward_embeds below. */
 int xl_policy_forward(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
                       const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out, unsigned flags, void* stream);
+
+/* Context prefill and sequence forward from state embeddings (image observations: the ImpalaCNN embed_image output of
+ * every frame, discrete_decision_transformer_model.py:187-203, or the reference's img_is_encoded inputs :185-186).
+ *  - state_embeds: device fp32 [B, Tn, d], 16-byte aligned: the state-token embedding of every timestep, as
+ *    xl_policy_step takes it with XL_FLAG_STATE_EMBEDS (the embed_state Linear is skipped). rtg, rewards: as for
+ *    xl_policy_prefill. lengths: NULL (every env has Tn timesteps) or a HOST int32 [B] array as for
+ *    xl_policy_prefill_ragged.
+ *  - Results: those of xl_policy_prefill / xl_policy_prefill_ragged / xl_policy_forward with each timestep's state token
+ *    replaced by the given embedding. Outputs at (b, t) are what xl_policy_step(XL_FLAG_STATE_EMBEDS) returns when env b
+ *    is stepped over its timesteps 0..t; timesteps that run as eager steps (the last Tn mod 8 of a uniform call) are
+ *    bit-identical to those steps. The state after xl_policy_forward_embeds is bit-identical to
+ *    xl_policy_prefill_embeds on the same arguments.
+ *  - Inherited from the calls above: inputs past lengths[b] are never read (they may hold NaN); an env with length 0
+ *    keeps every byte of its state slot; outputs past the length are -1 / 0; lengths all Tn are the uniform call
+ *    (bit-identical); always the argmax; the sampler step counter and the token ring slot do not move; not
+ *    graph-capturable; on shapes without the sequence path, lengths that are neither all Tn nor all 0 give
+ *    XL_ERR_UNSUPPORTED with state and outputs untouched.
+ *  - Each chunk's tokens come from one kernel (seq_embed_tokens_kernel) that reads the embedding, rtg and reward of
+ *    every (env, timestep) row from these buffers and applies embed_ln, writing the prefill's token rows; it shares its
+ *    per-row arithmetic with the step's embed kernel, so a state token gets the bits xl_policy_step gives it.
+ *  - Flags: XL_FLAG_DISCRETE and XL_FLAG_SIMPLE_GEMM as for xl_policy_forward; XL_FLAG_STATE_EMBEDS is accepted and
+ *    redundant.
+ *  - XL_ERR_INVALID_ARG before any device work: a null required pointer, state_embeds not 16-byte aligned, logprobs
+ *    without targets, and the checks of xl_policy_prefill(_ragged). */
+int xl_policy_prefill_embeds(xl_handle* h, void* state, const float* state_embeds, const float* rtg,
+                             const float* rewards, const int32_t* lengths, int B, int Tn, unsigned flags,
+                             void* stream);
+int xl_policy_forward_embeds(xl_handle* h, void* state, const float* state_embeds, const float* rtg,
+                             const float* rewards, const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out,
+                             unsigned flags, void* stream);
 
 /* out[M,N] = A[M,K] @ W[N,K]^T (+ bias[N]) (+ residual[M,N]); A fp32, W bf16, fp32 accumulate.
  * The nn.Linear of proj_up / proj_down / embed_state / action_net. impl: 0 auto, 1 CUDA-core, 2 tcgen05. */

@@ -56,7 +56,7 @@ class XLSampling(C.Structure):
 
 
 class XLSeqOutputs(C.Structure):
-    """xl_seq_outputs: device buffers of xl_policy_forward (each nullable)."""
+    """xl_seq_outputs: device buffers of xl_policy_forward(_embeds) (each nullable)."""
     _fields_ = [("tokens", C.c_void_p), ("actions", C.c_void_p), ("logits", C.c_void_p), ("targets", C.c_void_p),
                 ("logprobs", C.c_void_p)]
 
@@ -129,6 +129,10 @@ def load():
     lib.xl_policy_prefill_ragged.restype = i32
     lib.xl_policy_forward.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, C.POINTER(XLSeqOutputs), u32, vp]
     lib.xl_policy_forward.restype = i32
+    lib.xl_policy_prefill_embeds.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, u32, vp]
+    lib.xl_policy_prefill_embeds.restype = i32
+    lib.xl_policy_forward_embeds.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, C.POINTER(XLSeqOutputs), u32, vp]
+    lib.xl_policy_forward_embeds.restype = i32
     lib.xl_linear.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
     lib.xl_linear.restype = i32
     lib.xl_set_token_ring.argtypes = [vp, vp, i32, i32, vp]

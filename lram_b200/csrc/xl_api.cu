@@ -76,6 +76,7 @@ struct xl_handle {
   float *x = nullptr, *xn = nullptr, *u = nullptr, *qkv = nullptr, *act = nullptr, *gate_part = nullptr,
         *gated = nullptr, *partial = nullptr, *s_emb = nullptr, *states_pad = nullptr, *logits = nullptr,
         *d_states = nullptr, *d_rtg = nullptr, *d_rew = nullptr, *d_actions = nullptr, *xtok = nullptr, *hid = nullptr;
+  float* d_embeds = nullptr;    // [B, d] state embeddings staged by the eager tail of xl_policy_*_embeds
   int32_t* d_tokens = nullptr;
   unsigned int* counters = nullptr;
   __nv_bfloat16 *a_hi = nullptr, *a_lo = nullptr;
@@ -1345,6 +1346,7 @@ int xl_create(const xl_config* cfg, xl_handle** out) {
   h->part_rows = M < kSplitRows ? M : kSplitRows;
   const size_t o_pu = carve(4 * (size_t)kSplitMax * h->part_rows * 2 * inner);
   const size_t o_pd = carve(4 * (size_t)kSplitMax * h->part_rows * d);
+  const size_t o_de = carve(4 * B * d);   // last, so that the step's buffers keep their places
   h->ws_bytes = off;
   cudaError_t e = cudaMalloc((void**)&h->ws, h->ws_bytes);
   if (e != cudaSuccess) {
@@ -1371,6 +1373,7 @@ int xl_create(const xl_config* cfg, xl_handle** out) {
 
   h->a_hi = (__nv_bfloat16*)(h->ws + o_hi); h->a_lo = (__nv_bfloat16*)(h->ws + o_lo);
   h->part_up = (float*)(h->ws + o_pu); h->part_down = (float*)(h->ws + o_pd);
+  h->d_embeds = (float*)(h->ws + o_de);
   *out = h;
   return XL_OK;
 }
@@ -1827,7 +1830,27 @@ int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B
   return XL_OK;
 }
 
-// xl_policy_prefill; with a head hook (xl_policy_forward) also the action outputs of every timestep
+// Tokens of one prefill chunk (Bk envs x Tc timesteps from timestep pos) straight from given state embeddings
+// [B, Tn, d] into pf_x: one launch where raw states take a staging copy, pad_rows, the embed_state Linear and the embed
+// kernel. perm / len as in launch_ragged_rows (nullptr: envs 0..Bk-1, every timestep valid).
+static void seq_embed_chunk(xl_handle* h, const float* embeds, const float* rtg, const float* rewards,
+                            const int32_t* perm, const int32_t* len, int Bk, int Tn, int Tc, int pos, cudaStream_t s) {
+  const xl_config& c = h->cfg;
+  auto PW = [&](int id) { return (const float*)h->pw[id - XL_W_POST_NORM]; };
+  xl::SeqEmbedParams p;
+  p.s_emb = embeds; p.rtg = rtg; p.rew = rewards;
+  p.perm = perm; p.len = len; p.len_div = c.tokens_per_step;
+  p.Tn = Tn; p.Tc = Tc; p.pos = pos; p.rows = Bk * Tc; p.d = c.embedding_dim;
+  p.w_ret = PW(XL_W_EMBED_RETURN_W); p.b_ret = PW(XL_W_EMBED_RETURN_B);
+  p.w_rew = PW(XL_W_EMBED_REWARD_W); p.b_rew = PW(XL_W_EMBED_REWARD_B);
+  p.ln_w = PW(XL_W_EMBED_LN_W); p.ln_b = PW(XL_W_EMBED_LN_B); p.eps = c.embed_ln_eps;
+  p.x = prefill_ws(h).x;
+  xl::launch_seq_embed_tokens(p, s);
+  h->launches += 1;
+}
+
+// xl_policy_prefill; with a head hook (xl_policy_forward) also the action outputs of every timestep. With
+// XL_FLAG_STATE_EMBEDS (the _embeds entries) `states` holds state embeddings [B, Tn, d].
 static int policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
                           int Tn, unsigned flags, void* stream, const SeqHead* head) {
   int rc = check_batch(h, B);
@@ -1841,6 +1864,8 @@ static int policy_prefill(xl_handle* h, void* state, const float* states, const 
   const int d = c.embedding_dim, sd = c.state_dim, T = c.tokens_per_step;
   const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
   auto PW = [&](int id) { return h->pw[id - XL_W_POST_NORM]; };
+  const bool embeds = (flags & XL_FLAG_STATE_EMBEDS) != 0;
+  const int sw = embeds ? d : sd;   // row width of `states`
   int pos = 0;   // timesteps done
   if (prefill_fast_path(h)) {
     const int tc_max = prefill_chunk_tokens(h, B) / T;
@@ -1851,28 +1876,32 @@ static int policy_prefill(xl_handle* h, void* state, const float* states, const 
       const int rows = B * Tc;
       rc = ensure_prefill_ws(h, rows * T);
       if (rc) return rc;
-      const Ws ws = prefill_ws(h);
-      // gather the chunk's timesteps of every env: [B, Tc, sd], [B, Tc]
-      XL_CUDA(cudaMemcpy2DAsync(h->pf_sin, sizeof(float) * (size_t)Tc * sd, states + (size_t)pos * sd,
-                                sizeof(float) * (size_t)Tn * sd, sizeof(float) * (size_t)Tc * sd, B,
-                                cudaMemcpyDeviceToDevice, s));
-      XL_CUDA(cudaMemcpy2DAsync(h->pf_rtg, sizeof(float) * (size_t)Tc, rtg + pos, sizeof(float) * (size_t)Tn,
-                                sizeof(float) * (size_t)Tc, B, cudaMemcpyDeviceToDevice, s));
-      if (rewards)
-        XL_CUDA(cudaMemcpy2DAsync(h->pf_rew, sizeof(float) * (size_t)Tc, rewards + pos, sizeof(float) * (size_t)Tn,
+      if (embeds) {
+        seq_embed_chunk(h, states, rtg, rewards, nullptr, nullptr, B, Tn, Tc, pos, s);
+      } else {
+        const Ws ws = prefill_ws(h);
+        // gather the chunk's timesteps of every env: [B, Tc, sd], [B, Tc]
+        XL_CUDA(cudaMemcpy2DAsync(h->pf_sin, sizeof(float) * (size_t)Tc * sd, states + (size_t)pos * sd,
+                                  sizeof(float) * (size_t)Tn * sd, sizeof(float) * (size_t)Tc * sd, B,
+                                  cudaMemcpyDeviceToDevice, s));
+        XL_CUDA(cudaMemcpy2DAsync(h->pf_rtg, sizeof(float) * (size_t)Tc, rtg + pos, sizeof(float) * (size_t)Tn,
                                   sizeof(float) * (size_t)Tc, B, cudaMemcpyDeviceToDevice, s));
-      // embed: rows (env, timestep) -> tokens (env, timestep, {s, rtg, r}) == the env's sequence order
-      xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
-      h->launches += 1;
-      rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
-                  rows, d, h->Kpad, impl, s);
-      if (rc) return rc;
-      xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
-                              (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
-                              (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
-                              (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
-                              0.f, nullptr, nullptr, nullptr, s);
-      h->launches += 1;
+        if (rewards)
+          XL_CUDA(cudaMemcpy2DAsync(h->pf_rew, sizeof(float) * (size_t)Tc, rewards + pos, sizeof(float) * (size_t)Tn,
+                                    sizeof(float) * (size_t)Tc, B, cudaMemcpyDeviceToDevice, s));
+        // embed: rows (env, timestep) -> tokens (env, timestep, {s, rtg, r}) == the env's sequence order
+        xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
+        h->launches += 1;
+        rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
+                    rows, d, h->Kpad, impl, s);
+        if (rc) return rc;
+        xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
+                                (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
+                                (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
+                                (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
+                                0.f, nullptr, nullptr, nullptr, s);
+        h->launches += 1;
+      }
       rc = prefill_blocks(h, state, B, B, Tc * T, flags, s);
       if (rc) return rc;
       if (head && (rc = seq_head_chunk(h, *head, B, Tc, pos, nullptr, nullptr, flags, s))) return rc;
@@ -1883,15 +1912,16 @@ static int policy_prefill(xl_handle* h, void* state, const float* states, const 
   // of one timestep)
   if (head && pos < Tn && (rc = ensure_seq_logits(h, (size_t)B * head->n_out))) return rc;
   for (; pos < Tn; ++pos) {
-    XL_CUDA(cudaMemcpy2DAsync(h->d_states, sizeof(float) * (size_t)sd, states + (size_t)pos * sd,
-                              sizeof(float) * (size_t)Tn * sd, sizeof(float) * (size_t)sd, B, cudaMemcpyDeviceToDevice, s));
+    float* stage = embeds ? h->d_embeds : h->d_states;
+    XL_CUDA(cudaMemcpy2DAsync(stage, sizeof(float) * (size_t)sw, states + (size_t)pos * sw,
+                              sizeof(float) * (size_t)Tn * sw, sizeof(float) * (size_t)sw, B, cudaMemcpyDeviceToDevice, s));
     XL_CUDA(cudaMemcpy2DAsync(h->d_rtg, sizeof(float), rtg + pos, sizeof(float) * (size_t)Tn, sizeof(float), B,
                               cudaMemcpyDeviceToDevice, s));
     if (rewards)
       XL_CUDA(cudaMemcpy2DAsync(h->d_rew, sizeof(float), rewards + pos, sizeof(float) * (size_t)Tn, sizeof(float), B,
                                 cudaMemcpyDeviceToDevice, s));
     StepArgs a;
-    a.state = state; a.states = h->d_states; a.rtg = h->d_rtg; a.rewards = rewards ? h->d_rew : nullptr;
+    a.state = state; a.states = stage; a.rtg = h->d_rtg; a.rewards = rewards ? h->d_rew : nullptr;
     a.tokens = h->d_tokens; a.actions = h->d_actions; a.logits = head ? h->sq_logits : nullptr; a.hidden = nullptr;
     a.B = B; a.mode = XL_MODE_FUSED; a.flags = (flags & ~(unsigned)XL_FLAG_GRAPH) | kFlagNoRing;
     rc = run_policy(h, a, s);
@@ -1901,8 +1931,17 @@ static int policy_prefill(xl_handle* h, void* state, const float* states, const 
   return XL_OK;
 }
 
+// raw-state policy prefills: state embeddings go through the _embeds entries (the loops would read them as [B, Tn, sd])
+static int reject_state_embeds(const char* fn, unsigned flags) {
+  if (flags & XL_FLAG_STATE_EMBEDS)
+    return fail(XL_ERR_UNSUPPORTED, "%s takes raw states; state embeddings go through xl_policy_prefill_embeds / "
+                                    "xl_policy_forward_embeds", fn);
+  return XL_OK;
+}
+
 int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
                       int Tn, unsigned flags, void* stream) {
+  if (int rc = reject_state_embeds("xl_policy_prefill", flags)) return rc;
   return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, nullptr);
 }
 
@@ -1944,7 +1983,8 @@ int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out
   return ragged_end(h, state, B, p, s);
 }
 
-// xl_policy_prefill_ragged; with a head hook (xl_policy_forward) also the action outputs of every timestep
+// xl_policy_prefill_ragged; with a head hook (xl_policy_forward) also the action outputs of every timestep. With
+// XL_FLAG_STATE_EMBEDS `states` holds state embeddings [B, Tn, d].
 static int policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
                                  const int32_t* lengths, int B, int Tn, unsigned flags, void* stream,
                                  const SeqHead* head) {
@@ -1972,23 +2012,27 @@ static int policy_prefill_ragged(xl_handle* h, void* state, const float* states,
   if ((rc = ragged_chunks(h, p.len, T, chunks))) return rc;
   for (const RaggedChunk& ch : chunks) {
     const int Tc = ch.n, rows = ch.Bk * Tc;
-    const Ws ws = prefill_ws(h);
-    // the chunk's timesteps of the prefix envs, pads zero-filled: [Bk, Tc, sd], [Bk, Tc]
-    xl::launch_ragged_rows(const_cast<float*>(states), h->pf_sin, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, sd, 0, s);
-    xl::launch_ragged_rows(const_cast<float*>(rtg), h->pf_rtg, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
-    if (rewards)
-      xl::launch_ragged_rows(const_cast<float*>(rewards), h->pf_rew, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
-    xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
-    h->launches += rewards ? 4 : 3;
-    rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
-                rows, d, h->Kpad, impl, s);
-    if (rc) return rc;
-    xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
-                            (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
-                            (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
-                            (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
-                            0.f, nullptr, nullptr, nullptr, s);
-    h->launches += 1;
+    if (flags & XL_FLAG_STATE_EMBEDS) {
+      seq_embed_chunk(h, states, rtg, rewards, p.d_perm, p.d_len, ch.Bk, Tn, Tc, ch.pos, s);
+    } else {
+      const Ws ws = prefill_ws(h);
+      // the chunk's timesteps of the prefix envs, pads zero-filled: [Bk, Tc, sd], [Bk, Tc]
+      xl::launch_ragged_rows(const_cast<float*>(states), h->pf_sin, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, sd, 0, s);
+      xl::launch_ragged_rows(const_cast<float*>(rtg), h->pf_rtg, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
+      if (rewards)
+        xl::launch_ragged_rows(const_cast<float*>(rewards), h->pf_rew, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
+      xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
+      h->launches += rewards ? 4 : 3;
+      rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
+                  rows, d, h->Kpad, impl, s);
+      if (rc) return rc;
+      xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
+                              (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
+                              (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
+                              (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
+                              0.f, nullptr, nullptr, nullptr, s);
+      h->launches += 1;
+    }
     rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, Tc * T, flags, s, p.d_len, ch.pos * T);
     if (rc) return rc;
     if (head && (rc = seq_head_chunk(h, *head, ch.Bk, Tc, ch.pos, p.d_perm, p.d_len, flags, s))) return rc;
@@ -1999,6 +2043,7 @@ static int policy_prefill_ragged(xl_handle* h, void* state, const float* states,
 
 int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
                              const int32_t* lengths, int B, int Tn, unsigned flags, void* stream) {
+  if (int rc = reject_state_embeds("xl_policy_prefill_ragged", flags)) return rc;
   return policy_prefill_ragged(h, state, states, rtg, rewards, lengths, B, Tn, flags, stream, nullptr);
 }
 
@@ -2016,6 +2061,41 @@ int xl_policy_forward(xl_handle* h, void* state, const float* states, const floa
   hd.Tn = Tn;
   if (!lengths) return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, &hd);
   return policy_prefill_ragged(h, state, states, rtg, rewards, lengths, B, Tn, flags, stream, &hd);
+}
+
+// the state-embedding forms run the same loops with XL_FLAG_STATE_EMBEDS: each chunk's tokens come from one
+// seq_embed_tokens launch, the eager tail stages [B, d] rows into d_embeds for policy_front
+static int check_embeds(const float* state_embeds) {
+  if ((uintptr_t)state_embeds % 16)
+    return fail(XL_ERR_INVALID_ARG, "state_embeds must be 16-byte aligned (rows are loaded as float4)");
+  return XL_OK;
+}
+
+int xl_policy_prefill_embeds(xl_handle* h, void* state, const float* state_embeds, const float* rtg,
+                             const float* rewards, const int32_t* lengths, int B, int Tn, unsigned flags,
+                             void* stream) {
+  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+  if (int rc = check_embeds(state_embeds)) return rc;
+  flags |= XL_FLAG_STATE_EMBEDS;
+  if (!lengths) return policy_prefill(h, state, state_embeds, rtg, rewards, B, Tn, flags, stream, nullptr);
+  return policy_prefill_ragged(h, state, state_embeds, rtg, rewards, lengths, B, Tn, flags, stream, nullptr);
+}
+
+int xl_policy_forward_embeds(xl_handle* h, void* state, const float* state_embeds, const float* rtg,
+                             const float* rewards, const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out,
+                             unsigned flags, void* stream) {
+  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+  if (!out) return fail(XL_ERR_INVALID_ARG, "null outputs");
+  if (out->logprobs && !out->targets) return fail(XL_ERR_INVALID_ARG, "logprobs need targets");
+  if (int rc = check_embeds(state_embeds)) return rc;
+  SeqHead hd;
+  hd.out = *out;
+  hd.discrete = (flags & XL_FLAG_DISCRETE) ? 1 : 0;
+  hd.n_out = hd.discrete ? h->num_actions : h->head_out;
+  hd.Tn = Tn;
+  flags |= XL_FLAG_STATE_EMBEDS;
+  if (!lengths) return policy_prefill(h, state, state_embeds, rtg, rewards, B, Tn, flags, stream, &hd);
+  return policy_prefill_ragged(h, state, state_embeds, rtg, rewards, lengths, B, Tn, flags, stream, &hd);
 }
 
 int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bias, const float* residual,

@@ -196,8 +196,35 @@ void launch_ln_rows_gather(const float* x, const float* part, int splits, int64_
 // ------------------------------------------------------------------------------------------------
 // Token embedding: embed_inputs + stack (s, rtg, r) + embed_ln
 // (online_decision_transformer_model.py:522-530,588-612; discrete_decision_transformer_model.py:266-275)
-// one warp per (b, tok) row.
+// The per-row arithmetic lives in embed_token_row_warp / embed_token_row_cta, shared by the step's embed kernels and the
+// sequence embed kernels below, so that a timestep's tokens get the same bits on either path.
 // ------------------------------------------------------------------------------------------------
+
+// One token row, one warp: o[0, d) = embed_ln(tok == 0 ? s_row : scal * wv + bv). kPads: s_row == nullptr is a zero
+// state embedding (the step always has one; its instantiation is free of the check).
+template <bool kPads>
+__device__ __forceinline__ void embed_token_row_warp(int tok, int lane, const float* __restrict__ s_row, float scal,
+                                                     const float* __restrict__ wv, const float* __restrict__ bv,
+                                                     const float* __restrict__ ln_w, const float* __restrict__ ln_b,
+                                                     float eps, float* __restrict__ o, int d) {
+  auto val = [&](int i) -> float {
+    return tok == 0 ? ((!kPads || s_row) ? s_row[i] : 0.f) : fmaf(scal, wv[i], bv[i]);
+  };
+  float s = 0.f;
+  for (int i = lane; i < d; i += 32) s += val(i);
+  s = warp_sum(s);
+  const float mean = s / (float)d;
+  float q = 0.f;
+  for (int i = lane; i < d; i += 32) {
+    float a = val(i) - mean;
+    q += a * a;
+  }
+  q = warp_sum(q);
+  const float rstd = rsqrtf(q / (float)d + eps);
+  for (int i = lane; i < d; i += 32) o[i] = (val(i) - mean) * rstd * ln_w[i] + ln_b[i];
+}
+
+// one warp per (b, tok) row
 __global__ void __launch_bounds__(256) embed_tokens_kernel(
     const float* __restrict__ s_emb, const float* __restrict__ rtg, const float* __restrict__ rew,
     const float* __restrict__ w_ret, const float* __restrict__ b_ret, const float* __restrict__ w_rew,
@@ -218,23 +245,9 @@ __global__ void __launch_bounds__(256) embed_tokens_kernel(
   if (row >= 3 * B) return;
   const int b = row / 3, tok = row - 3 * b;
   const float scal = (tok == 1) ? rtg[b] : ((tok == 2 && rew) ? rew[b] : 0.f);
-  const float* wv = (tok == 1) ? w_ret : w_rew;
-  const float* bv = (tok == 1) ? b_ret : b_rew;
-  const float* se = s_emb + (int64_t)b * d;
-  auto val = [&](int i) -> float { return tok == 0 ? se[i] : fmaf(scal, wv[i], bv[i]); };
-  float s = 0.f;
-  for (int i = lane; i < d; i += 32) s += val(i);
-  s = warp_sum(s);
-  const float mean = s / (float)d;
-  float q = 0.f;
-  for (int i = lane; i < d; i += 32) {
-    float a = val(i) - mean;
-    q += a * a;
-  }
-  q = warp_sum(q);
-  const float rstd = rsqrtf(q / (float)d + eps);
   float* o = x + (int64_t)row * d;
-  for (int i = lane; i < d; i += 32) o[i] = (val(i) - mean) * rstd * ln_w[i] + ln_b[i];
+  embed_token_row_warp<false>(tok, lane, s_emb + (int64_t)b * d, scal, tok == 1 ? w_ret : w_rew, tok == 1 ? b_ret : b_rew,
+                       ln_w, ln_b, eps, o, d);
   if (!ln0_w) return;
   // the first block's pre-norm (xlstm LayerNorm, gamma = 1 + w) on the row this warp just produced: the block stack's
   // first LayerNorm launch disappears. Each lane re-reads only what it wrote itself.
@@ -260,8 +273,46 @@ __global__ void __launch_bounds__(256) embed_tokens_kernel(
   }
 }
 
-// CTA-per-row version (d <= 4096): one float4 per thread held in registers, block reductions; the token row is read
-// once and both LayerNorms (embed_ln, then optionally block 0's pre-norm) run on registers.
+// CTA-per-row form (d <= 4096): thread i holds channels 4i..4i+3 (ok: 4i < d) in registers, block reductions.
+// The weights of token `tok`, loaded before the dependency wait.
+__device__ __forceinline__ void embed_token_weights_cta(int tok, int i, bool ok, const float* __restrict__ w_ret,
+                                                        const float* __restrict__ b_ret, const float* __restrict__ w_rew,
+                                                        const float* __restrict__ b_rew, const float* __restrict__ ln_w,
+                                                        const float* __restrict__ ln_b, float4& g, float4& bb,
+                                                        float4& wv, float4& bv) {
+  g = bb = wv = bv = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (!ok) return;
+  g = reinterpret_cast<const float4*>(ln_w)[i];
+  bb = reinterpret_cast<const float4*>(ln_b)[i];
+  if (tok != 0) {
+    wv = reinterpret_cast<const float4*>(tok == 1 ? w_ret : w_rew)[i];
+    bv = reinterpret_cast<const float4*>(tok == 1 ? b_ret : b_rew)[i];
+  }
+}
+
+// One token row: embed_ln(tok == 0 ? s_row : scal() * wv + bv), this thread's four channels; scal() reads the rtg /
+// reward. kPads: s_row == nullptr is a zero state embedding (the step's instantiation is free of the check).
+template <bool kPads, typename Scal>
+__device__ __forceinline__ float4 embed_token_row_cta(int tok, int i, bool ok, const float* __restrict__ s_row,
+                                                      Scal scal_of, float4 wv, float4 bv, float4 g, float4 bb, int d,
+                                                      float eps, float* red) {
+  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+  if (ok) {
+    if (tok == 0) {
+      if (!kPads || s_row) v = reinterpret_cast<const float4*>(s_row)[i];
+    } else {
+      const float scal = scal_of();
+      v = make_float4(fmaf(scal, wv.x, bv.x), fmaf(scal, wv.y, bv.y), fmaf(scal, wv.z, bv.z), fmaf(scal, wv.w, bv.w));
+    }
+  }
+  const float mean = block_sum((v.x + v.y) + (v.z + v.w), red) / (float)d;
+  const float a0 = v.x - mean, a1 = v.y - mean, a2 = v.z - mean, a3 = v.w - mean;
+  const float rstd = rsqrtf(block_sum(ok ? (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3) : 0.f, red) / (float)d + eps);
+  return make_float4(a0 * rstd * g.x + bb.x, a1 * rstd * g.y + bb.y, a2 * rstd * g.z + bb.z, a3 * rstd * g.w + bb.w);
+}
+
+// the step's embed kernel: one CTA per (b, tok) row; the token row is read once and both LayerNorms (embed_ln, then
+// optionally block 0's pre-norm) run on registers.
 __global__ void __launch_bounds__(1024) embed_tokens_cta_kernel(
     const float* __restrict__ s_emb, const float* __restrict__ rtg, const float* __restrict__ rew,
     const float* __restrict__ w_ret, const float* __restrict__ b_ret, const float* __restrict__ w_rew,
@@ -275,39 +326,22 @@ __global__ void __launch_bounds__(1024) embed_tokens_cta_kernel(
   const bool ok = i < (d >> 2);
   const int b = row / 3, tok = row - 3 * b;
   // weights before the dependency wait
-  float4 g = make_float4(0.f, 0.f, 0.f, 0.f), bb = g, wv = g, bv = g, g0 = g;
-  if (ok) {
-    g = reinterpret_cast<const float4*>(ln_w)[i];
-    bb = reinterpret_cast<const float4*>(ln_b)[i];
-    if (tok != 0) {
-      wv = reinterpret_cast<const float4*>(tok == 1 ? w_ret : w_rew)[i];
-      bv = reinterpret_cast<const float4*>(tok == 1 ? b_ret : b_rew)[i];
-    }
-    if (ln0_w) g0 = reinterpret_cast<const float4*>(ln0_w)[i];
-  }
+  float4 g, bb, wv, bv, g0 = make_float4(0.f, 0.f, 0.f, 0.f);
+  embed_token_weights_cta(tok, i, ok, w_ret, b_ret, w_rew, b_rew, ln_w, ln_b, g, bb, wv, bv);
+  if (ok && ln0_w) g0 = reinterpret_cast<const float4*>(ln0_w)[i];
   pdl_wait();
   if (step_counter && blockIdx.x == 0 && threadIdx.x == 0) *step_counter = *step_counter + 1;   // token ring slot
   if (sample_counter && blockIdx.x == 0 && threadIdx.x == 0) *sample_counter = *sample_counter + 1;   // sampler step
   pdl_trigger();
-  float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
-  if (ok) {
-    if (tok == 0) {
-      v = reinterpret_cast<const float4*>(s_emb + (int64_t)b * d)[i];
-    } else {
-      const float scal = (tok == 1) ? rtg[b] : (rew ? rew[b] : 0.f);
-      v = make_float4(fmaf(scal, wv.x, bv.x), fmaf(scal, wv.y, bv.y), fmaf(scal, wv.z, bv.z), fmaf(scal, wv.w, bv.w));
-    }
-  }
-  float mean = block_sum((v.x + v.y) + (v.z + v.w), red) / (float)d;
-  float a0 = v.x - mean, a1 = v.y - mean, a2 = v.z - mean, a3 = v.w - mean;
-  float rstd = rsqrtf(block_sum(ok ? (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3) : 0.f, red) / (float)d + eps);
-  float4 o = make_float4(a0 * rstd * g.x + bb.x, a1 * rstd * g.y + bb.y, a2 * rstd * g.z + bb.z, a3 * rstd * g.w + bb.w);
+  float4 o = embed_token_row_cta<false>(
+      tok, i, ok, s_emb + (int64_t)b * d, [&] { return (tok == 1) ? rtg[b] : (rew ? rew[b] : 0.f); }, wv, bv, g, bb, d,
+      eps, red);
   if (ok) reinterpret_cast<float4*>(x + (int64_t)row * d)[i] = o;
   if (!ln0_w) return;
   if (!ok) o = make_float4(0.f, 0.f, 0.f, 0.f);
-  mean = block_sum((o.x + o.y) + (o.z + o.w), red) / (float)d;
-  a0 = o.x - mean; a1 = o.y - mean; a2 = o.z - mean; a3 = o.w - mean;
-  rstd = rsqrtf(block_sum(ok ? (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3) : 0.f, red) / (float)d + ln0_eps);
+  const float mean = block_sum((o.x + o.y) + (o.z + o.w), red) / (float)d;
+  const float a0 = o.x - mean, a1 = o.y - mean, a2 = o.z - mean, a3 = o.w - mean;
+  const float rstd = rsqrtf(block_sum(ok ? (a0 * a0 + a1 * a1) + (a2 * a2 + a3 * a3) : 0.f, red) / (float)d + ln0_eps);
   if (!ok) return;
   const float r[4] = {a0 * rstd * (1.f + g0.x), a1 * rstd * (1.f + g0.y), a2 * rstd * (1.f + g0.z), a3 * rstd * (1.f + g0.w)};
   if (xn0) reinterpret_cast<float4*>(xn0 + (int64_t)row * d)[i] = make_float4(r[0], r[1], r[2], r[3]);
@@ -339,6 +373,61 @@ void launch_embed_tokens(const float* s_emb, const float* rtg, const float* rew,
   dim3 grid((rows + 7) / 8);
   launch_k(embed_tokens_kernel, grid, dim3(256), 0, s, s_emb, rtg, rew, w_ret, b_ret, w_rew, b_rew, ln_w, ln_b, eps,
            x, B, d, step_counter, sample_counter, ln0_w, ln0_eps, xn0, (__nv_bfloat16*)a_hi, (__nv_bfloat16*)a_lo);
+}
+
+// ---- sequence embed: the tokens of a prefill chunk straight from the caller's [B, Tn, ...] buffers ---------------
+// Token row (k * Tc + t) * 3 + tok of the chunk reads env (perm ? perm[k] : k), timestep pos + t. Rows at or past the
+// env's length (len[k] / len_div - pos) never touch caller memory: they are the tokens of a zero embedding, zero rtg
+// and zero reward (finite; the prefill turns them into identity tokens through len).
+// s_row: the row's state embedding (tok 0); scal: its rtg / reward (tok 1 / 2); nullptr = zero.
+__device__ __forceinline__ void seq_embed_source(const SeqEmbedParams& p, int row, int tok, const float*& s_row,
+                                                 const float*& scal) {
+  const int kt = row / 3, k = kt / p.Tc, t = kt - k * p.Tc;
+  s_row = scal = nullptr;
+  const int n = p.len ? min(max(p.len[k] / p.len_div - p.pos, 0), p.Tc) : p.Tc;
+  if (t >= n) return;
+  const int64_t off = (int64_t)(p.perm ? p.perm[k] : k) * p.Tn + p.pos + t;
+  if (tok == 0) s_row = p.s_emb + off * p.d;
+  else scal = tok == 1 ? p.rtg + off : (p.rew ? p.rew + off : nullptr);
+}
+
+__global__ void __launch_bounds__(1024) seq_embed_tokens_kernel(SeqEmbedParams p) {
+  __shared__ float red[32];
+  const int row = blockIdx.x, i = threadIdx.x;
+  const bool ok = i < (p.d >> 2);
+  const int tok = row % 3;
+  float4 g, bb, wv, bv;
+  embed_token_weights_cta(tok, i, ok, p.w_ret, p.b_ret, p.w_rew, p.b_rew, p.ln_w, p.ln_b, g, bb, wv, bv);
+  pdl_wait();
+  pdl_trigger();
+  const float *s_row, *scal;
+  seq_embed_source(p, row, tok, s_row, scal);
+  const float4 o = embed_token_row_cta<true>(tok, i, ok, s_row, [&] { return scal ? *scal : 0.f; }, wv, bv, g, bb, p.d,
+                                             p.eps, red);
+  if (ok) reinterpret_cast<float4*>(p.x + (int64_t)row * p.d)[i] = o;
+}
+
+// d > 4096: one warp per token row
+__global__ void __launch_bounds__(256) seq_embed_tokens_warp_kernel(SeqEmbedParams p) {
+  const int row = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
+  pdl_wait();
+  pdl_trigger();
+  if (row >= 3 * p.rows) return;
+  const int tok = row % 3;
+  const float *s_row, *scal;
+  seq_embed_source(p, row, tok, s_row, scal);
+  embed_token_row_warp<true>(tok, lane, s_row, scal ? *scal : 0.f, tok == 1 ? p.w_ret : p.w_rew,
+                       tok == 1 ? p.b_ret : p.b_rew, p.ln_w, p.ln_b, p.eps, p.x + (int64_t)row * p.d, p.d);
+}
+
+void launch_seq_embed_tokens(const SeqEmbedParams& p, cudaStream_t s) {
+  if (p.rows <= 0) return;
+  const int64_t rows = 3 * (int64_t)p.rows;
+  if (p.d <= 4096 && (p.d & 3) == 0) {
+    launch_k(seq_embed_tokens_kernel, dim3((unsigned)rows), dim3((((p.d >> 2) + 31) / 32) * 32), 0, s, p);
+    return;
+  }
+  launch_k(seq_embed_tokens_warp_kernel, dim3((unsigned)((rows + 7) / 8)), dim3(256), 0, s, p);
 }
 
 // zero-pad states [rows, K] -> bf16 hi/lo operand planes [rows, Kpad] of the embed_state GEMM (pad + split in one)

@@ -136,6 +136,24 @@ struct SeqHeadParams {
 };
 void launch_seq_head(const SeqHeadParams& p, cudaStream_t s);
 
+// Embedded (s, rtg, r) tokens of one prefill chunk from given state embeddings (xl_policy_forward_embeds /
+// xl_policy_prefill_embeds), with the step embed kernel's per-row arithmetic: x row (k * Tc + t) * 3 + tok from caller
+// env perm[k], timestep pos + t. Rows past the env's length read nothing and are the tokens of zeros (see
+// xl_elementwise.cu).
+struct SeqEmbedParams {
+  const float* s_emb;           // [B, Tn, d] state-token embeddings (16-byte aligned)
+  const float* rtg;             // [B, Tn]
+  const float* rew;             // [B, Tn] or nullptr (= 0)
+  const int32_t* perm;          // compact env k -> caller env perm[k]; nullptr = identity
+  const int32_t* len;           // env k's valid timesteps are t < len[k] / len_div - pos; nullptr = all Tc
+  int len_div, Tn, Tc, pos;
+  int rows, d;                  // rows = Bk * Tc timesteps
+  const float *w_ret, *b_ret, *w_rew, *b_rew, *ln_w, *ln_b;
+  float eps;
+  float* x;                     // [Bk, Tc, 3, d]
+};
+void launch_seq_embed_tokens(const SeqEmbedParams& p, cudaStream_t s);
+
 // bulk L2 prefetch of [base, base+bytes) (side stream, plain launch; see xl_elementwise.cu)
 void launch_l2_prefetch(const void* base, size_t bytes, int num_sms, int evict_last, cudaStream_t s);
 

@@ -33,7 +33,7 @@ import torch.nn as nn
 from . import _lib as L
 from .config import XLSTMPolicyConfig
 from .engine import StateCache, XLSTMEngine, strip_checkpoint_prefixes
-from .image_encoder import ImpalaCNN, scale_frames
+from .image_encoder import ImpalaCNN, embed_frames, scale_frames
 from .tokenizers import make_tokenizer
 
 
@@ -316,6 +316,7 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
         self.use_graph = use_graph
         self.image_shape = tuple(image_shape) if image_shape is not None else None
         self.img_is_encoded = img_is_encoded
+        self.image_max_frames = 2048        # frames per ImpalaCNN call on the sequence forward (embed_frames)
         d = cfg.d
         # LRAM-side modules, reference names (online_decision_transformer_model.py:92-94, multi_domain...:47-49,67-81)
         self.embed_state = nn.Linear(cfg.state_dim, d)
@@ -508,22 +509,30 @@ class MultiDomainDiscreteDecisionXLSTMModel(nn.Module):
         rtg token (SURVEY.md a10/a11), from a fresh zero state; no cache is kept (`past_key_values=None`). Runs as one
         `XLSTMEngine.policy_forward`. Returns action_preds [B,T,A] (discrete [B,T,1]), action_logits [B,T,A,num_actions]
         (discrete [B,T,1,num_actions]) and action_tokens. `last_hidden_state` is None: the sequence forward returns no
-        hidden states. `attention_mask` is not read, as the reference's encoder does not read it. Rewards None = 0."""
+        hidden states. `attention_mask` is not read, as the reference's encoder does not read it. Rewards None = 0.
+        Image observations take the cache path's two forms: raw frames [B,T,C,H,W] (0..255) through embed_image
+        (`image_encoder.embed_frames`, in slices of `image_max_frames` frames), or [B,T,d] embeddings with
+        `img_is_encoded`; both run as one `policy_forward(state_embeds=True)`."""
         cfg = self.cfg
-        if states.dim() == 5 or (states.dim() == 3 and self.img_is_encoded and states.shape[-1] == cfg.d):
-            raise NotImplementedError("image observations are not implemented on the sequence forward")
-        if states.dim() != 3:
-            raise ValueError(f"states must be [B,T,{cfg.state_dim}], got {tuple(states.shape)}")
-        if states.shape[-1] != cfg.state_dim:
+        encoded = states.dim() == 3 and self.img_is_encoded and states.shape[-1] == cfg.d
+        if states.dim() == 5 and self.embed_image is None:
+            raise NotImplementedError("image observations on the sequence forward need embed_image.* weights")
+        if states.dim() == 3 and not encoded and states.shape[-1] != cfg.state_dim:
             raise ValueError(f"states must be padded to {cfg.state_dim} (DecisionXLSTM.pad_inputs)")
+        if states.dim() not in (3, 5):
+            raise ValueError(f"states must be [B,T,{cfg.state_dim}] or [B,T,C,H,W], got {tuple(states.shape)}")
         B, T = states.shape[:2]
         engine = self.engine_for(B)
         dev = engine.device
         discrete = bool(self.is_discrete and actions is not None and actions.shape[-1] == 1)
-        st = states.to(dev, torch.float32).contiguous()
+        if states.dim() == 5:
+            st = embed_frames(self.embed_image, states, max_frames=self.image_max_frames)
+        else:
+            st = states.to(dev, torch.float32).contiguous()
         rtg = returns_to_go.to(dev, torch.float32).reshape(B, T).contiguous()
         rew = None if rewards is None else rewards.to(dev, torch.float32).reshape(B, T).contiguous()
-        out = engine.policy_forward(engine.new_state(B), st, rtg, rew, discrete=discrete, want_logits=True)
+        out = engine.policy_forward(engine.new_state(B), st, rtg, rew, discrete=discrete, want_logits=True,
+                                    state_embeds=states.dim() == 5 or encoded)
         tokens = out["action_tokens"].to(torch.long)
         if discrete:
             action_preds = tokens[:, :, :1]

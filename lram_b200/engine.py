@@ -338,26 +338,54 @@ class XLSTMEngine:
                                                self._stream()))
         return out
 
+    def _check_state_embeds(self, states, B: int):
+        """`states` of a sequence call with state_embeds=True: fp32 [B, Tn, d] on this engine's device."""
+        want = f"an fp32 tensor [B={B}, Tn, d={self.cfg.d}] on {self.device}"
+        if not isinstance(states, torch.Tensor):
+            raise ValueError(f"state embeddings must be {want}, got {type(states).__name__}")
+        if states.dim() != 3 or states.shape[0] != B or states.shape[2] != self.cfg.d:
+            raise ValueError(f"state embeddings must be {want}, got shape {tuple(states.shape)}")
+        if states.dtype != torch.float32:
+            raise ValueError(f"state embeddings must be {want}, got {states.dtype}")
+        if states.device != self.device:
+            raise ValueError(f"state embeddings must be {want}, got a tensor on {states.device}")
+
+    @staticmethod
+    def _embeds_operand(states: torch.Tensor) -> torch.Tensor:
+        """Contiguous and 16-byte aligned, as the _embeds entries load rows as float4."""
+        states = states.contiguous()
+        return states.clone() if states.data_ptr() % 16 else states
+
     def policy_prefill(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,
-                       rewards: Optional[torch.Tensor] = None, flags: int = 0, lengths=None):
+                       rewards: Optional[torch.Tensor] = None, flags: int = 0, lengths=None,
+                       state_embeds: bool = False):
         """Warm the recurrent state with Tn timesteps of context per env: states [B,Tn,state_dim], rtg [B,Tn],
         rewards [B,Tn] or None (= the 0 placeholder the rollout feeds). No action outputs (xl_policy_prefill).
         `lengths` (B ints in [0, Tn]): env b takes its first lengths[b] timesteps only, an env with 0 keeps its state
-        (xl_policy_prefill_ragged). Checked before anything reaches the library."""
+        (xl_policy_prefill_ragged). With `state_embeds=True`, `states` is instead the state-token embedding of every
+        timestep, fp32 [B,Tn,d] on this engine's device (image observations: `image_encoder.embed_frames`), and
+        embed_state is skipped (xl_policy_prefill_embeds). Checked before anything reaches the library."""
+        if state_embeds:
+            self._check_state_embeds(states, state.B)
         lens = None if lengths is None else check_lengths(lengths, state.B, states.shape[1], "Tn")
-        return self._policy_prefill(state, states, rtg, rewards, flags, lens)
+        return self._policy_prefill(state, states, rtg, rewards, flags, lens, state_embeds)
 
     @_on_device
-    def _policy_prefill(self, state, states, rtg, rewards, flags, lens):
+    def _policy_prefill(self, state, states, rtg, rewards, flags, lens, state_embeds=False):
         cfg = self.cfg
         B, Tn = state.B, states.shape[1]
-        assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == (B, Tn, cfg.state_dim)
+        assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == \
+            (B, Tn, cfg.d if state_embeds else cfg.state_dim)
         assert rtg.is_cuda and rtg.dtype == torch.float32 and rtg.numel() == B * Tn
         states, rtg = states.contiguous(), rtg.contiguous()
         if rewards is not None:
             rewards = rewards.to(self.device, torch.float32).contiguous()
             assert rewards.numel() == B * Tn
-        if lens is None:
+        if state_embeds:
+            L.check(self.lib.xl_policy_prefill_embeds(
+                self.handle, _ptr(state.buf), _ptr(self._embeds_operand(states)), _ptr(rtg), _ptr(rewards),
+                None if lens is None else lens.ctypes.data_as(C.c_void_p), B, Tn, flags, self._stream()))
+        elif lens is None:
             L.check(self.lib.xl_policy_prefill(self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards), B,
                                                Tn, flags, self._stream()))
         else:
@@ -367,7 +395,8 @@ class XLSTMEngine:
 
     def policy_forward(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,
                        rewards: Optional[torch.Tensor] = None, lengths=None, discrete: bool = False,
-                       targets: Optional[torch.Tensor] = None, want_logits: bool = False) -> dict:
+                       targets: Optional[torch.Tensor] = None, want_logits: bool = False,
+                       state_embeds: bool = False) -> dict:
         """Action outputs of every timestep of whole trajectories in one chunkwise pass (xl_policy_forward): what
         `policy_step` would return at each timestep when stepped from `state` over states [B,Tn,state_dim], rtg [B,Tn],
         rewards [B,Tn] or None (= 0). The state ends where `policy_prefill` on the same arguments leaves it.
@@ -377,9 +406,14 @@ class XLSTMEngine:
         values in [-1, num_actions); -1 = a padded action dim, scored 0) "action_logprobs" [B,Tn,act_dim]: the log-softmax
         of each action row's logits at the target (discrete: column 0). `lengths` (B ints in [0, Tn]) gives env b its
         first lengths[b] timesteps only; outputs past them are -1 / 0 and an env with 0 keeps its state.
-        Lengths and targets are checked before anything reaches the library; the range check of `targets` costs one
-        device reduction and a synchronisation."""
+        With `state_embeds=True`, `states` is the state-token embedding of every timestep, fp32 [B,Tn,d] on this
+        engine's device (image observations: `image_encoder.embed_frames`), as `policy_step(state_embeds=True)` takes
+        it (xl_policy_forward_embeds).
+        Lengths, targets and embeddings are checked before anything reaches the library; the range check of `targets`
+        costs one device reduction and a synchronisation."""
         cfg = self.cfg
+        if state_embeds:
+            self._check_state_embeds(states, state.B)
         B, Tn = state.B, states.shape[1]
         lens = None if lengths is None else check_lengths(lengths, B, Tn, "Tn")
         if targets is not None:
@@ -395,13 +429,14 @@ class XLSTMEngine:
                 lo, hi = (int(v) for v in torch.aminmax(targets))
                 if lo < -1 or hi >= cfg.num_actions:
                     raise ValueError(f"targets must lie in [-1, num_actions={cfg.num_actions}), got min {lo} max {hi}")
-        return self._policy_forward(state, states, rtg, rewards, lens, discrete, targets, want_logits)
+        return self._policy_forward(state, states, rtg, rewards, lens, discrete, targets, want_logits, state_embeds)
 
     @_on_device
-    def _policy_forward(self, state, states, rtg, rewards, lens, discrete, targets, want_logits):
+    def _policy_forward(self, state, states, rtg, rewards, lens, discrete, targets, want_logits, state_embeds=False):
         cfg = self.cfg
         B, Tn = state.B, states.shape[1]
-        assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == (B, Tn, cfg.state_dim)
+        assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == \
+            (B, Tn, cfg.d if state_embeds else cfg.state_dim)
         assert rtg.is_cuda and rtg.dtype == torch.float32 and rtg.numel() == B * Tn
         states, rtg = states.contiguous(), rtg.contiguous()
         if rewards is not None:
@@ -418,7 +453,10 @@ class XLSTMEngine:
         so = L.XLSeqOutputs(tokens=out["action_tokens"].data_ptr(), actions=out["action_preds"].data_ptr(),
                             logits=_ptr(out.get("action_logits")).value, targets=_ptr(targets).value,
                             logprobs=_ptr(out.get("action_logprobs")).value)
-        L.check(self.lib.xl_policy_forward(
+        if state_embeds:
+            states = self._embeds_operand(states)
+        fn = self.lib.xl_policy_forward_embeds if state_embeds else self.lib.xl_policy_forward
+        L.check(fn(
             self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards),
             None if lens is None else lens.ctypes.data_as(C.c_void_p), B, Tn, C.byref(so),
             L.XL_FLAG_DISCRETE if discrete else 0, self._stream()))

@@ -10,7 +10,8 @@ Per SURVEY.md §8 a12 this stage stays in PyTorch / cuDNN (it is not on the HBM-
 stages of conv3x3 -> maxpool(3, stride 2, pad 1) -> 2 residual units (relu -> conv3x3 -> relu -> conv3x3, skip),
 channels 16/32/32 x model_size, then ReLU, flatten, Linear(n_flat -> d), ReLU. Parameter names equal the
 reference's, so `embed_image.*` entries of an LRAM checkpoint load with `load_state_dict`. The resulting state
-embeddings [B, d] enter the CUDA path through `xl_policy_step(..., XL_FLAG_STATE_EMBEDS)`.
+embeddings [B, d] enter the CUDA path through `xl_policy_step(..., XL_FLAG_STATE_EMBEDS)`; whole trajectories
+([B, T, d] from `embed_frames`) through `xl_policy_prefill_embeds` / `xl_policy_forward_embeds`.
 (Spectral-norm and modulation-vector variants of the reference class are training options, unused by the
 multi_domain configuration, and are not reproduced.)
 """
@@ -18,6 +19,7 @@ from __future__ import annotations
 
 from typing import Dict, Sequence
 
+import numpy as np
 import torch
 import torch.nn as nn
 import torch.nn.functional as F
@@ -76,6 +78,37 @@ def scale_frames(frames: torch.Tensor) -> torch.Tensor:
     reach the policy as raw 0..255 values whether their dtype is uint8 or — after `pad_inputs` returned
     `states.float()` (src/algos/decision_xlstm.py:25) — float."""
     return frames.float() / 255.0
+
+
+@torch.no_grad()
+def embed_frames(cnn: ImpalaCNN, frames: torch.Tensor, lengths=None, max_frames: int = 2048) -> torch.Tensor:
+    """State embeddings of whole trajectories of raw frames, the input of the sequence calls with `state_embeds=True`
+    (`XLSTMEngine.policy_forward` / `policy_prefill`): frames [B, T, C, H, W], uint8 or float with values 0..255, on
+    any device -> fp32 [B, T, d] on the CNN's device. `scale_frames` is applied once per frame, and the CNN runs on at
+    most `max_frames` frames at a time (at T in the tens of thousands one batch of first-stage activations would not
+    fit). `lengths` (B ints in [0, T]): frames at or past lengths[b] are never fed to the CNN and their rows are 0."""
+    if not isinstance(frames, torch.Tensor) or frames.dim() != 5:
+        raise ValueError(f"frames must be a [B, T, C, H, W] tensor, got {getattr(frames, 'shape', type(frames))}")
+    if tuple(frames.shape[2:]) != tuple(cnn.image_shape):
+        raise ValueError(f"frames must be [B, T, {', '.join(map(str, cnn.image_shape))}], got {tuple(frames.shape)}")
+    if max_frames < 1:
+        raise ValueError(f"max_frames={max_frames} must be positive")
+    B, T = frames.shape[:2]
+    dev = cnn.linear[0].weight.device
+    out = torch.zeros(B, T, cnn.linear[0].out_features, dtype=torch.float32, device=dev)
+    flat, out_flat = frames.reshape(B * T, *frames.shape[2:]), out.view(B * T, -1)
+    if lengths is None:
+        for i in range(0, B * T, max_frames):
+            out_flat[i:i + max_frames] = cnn(scale_frames(flat[i:i + max_frames].to(dev)))
+        return out
+    from .engine import check_lengths
+    lens = torch.from_numpy(check_lengths(lengths, B, T, "T").astype(np.int64))
+    rows = (torch.arange(T).view(1, T) < lens.view(B, 1)).view(-1).nonzero().view(-1)   # valid frames, in order
+    for i in range(0, rows.numel(), max_frames):
+        idx = rows[i:i + max_frames]
+        x = flat.index_select(0, idx.to(flat.device))
+        out_flat.index_copy_(0, idx.to(dev), cnn(scale_frames(x.to(dev))))
+    return out
 
 
 def make_impala_state_dict(features_dim: int, image_shape: Sequence[int] = (3, 64, 64), seed: int = 0,
