@@ -133,7 +133,8 @@ struct xl_handle {
                                        // envs; -0.3 % at >= 1 GB, where nothing prefetched survives until it is read)
   // context-prefill workspace (lazily allocated by xl_prefill / xl_policy_prefill, grow-only)
   char* pf_buf = nullptr;
-  int pf_rows = 0;
+  int pf_rows = 0;                              // rows of every [rows, ...] buffer
+  size_t pf_gsc_floats = 0;                     // floats of the gate-scan scratch pf_gsc
   float *pf_x = nullptr, *pf_xn = nullptr, *pf_u = nullptr, *pf_qkv = nullptr, *pf_act = nullptr, *pf_gp = nullptr,
         *pf_gated = nullptr, *pf_num = nullptr, *pf_qn = nullptr, *pf_f = nullptr, *pf_i = nullptr, *pf_m = nullptr,
         *pf_semb = nullptr, *pf_spad = nullptr, *pf_sin = nullptr, *pf_rtg = nullptr, *pf_rew = nullptr, *pf_gsc = nullptr;
@@ -884,8 +885,11 @@ int run_policy(xl_handle* h, const StepArgs& a, cudaStream_t s) {
 }
 
 // ---- context prefill ----------------------------------------------------------------------------------
-int ensure_prefill_ws(xl_handle* h, int rows) {
-  if (rows <= h->pf_rows) return XL_OK;
+// Grows the workspace to `rows` rows and `gsc_floats` floats of gate-scan scratch (never shrinks either).
+int ensure_prefill_ws(xl_handle* h, int rows, size_t gsc_floats) {
+  if (rows <= h->pf_rows && gsc_floats <= h->pf_gsc_floats) return XL_OK;
+  rows = std::max(rows, h->pf_rows);
+  gsc_floats = std::max(gsc_floats, h->pf_gsc_floats);
   const xl_config& c = h->cfg;
   const size_t d = c.embedding_dim, inner = c.inner_dim, NH = c.num_heads, R = (size_t)rows;
   const size_t kmax = std::max(std::max(inner, d), (size_t)h->Kpad);
@@ -901,8 +905,7 @@ int ensure_prefill_ws(xl_handle* h, int rows) {
   const size_t o_f = carve(4 * R * NH), o_i = carve(4 * R * NH), o_m = carve(4 * R * NH);
   const size_t o_semb = carve(4 * R * d), o_spad = carve(4 * R * h->Kpad), o_sin = carve(4 * R * c.state_dim);
   const size_t o_rtg = carve(4 * R), o_rew = carve(4 * R);
-  // gate-scan maps: B*NH*(1 + 2*ceil(S/2048)) floats with B <= R/48 + 1 envs of S = R/B tokens
-  const size_t o_gsc = carve(4 * NH * (3 * (R / 48 + 16) + R / 1024 + 16));
+  const size_t o_gsc = carve(4 * gsc_floats);
   const size_t o_hi = carve(2 * R * kmax), o_lo = carve(2 * R * kmax);
   size_t pc_bytes = 0, pv_bytes = 0;
   if (xl::prefill_cell_mma_supported(h->DH)) xl::prefill_cell_mma_ws(rows, (int)NH, h->DH, &pc_bytes, &pv_bytes);
@@ -911,6 +914,7 @@ int ensure_prefill_ws(xl_handle* h, int rows) {
   if (h->pf_buf) cudaFree(h->pf_buf);
   h->pf_buf = nullptr;
   h->pf_rows = 0;
+  h->pf_gsc_floats = 0;
   cudaError_t e = cudaMalloc((void**)&h->pf_buf, off);
   if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaMalloc(prefill workspace %zu B) failed: %s", off, cudaGetErrorString(e));
   char* b = h->pf_buf;
@@ -924,6 +928,7 @@ int ensure_prefill_ws(xl_handle* h, int rows) {
   h->pf_hi = (__nv_bfloat16*)(b + o_hi); h->pf_lo = (__nv_bfloat16*)(b + o_lo);
   h->pf_pc = (uint8_t*)(b + o_pc); h->pf_pv = (uint8_t*)(b + o_pv);
   h->pf_rows = rows;
+  h->pf_gsc_floats = gsc_floats;
   return XL_OK;
 }
 
@@ -1054,21 +1059,28 @@ bool prefill_fast_path(const xl_handle* h) {
   return xl::prefill_cell_supported(h->DH) && h->cfg.conv_kernel == 4;
 }
 
-// ---- ragged prefill ----------------------------------------------------------------------------------------------
-// The active envs (length > 0) sorted by length, descending and stable: compact env k is caller env perm[k]. Once sorted,
-// the envs that still have tokens at position pos are a prefix Bk of the compact batch, so every chunk runs the
-// sequence kernels on that prefix (same base pointers, smaller B) and pads each env's end up to the chunk's length with
-// identity tokens. If the active envs already are envs 0..Bc-1 in that order, the chunks work on the caller's state in
-// place; otherwise the state is gathered into a compact one of Bc envs and scattered back at the end.
-struct RaggedPlan {
-  std::vector<int32_t> perm, len;     // len: in the caller's units (tokens or timesteps)
-  bool in_place = false;
+// ---- sequence plan -------------------------------------------------------------------------------------------------
+// Every sequence call (context prefill, policy prefill, sequence forward) runs chunks {pos, Bk, n}: units
+// [pos, pos + n) of the first Bk envs of the state the chunks advance, a unit being T tokens (1: encoder tokens;
+// tokens_per_step: timesteps). Units from `tail` on run as eager steps.
+// Uniform call (no lengths): all B envs of the caller's state, perm / len null.
+// Ragged call: the active envs (length > 0) sorted by length, descending and stable: compact env k is caller env perm[k].
+// Once sorted, the envs that still have tokens at position pos are a prefix Bk of the compact batch, so every chunk runs
+// the sequence kernels on that prefix (same base pointers, smaller B) and pads each env's end up to the chunk's length
+// with identity tokens. If the active envs already are envs 0..Bc-1 in that order, the chunks work on the caller's state
+// in place; otherwise the state is gathered into a compact one of Bc envs and scattered back at the end.
+struct SeqChunk {
+  int pos, Bk, n;
+};
+struct SeqPlan {
+  int T = 1;                          // tokens per unit
+  std::vector<SeqChunk> chunks;
+  int tail = 0;                       // first unit of the eager tail
+  std::vector<int32_t> perm, len;     // ragged: len in units
+  bool in_place = true;
   void* st = nullptr;                 // the state the chunks advance
   int Btot = 0;                       // envs of its layout
-  const int32_t *d_perm = nullptr, *d_len = nullptr;   // device copies; d_len in tokens
-};
-struct RaggedChunk {
-  int pos, Bk, n;                     // units [pos, pos + n) of the first Bk compact envs
+  const int32_t *d_perm = nullptr, *d_len = nullptr;   // ragged: device copies, d_len in tokens; uniform: null
 };
 
 int check_lengths(const int32_t* lengths, int B, int S, const char* what) {
@@ -1098,13 +1110,12 @@ xl::StateCopyGeom state_copy_geom(const xl_handle* h, int B, int Bc) {
   return g;
 }
 
-// Sort, upload the index, and gather the state when the active envs are not a sorted prefix. tok = tokens per unit.
-int ragged_begin(xl_handle* h, void* state, const int32_t* lengths, int B, int tok, RaggedPlan& p, cudaStream_t s) {
+// Sort, upload the index, and gather the state when the active envs are not a sorted prefix.
+int ragged_begin(xl_handle* h, void* state, const int32_t* lengths, int B, SeqPlan& p, cudaStream_t s) {
   for (int b = 0; b < B; ++b)
     if (lengths[b] > 0) p.perm.push_back(b);
   std::stable_sort(p.perm.begin(), p.perm.end(), [&](int a, int b) { return lengths[a] > lengths[b]; });
   const int Bc = (int)p.perm.size();
-  p.in_place = true;
   for (int k = 0; k < Bc; ++k) {
     p.len.push_back(lengths[p.perm[k]]);
     p.in_place = p.in_place && p.perm[k] == k;
@@ -1113,7 +1124,7 @@ int ragged_begin(xl_handle* h, void* state, const int32_t* lengths, int B, int t
   h->rg_host.assign(2 * (size_t)Bc, 0);
   for (int k = 0; k < Bc; ++k) {
     h->rg_host[k] = p.perm[k];
-    h->rg_host[Bc + k] = p.len[k] * tok;
+    h->rg_host[Bc + k] = p.len[k] * p.T;
   }
   XL_CUDA(cudaMemcpyAsync(h->rg_idx, h->rg_host.data(), sizeof(int32_t) * 2 * (size_t)Bc, cudaMemcpyHostToDevice, s));
   p.d_perm = h->rg_idx;
@@ -1142,7 +1153,7 @@ int ragged_begin(xl_handle* h, void* state, const int32_t* lengths, int B, int t
   return XL_OK;
 }
 
-int ragged_end(xl_handle* h, void* state, int B, const RaggedPlan& p, cudaStream_t s) {
+int ragged_end(xl_handle* h, void* state, int B, const SeqPlan& p, cudaStream_t s) {
   if (p.in_place) return XL_OK;
   const int Bc = (int)p.perm.size();
   xl::launch_state_permute(state, h->rg_state, p.d_perm, Bc, state_copy_geom(h, B, Bc), 1, s);
@@ -1151,27 +1162,79 @@ int ragged_end(xl_handle* h, void* state, int B, const RaggedPlan& p, cudaStream
   return XL_OK;
 }
 
-// Chunks of the shrinking active prefix, in units of T tokens (1: encoder tokens; tokens_per_step: timesteps): today's
-// chunk length for Bk envs (prefill_chunk_tokens), cut to the longest remaining context rounded up to 8 units (16 where
-// the chunkwise cells run: whole 16-token chunks of the mma.sync cell). Grows the prefill workspace to the largest.
-int ragged_chunks(xl_handle* h, const std::vector<int32_t>& len, int T, std::vector<RaggedChunk>& out) {
+// Chunks of the shrinking active prefix: today's chunk length for Bk envs (prefill_chunk_tokens), cut to the longest
+// remaining context rounded up to 8 units (16 where the chunkwise cells run: whole 16-token chunks of the mma.sync cell).
+void ragged_chunks(const xl_handle* h, SeqPlan& p) {
   const int gran = (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(h->DH)) ? 16 : 8;
-  int pos = 0, Bk = (int)len.size(), rows = 0;
+  const std::vector<int32_t>& len = p.len;
+  int pos = 0, Bk = (int)len.size();
   while (pos < len[0]) {
     while (len[Bk - 1] <= pos) --Bk;
-    const int cmax = prefill_chunk_tokens(h, Bk) / T;
+    const int cmax = prefill_chunk_tokens(h, Bk) / p.T;
     const int n = std::min(cmax, (len[0] - pos + gran - 1) / gran * gran);
-    out.push_back({pos, Bk, n});
-    // >= 48 tokens per env: room for the gate-scan maps of short chunks (ensure_prefill_ws sizes them for that)
-    rows = std::max(rows, Bk * std::max(n * T, 48));
+    p.chunks.push_back({pos, Bk, n});
     pos += n;
   }
-  return ensure_prefill_ws(h, rows);
 }
 
-// ---- sequence forward: the head hook of the policy-prefill loops --------------------------------------------------
-// With a hook, the loops also emit the action outputs of every timestep (xl_policy_forward); without one they are
-// xl_policy_prefill / xl_policy_prefill_ragged unchanged. The hook only reads what the loops leave behind.
+// Chunks of all B envs, each a multiple of 8 units (of 16 where the mma.sync cell runs; an 8-unit remainder takes the
+// fp32 cell); the last S mod 8 units, and every unit of a shape without the sequence path, form the eager tail.
+void uniform_chunks(const xl_handle* h, int B, int S, SeqPlan& p) {
+  int pos = 0;
+  if (prefill_fast_path(h)) {
+    const int cmax = prefill_chunk_tokens(h, B) / p.T;
+    while (S - pos >= 8) {
+      int n = std::min(cmax, (S - pos) / 8 * 8);
+      if (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(h->DH) && n >= 16) n = n / 16 * 16;
+      p.chunks.push_back({pos, B, n});
+      pos += n;
+    }
+  }
+  p.tail = pos;
+}
+
+// The plan of one call of B envs x S units (lengths: host, or nullptr for a uniform call), the ragged state gathered,
+// and the prefill workspace grown to its largest chunk: rows, and the gate-scan scratch of gate_pre_seq_kernel.
+int seq_plan(xl_handle* h, void* state, const int32_t* lengths, int B, int S, SeqPlan& p, cudaStream_t s) {
+  if (lengths) {
+    if (int rc = ragged_begin(h, state, lengths, B, p, s)) return rc;
+    ragged_chunks(h, p);
+    p.tail = S;
+  } else {
+    p.st = state;
+    p.Btot = B;
+    uniform_chunks(h, B, S, p);
+  }
+  int rows = 0;
+  size_t gsc = 0;
+  for (const SeqChunk& ch : p.chunks) {
+    rows = std::max(rows, ch.Bk * ch.n * p.T);
+    gsc = std::max(gsc, xl::gate_scan_seq_scratch_floats(ch.Bk, ch.n * p.T, h->cfg.num_heads));
+  }
+  return ensure_prefill_ws(h, rows, gsc);
+}
+
+// Moves chunk ch's rows between a caller's [B, S, width] buffer and a chunk buffer [Bk, n, width]: to the chunk
+// (to_caller 0; ragged pads zero-filled) or back to the caller (to_caller 1; ragged: valid rows only).
+int chunk_rows(xl_handle* h, const SeqPlan& p, const SeqChunk& ch, float* caller, float* chunk, int S, int width,
+               int to_caller, cudaStream_t s) {
+  if (p.d_len) {
+    xl::launch_ragged_rows(caller, chunk, p.d_perm, p.d_len, p.T, ch.Bk, S, ch.n, ch.pos, width, to_caller, s);
+    h->launches += 1;
+    return XL_OK;
+  }
+  const size_t cpitch = sizeof(float) * (size_t)S * width, kpitch = sizeof(float) * (size_t)ch.n * width;
+  float* c = caller + (size_t)ch.pos * width;
+  if (to_caller)
+    XL_CUDA(cudaMemcpy2DAsync(c, cpitch, chunk, kpitch, kpitch, ch.Bk, cudaMemcpyDeviceToDevice, s));
+  else
+    XL_CUDA(cudaMemcpy2DAsync(chunk, kpitch, c, cpitch, kpitch, ch.Bk, cudaMemcpyDeviceToDevice, s));
+  return XL_OK;
+}
+
+// ---- sequence forward: the action head of every timestep ----------------------------------------------------------
+// The forward calls run the policy prefill and also emit the action outputs of every timestep from what each chunk (and
+// each eager tail step) leaves behind, so their state is the prefill's.
 struct SeqHead {
   xl_seq_outputs out;
   int discrete, n_out, Tn;
@@ -1779,57 +1842,6 @@ int xl_policy_step_host(xl_handle* h, void* state, const float* h_states, const 
   return XL_OK;
 }
 
-int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B, int S, unsigned flags, void* stream) {
-  int rc = check_batch(h, B);
-  if (rc) return rc;
-  if (!state || !x_in) return fail(XL_ERR_INVALID_ARG, "null argument");
-  if (S <= 0) return fail(XL_ERR_INVALID_ARG, "S=%d must be positive", S);
-  rc = weights_ready(h, true);
-  if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
-  const xl_config& c = h->cfg;
-  const int d = c.embedding_dim;
-  const float* post_w = (const float*)h->pw[XL_W_POST_NORM - XL_W_POST_NORM];
-  int pos = 0;
-  if (prefill_fast_path(h)) {
-    const int sc_max = prefill_chunk_tokens(h, B);
-    while (S - pos >= 8) {
-      int Sc = std::min(sc_max, (S - pos) / 8 * 8);
-      // whole 16-token chunks go to the tensor-core cell; an 8-token remainder takes the fp32 cell next round
-      if (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(h->DH) && Sc >= 16) Sc = Sc / 16 * 16;
-      rc = ensure_prefill_ws(h, B * Sc);
-      if (rc) return rc;
-      XL_CUDA(cudaMemcpy2DAsync(h->pf_x, sizeof(float) * (size_t)Sc * d, x_in + (size_t)pos * d,
-                                sizeof(float) * (size_t)S * d, sizeof(float) * (size_t)Sc * d, B,
-                                cudaMemcpyDeviceToDevice, s));
-      rc = prefill_blocks(h, state, B, B, Sc, flags, s);
-      if (rc) return rc;
-      if (y_out) {
-        xl::launch_ln_rows(h->pf_x, d, h->pf_xn, d, post_w, nullptr, 1, c.ln_eps, B * Sc, d, nullptr, nullptr, s);
-        h->launches += 1;
-        XL_CUDA(cudaMemcpy2DAsync(y_out + (size_t)pos * d, sizeof(float) * (size_t)S * d, h->pf_xn,
-                                  sizeof(float) * (size_t)Sc * d, sizeof(float) * (size_t)Sc * d, B,
-                                  cudaMemcpyDeviceToDevice, s));
-      }
-      pos += Sc;
-    }
-  }
-  // remaining tokens (and shapes the sequence kernels do not cover): fused recurrent steps of <= 4 tokens
-  const Slice sl = make_slice(h, B, 0, B, s);
-  while (pos < S) {
-    const int T = std::min(4, S - pos);
-    XL_CUDA(cudaMemcpy2DAsync(sl.ws.x, sizeof(float) * (size_t)T * d, x_in + (size_t)pos * d,
-                              sizeof(float) * (size_t)S * d, sizeof(float) * (size_t)T * d, B, cudaMemcpyDeviceToDevice, s));
-    rc = run_encoder(h, state, sl, sl.ws.x, sl.ws.hid, T, XL_MODE_FUSED, flags);
-    if (rc) return rc;
-    if (y_out)
-      XL_CUDA(cudaMemcpy2DAsync(y_out + (size_t)pos * d, sizeof(float) * (size_t)S * d, sl.ws.hid,
-                                sizeof(float) * (size_t)T * d, sizeof(float) * (size_t)T * d, B, cudaMemcpyDeviceToDevice, s));
-    pos += T;
-  }
-  return XL_OK;
-}
-
 // Tokens of one prefill chunk (Bk envs x Tc timesteps from timestep pos) straight from given state embeddings
 // [B, Tn, d] into pf_x: one launch where raw states take a staging copy, pad_rows, the embed_state Linear and the embed
 // kernel. perm / len as in launch_ragged_rows (nullptr: envs 0..Bk-1, every timestep valid).
@@ -1849,253 +1861,204 @@ static void seq_embed_chunk(xl_handle* h, const float* embeds, const float* rtg,
   h->launches += 1;
 }
 
-// xl_policy_prefill; with a head hook (xl_policy_forward) also the action outputs of every timestep. With
-// XL_FLAG_STATE_EMBEDS (the _embeds entries) `states` holds state embeddings [B, Tn, d].
-static int policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
-                          int Tn, unsigned flags, void* stream, const SeqHead* head) {
-  int rc = check_batch(h, B);
+// One call of the sequence path; each entry point below only fills this in.
+struct SeqCall {
+  enum Input { kTokens, kStates, kEmbeds };
+  const char* fn;                     // the entry point, for messages
+  Input in;                           // x: encoder tokens [B, S, d], raw states [B, S, state_dim] or state embeddings [B, S, d]
+  void* state;
+  const float *x, *rtg, *rewards;     // rtg / rewards [B, S] of the policy forms (rewards nullable)
+  const int32_t* lengths;             // host [B] in units, or nullptr
+  int B, S;                           // S in units: tokens (encoder) or timesteps (policy)
+  unsigned flags;
+  void* stream;
+  bool ragged = false;                // lengths are required (the _ragged entries)
+  float* y_out = nullptr;             // encoder: post_blocks_norm hidden states [B, S, d], nullable
+  bool head = false;                  // forward entries: the action outputs of every timestep go to *out
+  const xl_seq_outputs* out = nullptr;
+  SeqCall(const char* fn, Input in, void* state, const float* x, const float* rtg, const float* rewards,
+          const int32_t* lengths, int B, int S, unsigned flags, void* stream)
+      : fn(fn), in(in), state(state), x(x), rtg(rtg), rewards(rewards), lengths(lengths), B(B), S(S), flags(flags),
+        stream(stream) {}
+};
+
+// Validate; all lengths full -> the uniform call; plan; per chunk: stage the inputs, the block stack, the outputs;
+// scatter the state back; the eager tail of a uniform call.
+static int run_seq(xl_handle* h, SeqCall c) {
+  const bool enc = c.in == SeqCall::kTokens;
+  if (c.head) {
+    if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+    if (!c.out) return fail(XL_ERR_INVALID_ARG, "null outputs");
+    if (c.out->logprobs && !c.out->targets) return fail(XL_ERR_INVALID_ARG, "logprobs need targets");
+  }
+  if (c.in == SeqCall::kStates && (c.flags & XL_FLAG_STATE_EMBEDS))   // they would be read as [B, S, state_dim] rows
+    return fail(XL_ERR_UNSUPPORTED, "%s takes raw states; state embeddings go through xl_policy_prefill_embeds / "
+                                    "xl_policy_forward_embeds", c.fn);
+  if (c.in == SeqCall::kEmbeds) {
+    if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+    if ((uintptr_t)c.x % 16)
+      return fail(XL_ERR_INVALID_ARG, "state_embeds must be 16-byte aligned (rows are loaded as float4)");
+    c.flags |= XL_FLAG_STATE_EMBEDS;
+  }
+  int rc = check_batch(h, c.B);
   if (rc) return rc;
-  if (!state || !states || !rtg) return fail(XL_ERR_INVALID_ARG, "null argument");
-  if (Tn <= 0) return fail(XL_ERR_INVALID_ARG, "Tn=%d must be positive", Tn);
-  rc = xl_weights_ready(h);
-  if (rc) return rc;
-  cudaStream_t s = (cudaStream_t)stream;
-  const xl_config& c = h->cfg;
-  const int d = c.embedding_dim, sd = c.state_dim, T = c.tokens_per_step;
-  const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
-  auto PW = [&](int id) { return h->pw[id - XL_W_POST_NORM]; };
-  const bool embeds = (flags & XL_FLAG_STATE_EMBEDS) != 0;
-  const int sw = embeds ? d : sd;   // row width of `states`
-  int pos = 0;   // timesteps done
-  if (prefill_fast_path(h)) {
-    const int tc_max = prefill_chunk_tokens(h, B) / T;
-    while (Tn - pos >= 8) {
-      int Tc = std::min(tc_max, (Tn - pos) / 8 * 8);             // 8 timesteps = 24 tokens = 3 cell stages
-      // 16 timesteps = 48 tokens = 3 chunks of the tensor-core cell; an 8-timestep remainder takes the fp32 cell
-      if (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(h->DH) && Tc >= 16) Tc = Tc / 16 * 16;
-      const int rows = B * Tc;
-      rc = ensure_prefill_ws(h, rows * T);
-      if (rc) return rc;
-      if (embeds) {
-        seq_embed_chunk(h, states, rtg, rewards, nullptr, nullptr, B, Tn, Tc, pos, s);
-      } else {
-        const Ws ws = prefill_ws(h);
-        // gather the chunk's timesteps of every env: [B, Tc, sd], [B, Tc]
-        XL_CUDA(cudaMemcpy2DAsync(h->pf_sin, sizeof(float) * (size_t)Tc * sd, states + (size_t)pos * sd,
-                                  sizeof(float) * (size_t)Tn * sd, sizeof(float) * (size_t)Tc * sd, B,
-                                  cudaMemcpyDeviceToDevice, s));
-        XL_CUDA(cudaMemcpy2DAsync(h->pf_rtg, sizeof(float) * (size_t)Tc, rtg + pos, sizeof(float) * (size_t)Tn,
-                                  sizeof(float) * (size_t)Tc, B, cudaMemcpyDeviceToDevice, s));
-        if (rewards)
-          XL_CUDA(cudaMemcpy2DAsync(h->pf_rew, sizeof(float) * (size_t)Tc, rewards + pos, sizeof(float) * (size_t)Tn,
-                                    sizeof(float) * (size_t)Tc, B, cudaMemcpyDeviceToDevice, s));
-        // embed: rows (env, timestep) -> tokens (env, timestep, {s, rtg, r}) == the env's sequence order
-        xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
-        h->launches += 1;
-        rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
-                    rows, d, h->Kpad, impl, s);
-        if (rc) return rc;
-        xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
-                                (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
-                                (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
-                                (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
-                                0.f, nullptr, nullptr, nullptr, s);
-        h->launches += 1;
-      }
-      rc = prefill_blocks(h, state, B, B, Tc * T, flags, s);
-      if (rc) return rc;
-      if (head && (rc = seq_head_chunk(h, *head, B, Tc, pos, nullptr, nullptr, flags, s))) return rc;
-      pos += Tc;
+  if (!c.state || !c.x || (!enc && !c.rtg)) return fail(XL_ERR_INVALID_ARG, "null argument");
+  const char* unit = enc ? "S" : "Tn";
+  if (c.S <= 0) return fail(XL_ERR_INVALID_ARG, "%s=%d must be positive", unit, c.S);
+  if ((c.lengths || c.ragged) && (rc = check_lengths(c.lengths, c.B, c.S, unit))) return rc;
+  if ((rc = weights_ready(h, enc))) return rc;
+  cudaStream_t s = (cudaStream_t)c.stream;
+  const xl_config& cf = h->cfg;
+  const int B = c.B, S = c.S, d = cf.embedding_dim, sd = cf.state_dim;
+  SeqHead hd;
+  const SeqHead* head = nullptr;
+  if (c.head) {
+    hd.out = *c.out;
+    hd.discrete = (c.flags & XL_FLAG_DISCRETE) ? 1 : 0;
+    hd.n_out = hd.discrete ? h->num_actions : h->head_out;
+    hd.Tn = S;
+    head = &hd;
+  }
+  const int32_t* lengths = c.lengths;
+  if (lengths) {
+    const int nfull = (int)std::count(lengths, lengths + B, S), nzero = (int)std::count(lengths, lengths + B, 0);
+    if (nfull == B) {
+      lengths = nullptr;          // the uniform call, bit for bit
+    } else {
+      if (nzero < B && !prefill_fast_path(h))
+        return fail(XL_ERR_UNSUPPORTED, "ragged prefill needs the sequence path (conv_kernel 4, a cell plan for DH=%d)",
+                    h->DH);
+      // output positions past an env's length keep these values (y_out 0; tokens -1, the rest 0)
+      if (c.y_out) XL_CUDA(cudaMemsetAsync(c.y_out, 0, sizeof(float) * (size_t)B * S * d, s));
+      if (head && (rc = seq_clear_outputs(h, hd, B, s))) return rc;
+      if (nzero == B) return XL_OK;
     }
   }
-  // remaining timesteps: ordinary fused policy steps, outputs discarded (head hook: their logits are reduced as a chunk
-  // of one timestep)
-  if (head && pos < Tn && (rc = ensure_seq_logits(h, (size_t)B * head->n_out))) return rc;
-  for (; pos < Tn; ++pos) {
-    float* stage = embeds ? h->d_embeds : h->d_states;
-    XL_CUDA(cudaMemcpy2DAsync(stage, sizeof(float) * (size_t)sw, states + (size_t)pos * sw,
-                              sizeof(float) * (size_t)Tn * sw, sizeof(float) * (size_t)sw, B, cudaMemcpyDeviceToDevice, s));
-    XL_CUDA(cudaMemcpy2DAsync(h->d_rtg, sizeof(float), rtg + pos, sizeof(float) * (size_t)Tn, sizeof(float), B,
-                              cudaMemcpyDeviceToDevice, s));
-    if (rewards)
-      XL_CUDA(cudaMemcpy2DAsync(h->d_rew, sizeof(float), rewards + pos, sizeof(float) * (size_t)Tn, sizeof(float), B,
-                                cudaMemcpyDeviceToDevice, s));
+  SeqPlan p;
+  p.T = enc ? 1 : cf.tokens_per_step;
+  if ((rc = seq_plan(h, c.state, lengths, B, S, p, s))) return rc;
+  auto gather = [&](const SeqChunk& ch, const float* src, float* dst, int width) {
+    return chunk_rows(h, p, ch, const_cast<float*>(src), dst, S, width, 0, s);
+  };
+  const Ws ws = prefill_ws(h);
+  const int impl = (c.flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
+  auto PW = [&](int id) { return (const float*)h->pw[id - XL_W_POST_NORM]; };
+  for (const SeqChunk& ch : p.chunks) {
+    const int rows = ch.Bk * ch.n;
+    if (c.in == SeqCall::kTokens) {
+      if ((rc = gather(ch, c.x, ws.x, d))) return rc;
+    } else if (c.in == SeqCall::kEmbeds) {
+      seq_embed_chunk(h, c.x, c.rtg, c.rewards, p.d_perm, p.d_len, ch.Bk, S, ch.n, ch.pos, s);
+    } else {
+      // the chunk's timesteps [Bk, n, state_dim], [Bk, n], then embed: rows (env, timestep) -> tokens
+      // (env, timestep, {s, rtg, r}) == the env's sequence order
+      if ((rc = gather(ch, c.x, h->pf_sin, sd)) || (rc = gather(ch, c.rtg, h->pf_rtg, 1)) ||
+          (c.rewards && (rc = gather(ch, c.rewards, h->pf_rew, 1))))
+        return rc;
+      xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
+      h->launches += 1;
+      rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), PW(XL_W_EMBED_STATE_B), nullptr,
+                  ws.s_emb, rows, d, h->Kpad, impl, s);
+      if (rc) return rc;
+      xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, c.rewards ? h->pf_rew : nullptr, PW(XL_W_EMBED_RETURN_W),
+                              PW(XL_W_EMBED_RETURN_B), PW(XL_W_EMBED_REWARD_W), PW(XL_W_EMBED_REWARD_B),
+                              PW(XL_W_EMBED_LN_W), PW(XL_W_EMBED_LN_B), cf.embed_ln_eps, ws.x, rows, d, nullptr, nullptr,
+                              nullptr, 0.f, nullptr, nullptr, nullptr, s);
+      h->launches += 1;
+    }
+    if ((rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, ch.n * p.T, c.flags, s, p.d_len, ch.pos * p.T))) return rc;
+    if (c.y_out) {
+      xl::launch_ln_rows(h->pf_x, d, h->pf_xn, d, PW(XL_W_POST_NORM), nullptr, 1, cf.ln_eps, rows, d, nullptr, nullptr,
+                         s);
+      h->launches += 1;
+      if ((rc = chunk_rows(h, p, ch, c.y_out, h->pf_xn, S, d, 1, s))) return rc;
+    }
+    if (head && (rc = seq_head_chunk(h, hd, ch.Bk, ch.n, ch.pos, p.d_perm, p.d_len, c.flags, s))) return rc;
+    XL_CUDA(cudaGetLastError());
+  }
+  if ((rc = ragged_end(h, c.state, B, p, s))) return rc;
+  // the eager tail (uniform calls only): fused encoder steps of <= 4 tokens ...
+  if (enc) {
+    const Slice sl = make_slice(h, B, 0, B, s);
+    for (int pos = p.tail; pos < S;) {
+      const SeqChunk ch = {pos, B, std::min(4, S - pos)};
+      if ((rc = gather(ch, c.x, sl.ws.x, d))) return rc;
+      if ((rc = run_encoder(h, c.state, sl, sl.ws.x, sl.ws.hid, ch.n, XL_MODE_FUSED, c.flags))) return rc;
+      if (c.y_out && (rc = chunk_rows(h, p, ch, c.y_out, sl.ws.hid, S, d, 1, s))) return rc;
+      pos += ch.n;
+    }
+    return XL_OK;
+  }
+  // ... or ordinary fused policy steps with their outputs discarded; a forward reduces each step's logits as a chunk
+  // of one timestep
+  if (head && p.tail < S && (rc = ensure_seq_logits(h, (size_t)B * hd.n_out))) return rc;
+  const bool embeds = c.in == SeqCall::kEmbeds;
+  float* stage = embeds ? h->d_embeds : h->d_states;
+  for (int pos = p.tail; pos < S; ++pos) {
+    const SeqChunk ch = {pos, B, 1};
+    if ((rc = gather(ch, c.x, stage, embeds ? d : sd)) || (rc = gather(ch, c.rtg, h->d_rtg, 1)) ||
+        (c.rewards && (rc = gather(ch, c.rewards, h->d_rew, 1))))
+      return rc;
     StepArgs a;
-    a.state = state; a.states = stage; a.rtg = h->d_rtg; a.rewards = rewards ? h->d_rew : nullptr;
+    a.state = c.state; a.states = stage; a.rtg = h->d_rtg; a.rewards = c.rewards ? h->d_rew : nullptr;
     a.tokens = h->d_tokens; a.actions = h->d_actions; a.logits = head ? h->sq_logits : nullptr; a.hidden = nullptr;
-    a.B = B; a.mode = XL_MODE_FUSED; a.flags = (flags & ~(unsigned)XL_FLAG_GRAPH) | kFlagNoRing;
-    rc = run_policy(h, a, s);
-    if (rc) return rc;
-    if (head) seq_head_reduce(h, *head, B, 1, pos, nullptr, nullptr, s);
+    a.B = B; a.mode = XL_MODE_FUSED; a.flags = (c.flags & ~(unsigned)XL_FLAG_GRAPH) | kFlagNoRing;
+    if ((rc = run_policy(h, a, s))) return rc;
+    if (head) seq_head_reduce(h, hd, B, 1, pos, nullptr, nullptr, s);
   }
   return XL_OK;
 }
 
-// raw-state policy prefills: state embeddings go through the _embeds entries (the loops would read them as [B, Tn, sd])
-static int reject_state_embeds(const char* fn, unsigned flags) {
-  if (flags & XL_FLAG_STATE_EMBEDS)
-    return fail(XL_ERR_UNSUPPORTED, "%s takes raw states; state embeddings go through xl_policy_prefill_embeds / "
-                                    "xl_policy_forward_embeds", fn);
-  return XL_OK;
-}
-
-int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
-                      int Tn, unsigned flags, void* stream) {
-  if (int rc = reject_state_embeds("xl_policy_prefill", flags)) return rc;
-  return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, nullptr);
+int xl_prefill(xl_handle* h, void* state, const float* x_in, float* y_out, int B, int S, unsigned flags, void* stream) {
+  SeqCall c("xl_prefill", SeqCall::kTokens, state, x_in, nullptr, nullptr, nullptr, B, S, flags, stream);
+  c.y_out = y_out;
+  return run_seq(h, c);
 }
 
 int xl_prefill_ragged(xl_handle* h, void* state, const float* x_in, float* y_out, const int32_t* lengths, int B, int S,
                       unsigned flags, void* stream) {
-  int rc = check_batch(h, B);
-  if (rc) return rc;
-  if (!state || !x_in) return fail(XL_ERR_INVALID_ARG, "null argument");
-  if (S <= 0) return fail(XL_ERR_INVALID_ARG, "S=%d must be positive", S);
-  if ((rc = check_lengths(lengths, B, S, "S"))) return rc;
-  rc = weights_ready(h, true);
-  if (rc) return rc;
-  const int nfull = (int)std::count(lengths, lengths + B, S), nzero = (int)std::count(lengths, lengths + B, 0);
-  if (nfull == B) return xl_prefill(h, state, x_in, y_out, B, S, flags, stream);
-  if (nzero < B && !prefill_fast_path(h))
-    return fail(XL_ERR_UNSUPPORTED, "ragged prefill needs the sequence path (conv_kernel 4, a cell plan for DH=%d)", h->DH);
-  cudaStream_t s = (cudaStream_t)stream;
-  const xl_config& c = h->cfg;
-  const int d = c.embedding_dim;
-  if (y_out) XL_CUDA(cudaMemsetAsync(y_out, 0, sizeof(float) * (size_t)B * S * d, s));
-  if (nzero == B) return XL_OK;
-  const float* post_w = (const float*)h->pw[XL_W_POST_NORM - XL_W_POST_NORM];
-  RaggedPlan p;
-  std::vector<RaggedChunk> chunks;
-  if ((rc = ragged_begin(h, state, lengths, B, 1, p, s))) return rc;
-  if ((rc = ragged_chunks(h, p.len, 1, chunks))) return rc;
-  for (const RaggedChunk& ch : chunks) {
-    xl::launch_ragged_rows(const_cast<float*>(x_in), h->pf_x, p.d_perm, p.d_len, 1, ch.Bk, S, ch.n, ch.pos, d, 0, s);
-    h->launches += 1;
-    rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, ch.n, flags, s, p.d_len, ch.pos);
-    if (rc) return rc;
-    if (y_out) {
-      xl::launch_ln_rows(h->pf_x, d, h->pf_xn, d, post_w, nullptr, 1, c.ln_eps, ch.Bk * ch.n, d, nullptr, nullptr, s);
-      xl::launch_ragged_rows(y_out, h->pf_xn, p.d_perm, p.d_len, 1, ch.Bk, S, ch.n, ch.pos, d, 1, s);
-      h->launches += 2;
-    }
-    XL_CUDA(cudaGetLastError());
-  }
-  return ragged_end(h, state, B, p, s);
+  SeqCall c("xl_prefill_ragged", SeqCall::kTokens, state, x_in, nullptr, nullptr, lengths, B, S, flags, stream);
+  c.ragged = true;
+  c.y_out = y_out;
+  return run_seq(h, c);
 }
 
-// xl_policy_prefill_ragged; with a head hook (xl_policy_forward) also the action outputs of every timestep. With
-// XL_FLAG_STATE_EMBEDS `states` holds state embeddings [B, Tn, d].
-static int policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
-                                 const int32_t* lengths, int B, int Tn, unsigned flags, void* stream,
-                                 const SeqHead* head) {
-  int rc = check_batch(h, B);
-  if (rc) return rc;
-  if (!state || !states || !rtg) return fail(XL_ERR_INVALID_ARG, "null argument");
-  if (Tn <= 0) return fail(XL_ERR_INVALID_ARG, "Tn=%d must be positive", Tn);
-  if ((rc = check_lengths(lengths, B, Tn, "Tn"))) return rc;
-  rc = xl_weights_ready(h);
-  if (rc) return rc;
-  const int nfull = (int)std::count(lengths, lengths + B, Tn), nzero = (int)std::count(lengths, lengths + B, 0);
-  if (nfull == B) return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, head);
-  if (nzero < B && !prefill_fast_path(h))
-    return fail(XL_ERR_UNSUPPORTED, "ragged prefill needs the sequence path (conv_kernel 4, a cell plan for DH=%d)", h->DH);
-  cudaStream_t s = (cudaStream_t)stream;
-  if (head && (rc = seq_clear_outputs(h, *head, B, s))) return rc;
-  if (nzero == B) return XL_OK;
-  const xl_config& c = h->cfg;
-  const int d = c.embedding_dim, sd = c.state_dim, T = c.tokens_per_step;
-  const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
-  auto PW = [&](int id) { return h->pw[id - XL_W_POST_NORM]; };
-  RaggedPlan p;
-  std::vector<RaggedChunk> chunks;
-  if ((rc = ragged_begin(h, state, lengths, B, T, p, s))) return rc;
-  if ((rc = ragged_chunks(h, p.len, T, chunks))) return rc;
-  for (const RaggedChunk& ch : chunks) {
-    const int Tc = ch.n, rows = ch.Bk * Tc;
-    if (flags & XL_FLAG_STATE_EMBEDS) {
-      seq_embed_chunk(h, states, rtg, rewards, p.d_perm, p.d_len, ch.Bk, Tn, Tc, ch.pos, s);
-    } else {
-      const Ws ws = prefill_ws(h);
-      // the chunk's timesteps of the prefix envs, pads zero-filled: [Bk, Tc, sd], [Bk, Tc]
-      xl::launch_ragged_rows(const_cast<float*>(states), h->pf_sin, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, sd, 0, s);
-      xl::launch_ragged_rows(const_cast<float*>(rtg), h->pf_rtg, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
-      if (rewards)
-        xl::launch_ragged_rows(const_cast<float*>(rewards), h->pf_rew, p.d_perm, p.d_len, T, ch.Bk, Tn, Tc, ch.pos, 1, 0, s);
-      xl::launch_pad_rows(h->pf_sin, sd, ws.states_pad, h->Kpad, rows, s);
-      h->launches += rewards ? 4 : 3;
-      rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr, ws.s_emb,
-                  rows, d, h->Kpad, impl, s);
-      if (rc) return rc;
-      xl::launch_embed_tokens(ws.s_emb, h->pf_rtg, rewards ? h->pf_rew : nullptr, (const float*)PW(XL_W_EMBED_RETURN_W),
-                              (const float*)PW(XL_W_EMBED_RETURN_B), (const float*)PW(XL_W_EMBED_REWARD_W),
-                              (const float*)PW(XL_W_EMBED_REWARD_B), (const float*)PW(XL_W_EMBED_LN_W),
-                              (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, ws.x, rows, d, nullptr, nullptr, nullptr,
-                              0.f, nullptr, nullptr, nullptr, s);
-      h->launches += 1;
-    }
-    rc = prefill_blocks(h, p.st, p.Btot, ch.Bk, Tc * T, flags, s, p.d_len, ch.pos * T);
-    if (rc) return rc;
-    if (head && (rc = seq_head_chunk(h, *head, ch.Bk, Tc, ch.pos, p.d_perm, p.d_len, flags, s))) return rc;
-    XL_CUDA(cudaGetLastError());
-  }
-  return ragged_end(h, state, B, p, s);
+int xl_policy_prefill(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards, int B,
+                      int Tn, unsigned flags, void* stream) {
+  return run_seq(h, SeqCall("xl_policy_prefill", SeqCall::kStates, state, states, rtg, rewards, nullptr, B, Tn, flags,
+                            stream));
 }
 
 int xl_policy_prefill_ragged(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
                              const int32_t* lengths, int B, int Tn, unsigned flags, void* stream) {
-  if (int rc = reject_state_embeds("xl_policy_prefill_ragged", flags)) return rc;
-  return policy_prefill_ragged(h, state, states, rtg, rewards, lengths, B, Tn, flags, stream, nullptr);
+  SeqCall c("xl_policy_prefill_ragged", SeqCall::kStates, state, states, rtg, rewards, lengths, B, Tn, flags, stream);
+  c.ragged = true;
+  return run_seq(h, c);
 }
 
 int xl_policy_forward(xl_handle* h, void* state, const float* states, const float* rtg, const float* rewards,
                       const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out, unsigned flags, void* stream) {
-  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
-  if (!out) return fail(XL_ERR_INVALID_ARG, "null outputs");
-  if (out->logprobs && !out->targets) return fail(XL_ERR_INVALID_ARG, "logprobs need targets");
-  if (flags & XL_FLAG_STATE_EMBEDS)
-    return fail(XL_ERR_UNSUPPORTED, "xl_policy_forward takes raw states (no state embeddings)");
-  SeqHead hd;
-  hd.out = *out;
-  hd.discrete = (flags & XL_FLAG_DISCRETE) ? 1 : 0;
-  hd.n_out = hd.discrete ? h->num_actions : h->head_out;
-  hd.Tn = Tn;
-  if (!lengths) return policy_prefill(h, state, states, rtg, rewards, B, Tn, flags, stream, &hd);
-  return policy_prefill_ragged(h, state, states, rtg, rewards, lengths, B, Tn, flags, stream, &hd);
-}
-
-// the state-embedding forms run the same loops with XL_FLAG_STATE_EMBEDS: each chunk's tokens come from one
-// seq_embed_tokens launch, the eager tail stages [B, d] rows into d_embeds for policy_front
-static int check_embeds(const float* state_embeds) {
-  if ((uintptr_t)state_embeds % 16)
-    return fail(XL_ERR_INVALID_ARG, "state_embeds must be 16-byte aligned (rows are loaded as float4)");
-  return XL_OK;
+  SeqCall c("xl_policy_forward", SeqCall::kStates, state, states, rtg, rewards, lengths, B, Tn, flags, stream);
+  c.head = true;
+  c.out = out;
+  return run_seq(h, c);
 }
 
 int xl_policy_prefill_embeds(xl_handle* h, void* state, const float* state_embeds, const float* rtg,
                              const float* rewards, const int32_t* lengths, int B, int Tn, unsigned flags,
                              void* stream) {
-  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
-  if (int rc = check_embeds(state_embeds)) return rc;
-  flags |= XL_FLAG_STATE_EMBEDS;
-  if (!lengths) return policy_prefill(h, state, state_embeds, rtg, rewards, B, Tn, flags, stream, nullptr);
-  return policy_prefill_ragged(h, state, state_embeds, rtg, rewards, lengths, B, Tn, flags, stream, nullptr);
+  return run_seq(h, SeqCall("xl_policy_prefill_embeds", SeqCall::kEmbeds, state, state_embeds, rtg, rewards, lengths, B,
+                            Tn, flags, stream));
 }
 
 int xl_policy_forward_embeds(xl_handle* h, void* state, const float* state_embeds, const float* rtg,
                              const float* rewards, const int32_t* lengths, int B, int Tn, const xl_seq_outputs* out,
                              unsigned flags, void* stream) {
-  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
-  if (!out) return fail(XL_ERR_INVALID_ARG, "null outputs");
-  if (out->logprobs && !out->targets) return fail(XL_ERR_INVALID_ARG, "logprobs need targets");
-  if (int rc = check_embeds(state_embeds)) return rc;
-  SeqHead hd;
-  hd.out = *out;
-  hd.discrete = (flags & XL_FLAG_DISCRETE) ? 1 : 0;
-  hd.n_out = hd.discrete ? h->num_actions : h->head_out;
-  hd.Tn = Tn;
-  flags |= XL_FLAG_STATE_EMBEDS;
-  if (!lengths) return policy_prefill(h, state, state_embeds, rtg, rewards, B, Tn, flags, stream, &hd);
-  return policy_prefill_ragged(h, state, state_embeds, rtg, rewards, lengths, B, Tn, flags, stream, &hd);
+  SeqCall c("xl_policy_forward_embeds", SeqCall::kEmbeds, state, state_embeds, rtg, rewards, lengths, B, Tn, flags,
+            stream);
+  c.head = true;
+  c.out = out;
+  return run_seq(h, c);
 }
 
 int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bias, const float* residual,

@@ -368,30 +368,33 @@ class XLSTMEngine:
         if state_embeds:
             self._check_state_embeds(states, state.B)
         lens = None if lengths is None else check_lengths(lengths, state.B, states.shape[1], "Tn")
-        return self._policy_prefill(state, states, rtg, rewards, flags, lens, state_embeds)
+        self._seq_call(state, states, rtg, rewards, lens, flags, state_embeds)
 
     @_on_device
-    def _policy_prefill(self, state, states, rtg, rewards, flags, lens, state_embeds=False):
-        cfg = self.cfg
+    def _seq_call(self, state, states, rtg, rewards, lens, flags, state_embeds, outputs=None):
+        """The one place a policy sequence call reaches the library: the prefill (outputs None) or the forward
+        (outputs: an XLSeqOutputs), from raw states or state embeddings, uniform (lens None) or ragged."""
         B, Tn = state.B, states.shape[1]
         assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == \
-            (B, Tn, cfg.d if state_embeds else cfg.state_dim)
+            (B, Tn, self.cfg.d if state_embeds else self.cfg.state_dim)
         assert rtg.is_cuda and rtg.dtype == torch.float32 and rtg.numel() == B * Tn
-        states, rtg = states.contiguous(), rtg.contiguous()
+        states = self._embeds_operand(states) if state_embeds else states.contiguous()
+        rtg = rtg.contiguous()
         if rewards is not None:
             rewards = rewards.to(self.device, torch.float32).contiguous()
             assert rewards.numel() == B * Tn
-        if state_embeds:
-            L.check(self.lib.xl_policy_prefill_embeds(
-                self.handle, _ptr(state.buf), _ptr(self._embeds_operand(states)), _ptr(rtg), _ptr(rewards),
-                None if lens is None else lens.ctypes.data_as(C.c_void_p), B, Tn, flags, self._stream()))
+        args = (self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards))
+        lp = None if lens is None else lens.ctypes.data_as(C.c_void_p)
+        if outputs is not None:
+            fn = self.lib.xl_policy_forward_embeds if state_embeds else self.lib.xl_policy_forward
+            rc = fn(*args, lp, B, Tn, C.byref(outputs), flags, self._stream())
+        elif state_embeds:
+            rc = self.lib.xl_policy_prefill_embeds(*args, lp, B, Tn, flags, self._stream())
         elif lens is None:
-            L.check(self.lib.xl_policy_prefill(self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards), B,
-                                               Tn, flags, self._stream()))
+            rc = self.lib.xl_policy_prefill(*args, B, Tn, flags, self._stream())
         else:
-            L.check(self.lib.xl_policy_prefill_ragged(self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg),
-                                                      _ptr(rewards), lens.ctypes.data_as(C.c_void_p), B, Tn, flags,
-                                                      self._stream()))
+            rc = self.lib.xl_policy_prefill_ragged(*args, lp, B, Tn, flags, self._stream())
+        L.check(rc)
 
     def policy_forward(self, state: StateCache, states: torch.Tensor, rtg: torch.Tensor,
                        rewards: Optional[torch.Tensor] = None, lengths=None, discrete: bool = False,
@@ -435,13 +438,6 @@ class XLSTMEngine:
     def _policy_forward(self, state, states, rtg, rewards, lens, discrete, targets, want_logits, state_embeds=False):
         cfg = self.cfg
         B, Tn = state.B, states.shape[1]
-        assert states.is_cuda and states.dtype == torch.float32 and tuple(states.shape) == \
-            (B, Tn, cfg.d if state_embeds else cfg.state_dim)
-        assert rtg.is_cuda and rtg.dtype == torch.float32 and rtg.numel() == B * Tn
-        states, rtg = states.contiguous(), rtg.contiguous()
-        if rewards is not None:
-            rewards = rewards.to(self.device, torch.float32).contiguous()
-            assert rewards.numel() == B * Tn
         out = {"action_tokens": torch.empty(B, Tn, cfg.act_dim, dtype=torch.int32, device=self.device),
                "action_preds": torch.empty(B, Tn, cfg.act_dim, dtype=torch.float32, device=self.device)}
         if want_logits:
@@ -453,13 +449,7 @@ class XLSTMEngine:
         so = L.XLSeqOutputs(tokens=out["action_tokens"].data_ptr(), actions=out["action_preds"].data_ptr(),
                             logits=_ptr(out.get("action_logits")).value, targets=_ptr(targets).value,
                             logprobs=_ptr(out.get("action_logprobs")).value)
-        if state_embeds:
-            states = self._embeds_operand(states)
-        fn = self.lib.xl_policy_forward_embeds if state_embeds else self.lib.xl_policy_forward
-        L.check(fn(
-            self.handle, _ptr(state.buf), _ptr(states), _ptr(rtg), _ptr(rewards),
-            None if lens is None else lens.ctypes.data_as(C.c_void_p), B, Tn, C.byref(so),
-            L.XL_FLAG_DISCRETE if discrete else 0, self._stream()))
+        self._seq_call(state, states, rtg, rewards, lens, L.XL_FLAG_DISCRETE if discrete else 0, state_embeds, so)
         return out
 
     @_on_device
