@@ -240,6 +240,22 @@ int xl_mlstm_cell_step(xl_handle* h, float* C, float* n, float* m, const float* 
                        const float* fgate, const float* outnorm_w, float* h_norm, float* h_raw, int B, int T,
                        int rows_split, int cols_per_cta, void* stream);
 
+/* The sequence-path counterpart of xl_mlstm_cell_step, for unit parity: the gate scan and the sequence cell that a
+ * context prefill of B envs x S tokens runs (chosen by the "prefill_cell" option under the same conditions), then the
+ * sequence finalize. C (slab-major), n [B,NH,DH], m [B,NH] updated in place by S tokens.
+ *   q, k, v   fp32 [B*S, inner] (rows [env][token], q and k unscaled)
+ *   gates     fp32 [B*S, 2, NH] pre-activations (input gates, then forget gates; bias already added)
+ *   act       fp32 [B*S, inner] a = silu(conv); u fp32 [B*S, 2*inner] (only the z half u[:, inner:] is read)
+ *   outnorm_w, skip fp32 [inner]
+ *   num  fp32 [B*S, inner] q^T C per token (un-normalised); qn fp32 [B*S, NH] q.n per token; mseq fp32 [B*NH, S] m
+ *   out  fp32 [B*S, inner] (MultiHeadLayerNorm(h) + skip * a) * silu(z), h = num / (max(|qn|, exp(-m)) + cell_eps)
+ *   cell (host, nullable) <- the cell that ran: 0 = fp32, 1 = mma.sync, 2 = tcgen05.
+ * XL_ERR_UNSUPPORTED (nothing launched) when the cell "prefill_cell" selects cannot take DH and S: the tcgen05 cell
+ * needs S >= 64, the mma.sync cell S % 16 == 0, the fp32 cell S % 8 == 0. */
+int xl_mlstm_cell_seq(xl_handle* h, float* C, float* n, float* m, const float* q, const float* k, const float* v,
+                      const float* gates, const float* act, const float* u, const float* outnorm_w, const float* skip,
+                      float* num, float* qn, float* mseq, float* out, int* cell, int B, int S, void* stream);
+
 /* One env step of the whole policy for B envs with device-resident inputs:
  * MultiDomainDiscreteDecisionXLSTMModel.forward on the inference-cache path (online_decision_transformer_
  * model.py:326-390 -> compute_hidden_states :392-461 -> encoder -> get_predictions discrete_decision_

@@ -115,6 +115,8 @@ def load():
     lib.xl_encoder_step.restype = i32
     lib.xl_mlstm_cell_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, vp]
     lib.xl_mlstm_cell_step.restype = i32
+    lib.xl_mlstm_cell_seq.argtypes = [vp] * 17 + [i32, i32, vp]
+    lib.xl_mlstm_cell_seq.restype = i32
     lib.xl_policy_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, u32, vp]
     lib.xl_policy_step.restype = i32
     lib.xl_policy_step_host.argtypes = [vp, vp, vp, vp, vp, vp, vp, i32, i32, u32, vp]

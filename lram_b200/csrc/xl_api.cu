@@ -957,6 +957,49 @@ Ws prefill_ws(const xl_handle* h) {
   return w;
 }
 
+// The sequence cell that runs B envs x Sc tokens of this handle: 2 = tcgen05, 1 = mma.sync, 0 = fp32; -1 when none
+// can. tcgen05 cell: whole 128-token chunks per (env, head) -- short runs of many envs (Sc < 64: more than half of
+// every chunk would be padding) or a workspace beyond 8 GiB fall through to the 16-token mma.sync cell.
+int seq_cell_choice(const xl_handle* h, int B, int Sc) {
+  const int NH = h->cfg.num_heads, DH = h->DH;
+  if (h->prefill_cell == 2 && xl::prefill_cell_tc_supported(DH) && Sc >= 64 &&
+      xl::prefill_cell_tc_ws_bytes(B, Sc, NH, DH) <= ((size_t)8 << 30))
+    return 2;
+  if (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(DH) && Sc % xl::prefill_cell_mma_chunk() == 0) return 1;
+  if (xl::prefill_cell_supported(DH) && Sc % 8 == 0) return 0;
+  return -1;
+}
+
+// Gate scan + sequence cell of one mLSTM block over B envs x Sc tokens (rows [env][token]): the carried C / n / m_state
+// advanced by the Sc tokens, per-token num [B*Sc, inner], qn [B*Sc, NH] and m [B*NH][Sc] (mseq) for the finalize.
+// gate_part [B*Sc, NCH, 2*NH] partial gate pre-activations, biases nullable; len / pos: ragged chunk (see
+// prefill_blocks). The prefill workspace must hold B*Sc rows and the gate-scan scratch. *cell (nullable) <- the cell
+// that ran (seq_cell_choice).
+int seq_cell(xl_handle* h, float* C, float* n, float* m_state, const float* q, const float* k, const float* v,
+             const float* gate_part, const float* igate_b, const float* fgate_b, float* num, float* qn, float* mseq,
+             int B, int Sc, int NCH, cudaStream_t s, const int32_t* len, int pos, int* cell) {
+  const int NH = h->cfg.num_heads, DH = h->DH, inner = h->cfg.inner_dim;
+  const int which = seq_cell_choice(h, B, Sc);
+  if (which < 0) return fail(XL_ERR_UNSUPPORTED, "no sequence cell takes DH=%d over %d tokens", DH, Sc);
+  xl::launch_gate_scan_seq(gate_part, igate_b, fgate_b, m_state, h->pf_f, h->pf_i, mseq, h->pf_gsc, B, Sc, NH, NCH, s,
+                           len, pos);
+  XL_CUDA(cudaGetLastError());
+  if (which == 2) {
+    if (int rcw = ensure_prefill_tc_ws(h, B, Sc)) return rcw;
+    const xl::CellSideStream side = {h->side[0], h->ev_fork, h->ev_join[0]};
+    XL_CUDA(xl::launch_cell_tc(C, n, q, k, v, h->pf_f, h->pf_i, num, qn, h->pf_tc, B, Sc, NH, DH, inner, s, &side));
+    h->launches += 6;
+    XL_CUDA(cudaGetLastError());
+  } else if (which == 1) {
+    XL_CUDA(xl::launch_cell_mma(C, n, q, k, v, h->pf_f, h->pf_i, num, qn, h->pf_pc, h->pf_pv, B, Sc, NH, DH, inner, s));
+    h->launches += 1;
+  } else {
+    XL_CUDA(xl::launch_cell_seq(C, n, q, k, v, h->pf_f, h->pf_i, num, qn, B, Sc, NH, DH, inner, s));
+  }
+  if (cell) *cell = which;
+  return XL_OK;
+}
+
 // tokens per env in one prefill chunk: ~2048 rows per chunk over all envs, a multiple of 48 (whole (s, rtg, r)
 // timesteps, whole 8-token stages of the fp32 cell and whole 16-token chunks of the tensor-core cell)
 int prefill_chunk_tokens(const xl_handle* h, int B) {
@@ -1018,30 +1061,10 @@ int prefill_blocks(xl_handle* h, void* state, int Btot, int B, int Sc, unsigned 
     if (!xl::launch_conv_qkv_gates_seq(cp, Sc, s, len, pos))
       return fail(XL_ERR_UNSUPPORTED, "sequence conv/qkv kernel not instantiated for KS=%d NH=%d", cp.KS, cp.NH);
     XL_CUDA(cudaGetLastError());
-    xl::launch_gate_scan_seq(ws.gate_part, (const float*)w.w[XL_W_IGATE_B], (const float*)w.w[XL_W_FGATE_B],
-                             (float*)(base + L.m_off), h->pf_f, h->pf_i, h->pf_m, h->pf_gsc, B, Sc, NH, h->NCH, s,
-                             len, pos);
-    XL_CUDA(cudaGetLastError());
-    // tcgen05 cell: whole 128-token chunks per (env, head) -- short runs of many envs (Sc < 64: more than half of every
-    // chunk would be padding) or a workspace beyond 8 GiB fall through to the 16-token mma.sync cell
-    if (h->prefill_cell == 2 && xl::prefill_cell_tc_supported(DH) && Sc >= 64 &&
-        xl::prefill_cell_tc_ws_bytes(B, Sc, NH, DH) <= ((size_t)8 << 30)) {
-      if (int rcw = ensure_prefill_tc_ws(h, B, Sc)) return rcw;
-      const xl::CellSideStream side = {h->side[0], h->ev_fork, h->ev_join[0]};
-      XL_CUDA(xl::launch_cell_tc((float*)(base + L.c_off), (float*)(base + L.n_off), cp.qk, cp.qk + (size_t)M * inner,
-                                 cp.v, h->pf_f, h->pf_i, h->pf_num, h->pf_qn, h->pf_tc, B, Sc, NH, DH, inner, s, &side));
-      h->launches += 6;
-      XL_CUDA(cudaGetLastError());
-    } else if (h->prefill_cell >= 1 && xl::prefill_cell_mma_supported(DH) && Sc % xl::prefill_cell_mma_chunk() == 0) {
-      XL_CUDA(xl::launch_cell_mma((float*)(base + L.c_off), (float*)(base + L.n_off), cp.qk,
-                                  cp.qk + (size_t)M * inner, cp.v, h->pf_f, h->pf_i, h->pf_num, h->pf_qn, h->pf_pc,
-                                  h->pf_pv, B, Sc, NH, DH, inner, s));
-      h->launches += 1;
-    } else {
-      XL_CUDA(xl::launch_cell_seq((float*)(base + L.c_off), (float*)(base + L.n_off), cp.qk,
-                                  cp.qk + (size_t)M * inner, cp.v, h->pf_f, h->pf_i, h->pf_num, h->pf_qn, B, Sc, NH,
-                                  DH, inner, s));
-    }
+    rc = seq_cell(h, (float*)(base + L.c_off), (float*)(base + L.n_off), (float*)(base + L.m_off), cp.qk,
+                  cp.qk + (size_t)M * inner, cp.v, ws.gate_part, (const float*)w.w[XL_W_IGATE_B],
+                  (const float*)w.w[XL_W_FGATE_B], h->pf_num, h->pf_qn, h->pf_m, B, Sc, h->NCH, s, len, pos, nullptr);
+    if (rc) return rc;
     XL_CUDA(xl::launch_finalize_seq(h->pf_num, h->pf_qn, h->pf_m, (const float*)w.w[XL_W_OUTNORM],
                                     (const float*)w.w[XL_W_SKIP], ws.act, ws.u, tc_down ? nullptr : ws.gated,
                                     tc_down ? ws.a_hi : nullptr, tc_down ? ws.a_lo : nullptr, B, Sc, NH, DH, inner,
@@ -1711,6 +1734,30 @@ int xl_mlstm_cell_step(xl_handle* h, float* C, float* n, float* m, const float* 
   }
   if (!xl::state_step_fuses_finalize(sp, h->num_sms)) XL_CUDA(xl::launch_state_finalize(sp, h->num_sms, s));
   h->launches += 3;
+  return XL_OK;
+}
+
+int xl_mlstm_cell_seq(xl_handle* h, float* C, float* n, float* m, const float* q, const float* k, const float* v,
+                      const float* gates, const float* act, const float* u, const float* outnorm_w, const float* skip,
+                      float* num, float* qn, float* mseq, float* out, int* cell, int B, int S, void* stream) {
+  int rc = check_batch(h, B);
+  if (rc) return rc;
+  if (!C || !n || !m || !q || !k || !v || !gates || !act || !u || !outnorm_w || !skip || !num || !qn || !mseq || !out)
+    return fail(XL_ERR_INVALID_ARG, "null argument");
+  if (S < 1) return fail(XL_ERR_INVALID_ARG, "S=%d", S);
+  const xl_config& c = h->cfg;
+  const int which = seq_cell_choice(h, B, S);
+  if (which != h->prefill_cell)
+    return fail(XL_ERR_UNSUPPORTED, "prefill_cell %d cannot take DH=%d over %d tokens of %d envs", h->prefill_cell,
+                h->DH, S, B);
+  cudaStream_t s = (cudaStream_t)stream;
+  rc = ensure_prefill_ws(h, B * S, xl::gate_scan_seq_scratch_floats(B, S, c.num_heads));
+  if (rc) return rc;
+  rc = seq_cell(h, C, n, m, q, k, v, gates, nullptr, nullptr, num, qn, mseq, B, S, 1, s, nullptr, 0, cell);
+  if (rc) return rc;
+  XL_CUDA(xl::launch_finalize_seq(num, qn, mseq, outnorm_w, skip, act, u, out, nullptr, nullptr, B, S, c.num_heads,
+                                  h->DH, c.inner_dim, c.ln_eps, c.cell_eps, s));
+  h->launches += 1;
   return XL_OK;
 }
 

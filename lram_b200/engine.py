@@ -512,6 +512,24 @@ class XLSTMEngine:
         return h_norm, h_raw
 
     @_on_device
+    def cell_seq(self, Cs, n, m, q, k, v, gates, act, u, outnorm_w, skip, B: int, S: int):
+        """Unit-parity entry point of the sequence cell the "prefill_cell" option selects (xl_mlstm_cell_seq). `Cs` is
+        given and updated in the REFERENCE layout [B,NH,DH,DH], n [B,NH,DH] and m [B,NH] in place. Returns
+        (num [B*S, inner], qn [B*S, NH], m [B*NH, S], out [B*S, inner], cell id: 0 fp32, 1 mma.sync, 2 tcgen05)."""
+        inner, NH = self.cfg.inner, self.cfg.num_heads
+        num = torch.empty(B * S, inner, dtype=torch.float32, device=self.device)
+        qn = torch.empty(B * S, NH, dtype=torch.float32, device=self.device)
+        mseq = torch.empty(B * NH, S, dtype=torch.float32, device=self.device)
+        out = torch.empty_like(num)
+        cell = C.c_int(-1)
+        Cp = c_to_slab(Cs)
+        L.check(self.lib.xl_mlstm_cell_seq(self.handle, _ptr(Cp), _ptr(n), _ptr(m), _ptr(q), _ptr(k), _ptr(v),
+                                           _ptr(gates), _ptr(act), _ptr(u), _ptr(outnorm_w), _ptr(skip), _ptr(num),
+                                           _ptr(qn), _ptr(mseq), _ptr(out), C.addressof(cell), B, S, self._stream()))
+        Cs.copy_(c_from_slab(Cp))
+        return num, qn, mseq, out, cell.value
+
+    @_on_device
     def linear(self, A: torch.Tensor, W_bf16: torch.Tensor, bias=None, residual=None, impl: int = 0):
         M, K = A.shape
         N = W_bf16.shape[0]
