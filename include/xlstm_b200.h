@@ -445,14 +445,11 @@ int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bia
  *                   bit-identical); "prefill_tc_overlap": [1] S = QK^T, P~ and the n scan on a side stream beside the chunk
  *                   update + scan when that kernel leaves >= 32 SMs idle (bit-identical); "prefill_scan_split": [2] epilogue warps
  *                   per TMEM lane quarter of that kernel (4 = 16 warps: bit-identical, measured 9 % slower)
- *   "microbatches": [1] env micro-batches of a fused step, pipelined on side streams; "pipeline_order": [1]
- *                   their state-stream kernels take turns
  *   measurement / probe switches (A/B records under profiles/; none changes results):
  *   "l2_prefetch_policy": [0] 1 = warm-up with an L2 evict_last policy; "host_zero_copy": [1] xl_policy_step_host reads and
  *                   writes pinned host buffers through their device aliases (0 = staged copies);
  *   "gemm_cluster": [1] 2 / 4 = A tile TMA-multicast across a cluster of column-tile CTAs (process-wide; measured slower);
  *   "gemm_m64_layout": [0] probe of the TMEM row layout of 64-row UMMA tiles (tests only);
- *   "prefill_gemm_2cta": [0] 1 = two shallow-ring Linear tiles per SM in the prefill (measured equal);
  *   "debug_skip": only in -DXL_DEBUG_OPTIONS builds (skips kernel classes to read their marginal cost; results garbage) */
 int xl_set_option(xl_handle* h, const char* name, int value);
 

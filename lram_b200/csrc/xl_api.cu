@@ -42,15 +42,26 @@ struct BlockWeights {
   const void* w[XL_W_PER_BLOCK_COUNT];
 };
 
+// What a captured step graph is specific to: the entry that captured it, its arguments and its pointers (baked into
+// the graph). Pointers an entry does not take are null.
+struct GraphKey {
+  enum Entry { kPolicyStep, kEncoderStep } entry;
+  void* state;
+  const void *in, *rtg, *rewards;             // in: the policy step's states, the encoder step's x_in
+  void *tokens, *actions, *logits, *out;      // out: the policy step's hidden, the encoder step's x_out
+  int B, T, mode;
+  unsigned flags;
+  bool operator==(const GraphKey& o) const {
+    return entry == o.entry && state == o.state && in == o.in && rtg == o.rtg && rewards == o.rewards &&
+           tokens == o.tokens && actions == o.actions && logits == o.logits && out == o.out && B == o.B && T == o.T &&
+           mode == o.mode && flags == o.flags;
+  }
+};
+
 struct GraphCacheEntry {
+  GraphKey key;
   cudaGraphExec_t exec = nullptr;
-  // key
-  void* state = nullptr;
-  const void *states = nullptr, *rtg = nullptr, *rewards = nullptr;
-  void *tokens = nullptr, *actions = nullptr, *logits = nullptr, *hidden = nullptr;
-  int B = 0, mode = 0;
-  unsigned flags = 0;
-  int64_t launches = 0;
+  int64_t launches = 0;   // kernel launches the graph replays
 };
 
 }  // namespace
@@ -58,7 +69,6 @@ struct GraphCacheEntry {
 // words of the handle's counters area: [0] token ring step, [1] sampler step, [2] step word of xl_sample_actions;
 // xl_sampling copies (32 B, 8-B aligned) of the armed sampler and of xl_sample_actions at kCntArmed / kCntUnit
 constexpr int kCntRing = 0, kCntSample = 1, kCntUnitStep = 2, kCntArmed = 8, kCntUnit = 16;
-constexpr int kMaxMicro = 8;   // env micro-batches pipelined on side streams
 constexpr int kSplitMax = 8;   // split-K planes of the skinny projections
 constexpr size_t kSplitRows = 1024;   // split-K only pays (and has plane storage) up to this many rows
 
@@ -83,11 +93,10 @@ struct xl_handle {
   int64_t launches = 0;
   std::vector<GraphCacheEntry> graphs;
   size_t a_cap = 0;                    // elements per bf16 hi/lo plane
-  size_t a_env = 0;                    // bf16 elements of a plane owned by one env (micro-batch slicing)
   int num_tickets = 0;
   cudaStream_t cap_stream = nullptr;   // graph capture never happens on the caller's (possibly legacy) stream
-  cudaStream_t side[kMaxMicro - 1] = {};   // micro-batches 1.. run here (forked from / joined to the main stream)
-  cudaEvent_t ev_fork = nullptr, ev_join[kMaxMicro - 1] = {}, ev_state[kMaxMicro] = {};
+  cudaStream_t side = nullptr;         // the step's L2 warm-up and the tcgen05 cell's overlapped kernels run here,
+  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;   // forked from / joined to the caller's stream by these events
   int state_impl = 1;                  // 1 = one-shot TMA ring (default), 2 = persistent stream-K TMA ring, 0 = plain loads
   int state_stages = 0;                // impl 2 ring depth (0 = default)        (xl_set_option "state_stages")
   int state_ctas_per_sm = 0;           // impl 2 persistent CTAs per SM (0 = 1)  (xl_set_option "state_ctas_per_sm")
@@ -125,8 +134,6 @@ struct xl_handle {
   int conv_impl = 2;                   // pre-cell kernel: 0 = thread per 4-channel block, 1 = thread per (block, token),
                                        // 2 (default) = as 0 on packed fp32 pairs, gate weights before the wait, butterfly
                                        // reduction (KS = 4, NH <= 4; other shapes run impl 0)
-  int microbatches = 0;                // 0 = automatic; env micro-batches per fused step ("microbatches")
-  int pipeline_order = 1;              // 1 = state-stream kernels of the micro-batches run one after another
   int l2_prefetch_mb = -1;             // MiB of the NEXT block's C warmed into L2 on a side stream while the chain
                                        // of the current block runs; 0 = off, -1 = automatic ("l2_prefetch_mb"):
                                        // 48 MiB when one block's C is 100..300 MB (measured +2 % at 151 MB, 48M x 64
@@ -149,7 +156,6 @@ struct xl_handle {
   // sequence forward (xl_policy_forward): logits of one chunk's timesteps [rows, n_out] (grow-only)
   float* sq_logits = nullptr;
   size_t sq_logits_floats = 0;
-  int prefill_gemm_2cta = 0;                    // A/B: shallow-ring Linear tiles, two CTAs per SM        ("prefill_gemm_2cta")
   int prefill_rows = 16384;                     // rows (envs x tokens) per prefill chunk                  ("prefill_rows")
   char* pf_tc = nullptr;                        // workspace of the tcgen05 chunkwise cell (grow-only)
   size_t pf_tc_bytes = 0;
@@ -221,28 +227,31 @@ int check_batch(const xl_handle* h, int B) {
   return XL_OK;
 }
 
-// The slice of the workspace owned by the envs [b0, b0 + Bk) of a step: every array is carved with a fixed
-// per-env stride (room for 4 tokens), so disjoint env ranges never overlap and micro-batches can run
-// concurrently on different streams.
+// Drops every captured step graph: they bake in weight pointers, options, the token ring and the sampler's kernel.
+void clear_graphs(xl_handle* h) {
+  for (auto& g : h->graphs)
+    if (g.exec) cudaGraphExecDestroy(g.exec);
+  h->graphs.clear();
+}
+
+// The buffers a Linear and the block kernels work in: the step's (step_ws) or the prefill's (prefill_ws).
+// a_cap: elements of the bf16 hi/lo operand planes a tcgen05 Linear may use.
 struct Ws {
   float *x, *xn, *xtok, *hid, *u, *qkv, *act, *gate_part, *gated, *partial, *s_emb, *states_pad, *logits;
   __nv_bfloat16 *a_hi, *a_lo;
   size_t a_cap;
-  int low_smem;     // 1: kernels of this slice run beside other micro-batches' state stream -> small smem footprints
 };
 
-Ws ws_slice(const xl_handle* h, int b0, int Bk) {
-  const xl_config& c = h->cfg;
-  const size_t d = c.embedding_dim, inner = c.inner_dim, e = (size_t)b0;
+// The handle's step workspace for a step over B envs. The tcgen05 Linear of a step takes at most 4 tokens x
+// max(inner, d) plane elements per env: which Linear path runs depends on B only, not on the planes' total size.
+Ws step_ws(const xl_handle* h, int B) {
+  const size_t kmax = std::max(h->cfg.inner_dim, h->cfg.embedding_dim);
   Ws w;
-  w.x = h->x + e * 4 * d; w.xn = h->xn + e * 4 * d; w.xtok = h->xtok + e * 4 * d; w.hid = h->hid + e * 4 * d;
-  w.u = h->u + e * 4 * 2 * inner; w.qkv = h->qkv + e * 4 * 3 * inner; w.act = h->act + e * 4 * inner;
-  w.gate_part = h->gate_part + e * 4 * h->gp_chunks * 2 * c.num_heads; w.gated = h->gated + e * 4 * inner;
-  w.partial = h->partial + e * c.num_heads * 32 * 4 * h->DH;
-  w.s_emb = h->s_emb + e * d; w.states_pad = h->states_pad + e * h->Kpad; w.logits = h->logits + e * h->head_out;
-  w.a_hi = h->a_hi + e * h->a_env; w.a_lo = h->a_lo + e * h->a_env;
-  w.a_cap = (size_t)Bk * h->a_env;     // a slice may only use its envs' share of the planes
-  w.low_smem = 0;
+  w.x = h->x; w.xn = h->xn; w.xtok = h->xtok; w.hid = h->hid; w.u = h->u; w.qkv = h->qkv; w.act = h->act;
+  w.gate_part = h->gate_part; w.gated = h->gated; w.partial = h->partial;
+  w.s_emb = h->s_emb; w.states_pad = h->states_pad; w.logits = h->logits;
+  w.a_hi = h->a_hi; w.a_lo = h->a_lo;
+  w.a_cap = (size_t)B * 4 * kmax;
   return w;
 }
 
@@ -263,7 +272,7 @@ int linear(xl_handle* h, const Ws& w, const float* A, const void* W, const float
       h->launches += 1;
     }
     XL_CUDA(xl::launch_gemm_tc(w.a_hi, w.a_lo, (const __nv_bfloat16*)W, bias, residual, out, M, N, K,
-                               h->num_sms, bn, splits, split_stride, w.low_smem, s));
+                               h->num_sms, bn, splits, split_stride, s));
     h->launches += 1;
     return XL_OK;
   }
@@ -274,31 +283,28 @@ int linear(xl_handle* h, const Ws& w, const float* A, const void* W, const float
   return XL_OK;
 }
 
-// One env range of one step: envs [b0, b0 + Bk) of a state buffer laid out for B envs, on stream s.
-struct Slice {
-  int B, b0, Bk;
+// One step over all B envs of a state buffer laid out for B envs, on stream s.
+struct Step {
+  int B;
   Ws ws;
   cudaStream_t s;
 };
 
-Slice make_slice(const xl_handle* h, int B, int b0, int Bk, cudaStream_t s) {
-  Slice sl;
-  sl.B = B; sl.b0 = b0; sl.Bk = Bk; sl.s = s;
-  sl.ws = ws_slice(h, b0, Bk);
-  return sl;
-}
+Step make_step(const xl_handle* h, int B, cudaStream_t s) { return {B, step_ws(h, B), s}; }
 
-// Gate-partial chunks of the small-batch front kernel (xl_smallm.cu) when it will run for this slice, else 0.
-int smallm_chunks(const xl_handle* h, const Slice& sl, int T, unsigned flags) {
+// Gate-partial chunks of the small-batch front kernel (xl_smallm.cu) when it will run for this step, else 0.
+int smallm_chunks(const xl_handle* h, const Step& sl, int T, unsigned flags) {
   const xl_config& c = h->cfg;
   if (!h->smallm || h->debug_skip || (flags & XL_FLAG_SIMPLE_GEMM)) return 0;
-  if (h->smallm < 0 && (sl.Bk * T > 4 || c.embedding_dim > 1024)) return 0;
-  if (sl.b0 != 0 || sl.Bk != sl.B || sl.ws.low_smem) return 0;
-  return xl::smallm_pre_chunks(sl.Bk, T, c.embedding_dim, c.inner_dim, c.num_heads, c.conv_kernel);
+  if (h->smallm < 0 && (sl.B * T > 4 || c.embedding_dim > 1024)) return 0;
+  return xl::smallm_pre_chunks(sl.B, T, c.embedding_dim, c.inner_dim, c.num_heads, c.conv_kernel);
 }
 
-constexpr unsigned kFlagLn0DoneEarly = 1u << 29;   // == kFlagLn0Done (defined with the policy-level flags below)
-constexpr unsigned kFlagHeadOnlyEarly = 1u << 28;  // == kFlagHeadOnly
+constexpr unsigned kFlagHeadOnly = 1u << 28;    // internal: nobody reads the hidden states: post_blocks_norm only on the
+                                                // action-token rows, fused with the head's operand split (policy_back)
+constexpr unsigned kFlagLn0Done = 1u << 29;     // internal: the embed kernel already ran block 0's pre-norm (operands in place)
+constexpr unsigned kFlagNoRing = 1u << 30;      // internal: steps run on behalf of xl_policy_prefill leave the token ring
+                                                // and the sampler alone (argmax, no step counted)
 
 struct BlockPlan {
   bool tc_up, tc_down;
@@ -307,9 +313,9 @@ struct BlockPlan {
   int up_bn, up_sp, down_bn, down_sp;     // tile width / split-K planes of proj_up and proj_down (sp = 1: none)
 };
 
-BlockPlan block_plan(const xl_handle* h, const Slice& sl, int T, unsigned flags) {
+BlockPlan block_plan(const xl_handle* h, const Step& sl, int T, unsigned flags) {
   const xl_config& c = h->cfg;
-  const int M = sl.Bk * T;
+  const int M = sl.B * T;
   BlockPlan p;
   p.impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
   // when the tensor-core Linear will run, the producers write its bf16 hi/lo operand planes directly
@@ -317,8 +323,8 @@ BlockPlan block_plan(const xl_handle* h, const Slice& sl, int T, unsigned flags)
             (size_t)M * c.embedding_dim <= sl.ws.a_cap;
   p.tc_down = p.impl != 1 && xl::gemm_tc_supported(M, c.embedding_dim, c.inner_dim) &&
               (size_t)M * c.inner_dim <= sl.ws.a_cap;
-  // split-K (planes summed by the consumer kernels): whole-batch slices only, rows within the plane storage
-  const bool can_split = !sl.ws.low_smem && sl.b0 == 0 && (size_t)M <= h->part_rows && c.embedding_dim <= 4096 &&
+  // split-K (planes summed by the consumer kernels): rows within the plane storage
+  const bool can_split = (size_t)M <= h->part_rows && c.embedding_dim <= 4096 &&
                          !smallm_chunks(h, sl, T, flags);   // the fused front kernel reads a complete x
   const int max_sp = can_split ? std::min(std::max(h->gemm_splitk, 1), kSplitMax) : 1;
   p.up_bn = p.down_bn = 0;
@@ -330,7 +336,7 @@ BlockPlan block_plan(const xl_handle* h, const Slice& sl, int T, unsigned flags)
         h->gemm_up_splits <= kSplitMax)
       p.up_sp = h->gemm_up_splits;
   }
-  p.up_fused = h->up_fuse && p.tc_up && !sl.ws.low_smem && !h->debug_skip && !smallm_chunks(h, sl, T, flags) &&
+  p.up_fused = h->up_fuse && p.tc_up && !h->debug_skip && !smallm_chunks(h, sl, T, flags) &&
                xl::gemm_up_conv_chunks(c.inner_dim) <= h->gp_chunks &&
                xl::gemm_up_conv_supported(T, c.conv_kernel, c.num_heads, c.inner_dim, c.embedding_dim);
   if (p.up_fused) { p.up_bn = 64; p.up_sp = 1; }
@@ -344,19 +350,19 @@ BlockPlan block_plan(const xl_handle* h, const Slice& sl, int T, unsigned flags)
   return p;
 }
 
-xl::StateStepParams state_params(const xl_handle* h, void* state, const Slice& sl, int i, int T, bool tc_down,
+xl::StateStepParams state_params(const xl_handle* h, void* state, const Step& sl, int i, int T, bool tc_down,
                                  int up_sp = 1, int small_nch = 0, bool up_fused = false) {
   const xl_config& c = h->cfg;
   const int inner = c.inner_dim, NH = c.num_heads, DH = h->DH;
   const StateLayout L = state_layout(h, sl.B);
   const BlockWeights& w = h->blocks[i];
   char* base = (char*)state + layer_base(h, L, i);
-  const int M = sl.Bk * T;
+  const int M = sl.B * T;
   xl::StateStepParams sp;
   memset(&sp, 0, sizeof(sp));
-  sp.C = (float*)(base + L.c_off) + (size_t)sl.b0 * NH * DH * DH;
-  sp.n = (float*)(base + L.n_off) + (size_t)sl.b0 * NH * DH;
-  sp.m = (float*)(base + L.m_off) + (size_t)sl.b0 * NH;
+  sp.C = (float*)(base + L.c_off);
+  sp.n = (float*)(base + L.n_off);
+  sp.m = (float*)(base + L.m_off);
   sp.qk = sl.ws.qkv;
   sp.v = sl.ws.qkv + (size_t)2 * M * inner;
   sp.gate_part = sl.ws.gate_part;
@@ -372,7 +378,7 @@ xl::StateStepParams state_params(const xl_handle* h, void* state, const Slice& s
   sp.out_hi = tc_down ? sl.ws.a_hi : nullptr;
   sp.out_lo = tc_down ? sl.ws.a_lo : nullptr;
   sp.partial = sl.ws.partial;
-  sp.B = sl.Bk; sp.T = T; sp.NH = NH; sp.DH = DH; sp.inner = inner; sp.NCH = h->NCH;
+  sp.B = sl.B; sp.T = T; sp.NH = NH; sp.DH = DH; sp.inner = inner; sp.NCH = h->NCH;
   if (small_nch) sp.NCH = small_nch;   // chunks of the small-batch front kernel (one per CTA cluster, <= 16)
   if (up_fused) sp.NCH = xl::gemm_up_conv_chunks(inner);   // one chunk per x_m tile of the proj_up epilogue
   sp.ln_eps = c.ln_eps; sp.cell_eps = c.cell_eps;
@@ -384,18 +390,14 @@ xl::StateStepParams state_params(const xl_handle* h, void* state, const Slice& s
     sp.fuse_finalize = 2;
     sp.max_cluster = h->small_state_fuse > 1 ? h->small_state_fuse : 0;
   }
-  if (sl.ws.low_smem) {          // leave shared memory for the co-resident kernels of the other micro-batches
-    if (sp.stages <= 0) sp.stages = 4;
-    sp.meta_slots = 2;
-  }
   return sp;
 }
 
 // block i, part 1: x_n = LN(x); u = x_n W_up^T; conv + SiLU + q/k/v + gate partials   (rows ordered [b][t])
-int block_pre(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned flags) {
+int block_pre(xl_handle* h, void* state, const Step& sl, int i, int T, unsigned flags) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim, inner = c.inner_dim, NH = c.num_heads;
-  const int M = sl.Bk * T;
+  const int M = sl.B * T;
   const StateLayout L = state_layout(h, sl.B);
   const BlockPlan bp = block_plan(h, sl, T, flags);
   const BlockWeights& w = h->blocks[i];
@@ -414,14 +416,14 @@ int block_pre(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned
     sp.conv_state = (float*)(base + L.conv_off);
     sp.u = ws.u; sp.qk = ws.qkv; sp.v = ws.qkv + (size_t)2 * M * inner; sp.act = ws.act;
     sp.gate_part = ws.gate_part;
-    sp.B = sl.Bk; sp.T = T; sp.d = d; sp.inner = inner; sp.NH = NH; sp.NCH = nch;
+    sp.B = sl.B; sp.T = T; sp.d = d; sp.inner = inner; sp.NH = NH; sp.NCH = nch;
     sp.ln_eps = c.ln_eps;
     XL_CUDA(xl::launch_smallm_pre(sp, sl.s));
     h->launches += 1;
     return XL_OK;
   }
   if (h->debug_skip & 1) {
-  } else if (i == 0 && (flags & kFlagLn0DoneEarly)) {
+  } else if (i == 0 && (flags & kFlagLn0Done)) {
     h->launches -= 1;    // block 0's pre-norm ran inside the embed kernel (policy_front): nothing to launch
   } else if (i > 0 && bp.down_sp > 1 && !is_slstm(h, i - 1)) {
     // the previous (mLSTM) block's proj_down left split-K planes: x += planes, then normalise
@@ -436,12 +438,12 @@ int block_pre(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned
   if (bp.up_fused) {
     // proj_up with the pre-cell epilogue: conv + SiLU + q/k/v + gate partials on the x_m tiles while they are on chip
     xl::UpEpiParams ep;
-    ep.conv_state = (float*)(base + L.conv_off) + (size_t)sl.b0 * c.conv_kernel * inner;
+    ep.conv_state = (float*)(base + L.conv_off);
     ep.conv_w = (const float*)w.w[XL_W_CONV_W]; ep.conv_b = (const float*)w.w[XL_W_CONV_B];
     ep.wq = (const float*)w.w[XL_W_Q_PROJ]; ep.wk = (const float*)w.w[XL_W_K_PROJ]; ep.wv = (const float*)w.w[XL_W_V_PROJ];
     ep.wi = (const float*)w.w[XL_W_IGATE_W]; ep.wf = (const float*)w.w[XL_W_FGATE_W];
     ep.qk = ws.qkv; ep.v = ws.qkv + (size_t)2 * M * inner; ep.act = ws.act; ep.gate_part = ws.gate_part;
-    ep.B = sl.Bk; ep.T = T; ep.inner = inner; ep.NCH = xl::gemm_up_conv_chunks(inner);
+    ep.B = sl.B; ep.T = T; ep.inner = inner; ep.NCH = xl::gemm_up_conv_chunks(inner);
     XL_CUDA(xl::launch_gemm_up_conv(ws.a_hi, ws.a_lo, (const __nv_bfloat16*)w.w[XL_W_PROJ_UP], ws.u, M, d, ep, sl.s));
     h->launches += 1;
     return XL_OK;
@@ -455,7 +457,7 @@ int block_pre(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned
   cp.u = bp.up_sp > 1 ? h->part_up : ws.u;
   cp.u_splits = bp.up_sp;
   cp.u_stride = (int64_t)M * 2 * inner;
-  cp.conv_state = (float*)(base + L.conv_off) + (size_t)sl.b0 * c.conv_kernel * inner;
+  cp.conv_state = (float*)(base + L.conv_off);
   cp.conv_w = (const float*)w.w[XL_W_CONV_W];
   cp.conv_b = (const float*)w.w[XL_W_CONV_B];
   cp.wq = (const float*)w.w[XL_W_Q_PROJ];
@@ -467,7 +469,7 @@ int block_pre(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned
   cp.v = ws.qkv + (size_t)2 * M * inner;
   cp.act = ws.act;
   cp.gate_part = ws.gate_part;
-  cp.B = sl.Bk; cp.T = T; cp.inner = inner; cp.NH = NH; cp.KS = c.conv_kernel; cp.NCH = h->NCH;
+  cp.B = sl.B; cp.T = T; cp.inner = inner; cp.NH = NH; cp.KS = c.conv_kernel; cp.NCH = h->NCH;
   cp.impl = h->conv_impl;
   if (!xl::launch_conv_qkv_gates(cp, sl.s))
     return fail(XL_ERR_UNSUPPORTED, "conv/qkv kernel not instantiated for KS=%d T=%d NH=%d", cp.KS, cp.T, cp.NH);
@@ -476,7 +478,7 @@ int block_pre(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned
 }
 
 // block i, part 2: the HBM-bound state stream (C update + partial numerators)
-int block_state(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned flags) {
+int block_state(xl_handle* h, void* state, const Step& sl, int i, int T, unsigned flags) {
   const BlockPlan bp = block_plan(h, sl, T, flags);
   const int small_nch = smallm_chunks(h, sl, T, flags);
   // (few-env path: fp32 g for the GEMV proj_down and no split-K planes -- the same parameters block_post() builds,
@@ -500,12 +502,12 @@ int block_state(xl_handle* h, void* state, const Slice& sl, int i, int T, unsign
 }
 
 // block i, part 3: n/m update + normalise + skip + output gate; x = x + gated W_down^T
-int block_post(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigned flags) {
+int block_post(xl_handle* h, void* state, const Step& sl, int i, int T, unsigned flags) {
   const xl_config& c = h->cfg;
   const BlockPlan bp = block_plan(h, sl, T, flags);
   const int small_nch = smallm_chunks(h, sl, T, flags);
   const Ws& ws = sl.ws;
-  const int M = sl.Bk * T;
+  const int M = sl.B * T;
   if (small_nch) {
     // M <= 16 rows: finalize emits fp32 g, then x += g W_down^T as warp GEMVs (xl_smallm.cu)
     xl::StateStepParams sp = state_params(h, state, sl, i, T, /*tc_down=*/false, 1, small_nch);
@@ -533,19 +535,19 @@ int block_post(xl_handle* h, void* state, const Slice& sl, int i, int T, unsigne
 }
 
 // sLSTM block i (sLSTM layer + gated feed-forward) over the M = Bk*T rows of ws.x (rows [env][token]), envs
-// [b0, b0+Bk) of a state holding Btot envs. pend_sp > 1: the previous mLSTM block left that many split-K
+// [0, Bk) of a state holding Btot envs. pend_sp > 1: the previous mLSTM block left that many split-K
 // proj_down planes, folded into x by this block's first LayerNorm. Workspace reuse: xn = LN(x), act = swish(conv),
 // u = gate pre-activations [M,4,d], gated = y [M,d], qkv = feed-forward up projection [M,2ff].
-// len / pos (ragged prefill, b0 == 0): env b of the slice has clamp(len[b] - pos, 0, T) real tokens, pads after them
-int slstm_block(xl_handle* h, void* state, const Ws& ws, int Btot, int b0, int Bk, int i, int T, unsigned flags,
+// len / pos (ragged prefill): env b has clamp(len[b] - pos, 0, T) real tokens, pads after them
+int slstm_block(xl_handle* h, void* state, const Ws& ws, int Btot, int Bk, int i, int T, unsigned flags,
                 int pend_sp, cudaStream_t s, const int32_t* len = nullptr, int pos = 0) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim, NH = c.num_heads, ff = c.ffn_dim, KS = c.conv_kernel, M = Bk * T;
   const StateLayout L = state_layout(h, Btot);
   const BlockWeights& w = h->blocks[i];
   char* base = (char*)state + layer_base(h, L, i);
-  float* st = (float*)(base + L.s_off) + (size_t)b0 * d;                   // (y,c,n,m), part stride Btot*d
-  float* conv = (float*)(base + L.sconv_off) + (size_t)b0 * KS * d;
+  float* st = (float*)(base + L.s_off);                   // (y,c,n,m), part stride Btot*d
+  float* conv = (float*)(base + L.sconv_off);
   const int impl = (flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
   const bool tc_up = impl != 1 && xl::gemm_tc_supported(M, 2 * ff, d) && (size_t)M * d <= ws.a_cap;
   const bool tc_down = impl != 1 && xl::gemm_tc_supported(M, d, ff) && (size_t)M * ff <= ws.a_cap;
@@ -577,15 +579,15 @@ int slstm_block(xl_handle* h, void* state, const Ws& ws, int Btot, int b0, int B
 }
 
 // split-K planes the block before i leaves for i's first LayerNorm (1 = none)
-int pending_planes(const xl_handle* h, const Slice& sl, int i, int T, unsigned flags) {
+int pending_planes(const xl_handle* h, const Step& sl, int i, int T, unsigned flags) {
   if (i == 0 || is_slstm(h, i - 1)) return 1;
   return block_plan(h, sl, T, flags).down_sp;
 }
 
-// post_blocks_norm over the M = Bk*T rows of ws.x left by run_blocks (folds the last block's split-K planes)
-void final_norm(xl_handle* h, const Slice& sl, int T, unsigned flags, float* out, int64_t out_stride) {
+// post_blocks_norm over the M = B*T rows of ws.x left by run_blocks (folds the last block's split-K planes)
+void final_norm(xl_handle* h, const Step& sl, int T, unsigned flags, float* out, int64_t out_stride) {
   const xl_config& c = h->cfg;
-  const int d = c.embedding_dim, M = sl.Bk * T;
+  const int d = c.embedding_dim, M = sl.B * T;
   const BlockPlan bp = block_plan(h, sl, T, flags);
   const float* post_w = (const float*)h->pw[XL_W_POST_NORM - XL_W_POST_NORM];
   if (bp.down_sp > 1 && !is_slstm(h, c.num_blocks - 1))
@@ -596,39 +598,39 @@ void final_norm(xl_handle* h, const Slice& sl, int T, unsigned flags, float* out
   h->launches += 1;
 }
 
-// One pass of the block stack over M = Bk*T rows held in ws.x (rows ordered [b][t]).
-int run_blocks(xl_handle* h, void* state, const Slice& sl, int T, unsigned flags) {
+// One pass of the block stack over M = B*T rows held in ws.x (rows ordered [b][t]).
+int run_blocks(xl_handle* h, void* state, const Step& sl, int T, unsigned flags) {
   const int L = h->cfg.num_blocks;
-  // L2 warm-up of the next block's C on side stream 0 (whole-batch slices only; side streams belong to the
-  // micro-batches otherwise). Block 0 of the NEXT env step is warmed after the last block's state kernel.
+  // L2 warm-up of the next block's C on the side stream. Block 0 of the NEXT env step is warmed after the last block's
+  // state kernel.
   const StateLayout lay = state_layout(h, sl.B);
   const size_t c_bytes = sizeof(float) * (size_t)sl.B * h->cfg.num_heads * h->DH * h->DH;
   int warm_mb = h->l2_prefetch_mb;
   if (warm_mb < 0) warm_mb = (c_bytes >= ((size_t)100 << 20) && c_bytes <= ((size_t)300 << 20)) ? 48 : 0;
-  const bool warm = warm_mb > 0 && sl.b0 == 0 && sl.Bk == sl.B && L > 1;
+  const bool warm = warm_mb > 0 && L > 1;
   const size_t warm_bytes = std::min(c_bytes, (size_t)warm_mb << 20);
   int rc = XL_OK;
   for (int i = 0; i < L && !rc; ++i) {
     if (is_slstm(h, i)) {
-      rc = slstm_block(h, state, sl.ws, sl.B, sl.b0, sl.Bk, i, T, flags, pending_planes(h, sl, i, T, flags), sl.s);
+      rc = slstm_block(h, state, sl.ws, sl.B, sl.B, i, T, flags, pending_planes(h, sl, i, T, flags), sl.s);
       continue;
     }
     rc = block_pre(h, state, sl, i, T, flags);
     if (!rc) rc = block_state(h, state, sl, i, T, flags);
     if (!rc && warm) {
-      XL_CUDA(cudaEventRecord(h->ev_state[0], sl.s));
-      XL_CUDA(cudaStreamWaitEvent(h->side[0], h->ev_state[0], 0));
+      XL_CUDA(cudaEventRecord(h->ev_fork, sl.s));
+      XL_CUDA(cudaStreamWaitEvent(h->side, h->ev_fork, 0));
       int nx = (i + 1) % L;
       while (is_slstm(h, nx) && nx != i) nx = (nx + 1) % L;        // next mLSTM block
       const char* next_c = (const char*)state + layer_base(h, lay, nx) + lay.c_off;
-      xl::launch_l2_prefetch(next_c, warm_bytes, h->num_sms, h->l2_prefetch_policy, h->side[0]);
+      xl::launch_l2_prefetch(next_c, warm_bytes, h->num_sms, h->l2_prefetch_policy, h->side);
       h->launches += 1;
     }
     if (!rc) rc = block_post(h, state, sl, i, T, flags);
   }
   if (warm) {   // join (also on the error path: a capture must not end with an unjoined stream)
-    cudaEventRecord(h->ev_join[0], h->side[0]);
-    cudaStreamWaitEvent(sl.s, h->ev_join[0], 0);
+    cudaEventRecord(h->ev_join, h->side);
+    cudaStreamWaitEvent(sl.s, h->ev_join, 0);
   }
   if (rc) return rc;
   XL_CUDA(cudaGetLastError());
@@ -636,11 +638,11 @@ int run_blocks(xl_handle* h, void* state, const Slice& sl, int T, unsigned flags
 }
 
 // Encoder over x_in [B,T,d] -> x_out [B,T,d] (post_blocks_norm applied), single stream.
-int run_encoder(xl_handle* h, void* state, const Slice& sl, const float* x_in, float* x_out, int T, int mode,
+int run_encoder(xl_handle* h, void* state, const Step& sl, const float* x_in, float* x_out, int T, int mode,
                 unsigned flags) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim;
-  const int B = sl.Bk;
+  const int B = sl.B;
   const Ws& ws = sl.ws;
   cudaStream_t s = sl.s;
   const float* post_w = (const float*)h->pw[XL_W_POST_NORM - XL_W_POST_NORM];
@@ -650,7 +652,7 @@ int run_encoder(xl_handle* h, void* state, const Slice& sl, const float* x_in, f
     }
     int rc = run_blocks(h, state, sl, T, flags);
     if (rc) return rc;
-    if (!(flags & kFlagHeadOnlyEarly)) final_norm(h, sl, T, flags, x_out, d);
+    if (!(flags & kFlagHeadOnly)) final_norm(h, sl, T, flags, x_out, d);
   } else if (mode == XL_MODE_PER_TOKEN) {
     // reference order: for token: for block  (decision_xlstm.py:161-165). x_in may alias x_out: token t's
     // input row is consumed (gathered) before its output row is written.
@@ -673,12 +675,6 @@ int run_encoder(xl_handle* h, void* state, const Slice& sl, const float* x_in, f
   return XL_OK;
 }
 
-constexpr unsigned kFlagLn0Done = 1u << 29;     // internal: the embed kernel already ran block 0's pre-norm (operands in place)
-constexpr unsigned kFlagHeadOnly = 1u << 28;    // internal: nobody reads the hidden states: post_blocks_norm only on the
-                                                // action-token rows, fused with the head's operand split (policy_back)
-constexpr unsigned kFlagNoRing = 1u << 30;      // internal: steps run on behalf of xl_policy_prefill leave the token ring
-                                                // and the sampler alone (argmax, no step counted)
-
 // Arguments of one policy step (device pointers for the WHOLE batch of B envs).
 struct StepArgs {
   void* state;
@@ -689,8 +685,8 @@ struct StepArgs {
   unsigned flags;
 };
 
-// embed_state Linear(204 -> d) on zero-padded K, (s, rtg, r) token embedding + embed_ln -> xt [Bk, 3, d]
-int policy_front(xl_handle* h, const StepArgs& a, const Slice& sl, float* xt) {
+// embed_state Linear(204 -> d) on zero-padded K, (s, rtg, r) token embedding + embed_ln -> xt [B, 3, d]
+int policy_front(xl_handle* h, const StepArgs& a, const Step& sl, float* xt) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim;
   const int impl = (a.flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
@@ -700,17 +696,17 @@ int policy_front(xl_handle* h, const StepArgs& a, const Slice& sl, float* xt) {
   if (a.flags & XL_FLAG_STATE_EMBEDS) {
     // a.states already holds the state-token embeddings [B, d] (image observations: embed_image = ImpalaCNN,
     // discrete_decision_transformer_model.py:187-203, runs in PyTorch/cuDNN before this call)
-    s_emb = a.states + (size_t)sl.b0 * d;
+    s_emb = a.states;
   } else {
-    const bool tc = impl != 1 && xl::gemm_tc_supported(sl.Bk, d, h->Kpad) && (size_t)sl.Bk * h->Kpad <= ws.a_cap;
+    const bool tc = impl != 1 && xl::gemm_tc_supported(sl.B, d, h->Kpad) && (size_t)sl.B * h->Kpad <= ws.a_cap;
     if (tc) {       // zero-pad + bf16 hi/lo split in one kernel, straight into the GEMM's operand planes
-      xl::launch_pad_split(a.states + (size_t)sl.b0 * c.state_dim, c.state_dim, ws.a_hi, ws.a_lo, h->Kpad, sl.Bk, sl.s);
+      xl::launch_pad_split(a.states, c.state_dim, ws.a_hi, ws.a_lo, h->Kpad, sl.B, sl.s);
     } else {
-      xl::launch_pad_rows(a.states + (size_t)sl.b0 * c.state_dim, c.state_dim, ws.states_pad, h->Kpad, sl.Bk, sl.s);
+      xl::launch_pad_rows(a.states, c.state_dim, ws.states_pad, h->Kpad, sl.B, sl.s);
     }
     h->launches += 1;
     int rc = linear(h, ws, ws.states_pad, PW(XL_W_EMBED_STATE_W), (const float*)PW(XL_W_EMBED_STATE_B), nullptr,
-                    ws.s_emb, sl.Bk, d, h->Kpad, impl, sl.s, /*presplit=*/tc);
+                    ws.s_emb, sl.B, d, h->Kpad, impl, sl.s, /*presplit=*/tc);
     if (rc) return rc;
   }
   // block 0's pre-norm rides on the embed kernel when the stack will consume it as is (kFlagLn0Done set by run_policy)
@@ -722,163 +718,98 @@ int policy_front(xl_handle* h, const StepArgs& a, const Slice& sl, float* xt) {
     ln0_w = (const float*)h->blocks[0].w[XL_W_XLSTM_NORM];
     if (bp.tc_up) { hi0 = ws.a_hi; lo0 = ws.a_lo; } else { xn0 = ws.xn; }
   }
-  xl::launch_embed_tokens(s_emb, a.rtg + sl.b0, a.rewards ? a.rewards + sl.b0 : nullptr,
+  xl::launch_embed_tokens(s_emb, a.rtg, a.rewards,
                           (const float*)PW(XL_W_EMBED_RETURN_W), (const float*)PW(XL_W_EMBED_RETURN_B),
                           (const float*)PW(XL_W_EMBED_REWARD_W), (const float*)PW(XL_W_EMBED_REWARD_B),
                           (const float*)PW(XL_W_EMBED_LN_W), (const float*)PW(XL_W_EMBED_LN_B), c.embed_ln_eps, xt,
-                          sl.Bk, d, (h->tok_ring && sl.b0 == 0 && !(a.flags & kFlagNoRing)) ? h->counters + kCntRing : nullptr,
-                          (h->sampling && sl.b0 == 0 && !(a.flags & kFlagNoRing)) ? h->counters + kCntSample : nullptr,
+                          sl.B, d, (h->tok_ring && !(a.flags & kFlagNoRing)) ? h->counters + kCntRing : nullptr,
+                          (h->sampling && !(a.flags & kFlagNoRing)) ? h->counters + kCntSample : nullptr,
                           ln0_w, c.ln_eps, xn0, hi0, lo0, sl.s);
   h->launches += 1;
   return XL_OK;
 }
 
-// action head on the rtg token of hid [Bk, T, d] -> logits -> argmax / inv_tokenize
-int policy_back(xl_handle* h, const StepArgs& a, const Slice& sl, const float* hid) {
+// action head on the rtg token of hid [B, T, d] -> logits -> argmax / inv_tokenize
+int policy_back(xl_handle* h, const StepArgs& a, const Step& sl, const float* hid) {
   const xl_config& c = h->cfg;
   const int d = c.embedding_dim, T = c.tokens_per_step;
   const int impl = (a.flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
   auto PW = [&](int id) { return h->pw[id - XL_W_POST_NORM]; };
   const Ws& ws = sl.ws;
   cudaStream_t s = sl.s;
-  const int Bk = sl.Bk;
-  // gather row b*T + pos to a dense [Bk,d], then Linear(d -> 2192 / 274)
-  float* xa = ws.s_emb;  // reuse [Bk,d]
+  const int B = sl.B;
+  // gather row b*T + pos to a dense [B,d], then Linear(d -> 2192 / 274)
+  float* xa = ws.s_emb;  // reuse [B,d]
   const bool head_only = (a.flags & kFlagHeadOnly) != 0;
   if (head_only) {
     // post_blocks_norm of the action-token rows only (+ the last proj_down's pending planes), emitted as the head
     // GEMM's bf16 hi/lo operand planes: one launch instead of norm-all-rows + gather + split
     const BlockPlan bp = block_plan(h, sl, T, a.flags);
     const int pend = is_slstm(h, c.num_blocks - 1) ? 1 : bp.down_sp;
-    xl::launch_ln_rows_gather(ws.x, h->part_down, pend, (int64_t)Bk * T * d, (const float*)PW(XL_W_POST_NORM), c.ln_eps,
-                              Bk, d, T, c.action_token_pos, ws.a_hi, ws.a_lo, s);
+    xl::launch_ln_rows_gather(ws.x, h->part_down, pend, (int64_t)B * T * d, (const float*)PW(XL_W_POST_NORM), c.ln_eps,
+                              B, d, T, c.action_token_pos, ws.a_hi, ws.a_lo, s);
   } else {
-    xl::launch_copy_rows(hid + (size_t)c.action_token_pos * d, (int64_t)T * d, xa, d, Bk, d, s);
+    xl::launch_copy_rows(hid + (size_t)c.action_token_pos * d, (int64_t)T * d, xa, d, B, d, s);
   }
   h->launches += 1;
   const bool discrete = (a.flags & XL_FLAG_DISCRETE) != 0;
   // discrete branch only needs the first num_actions logits (multi_domain_discrete_dt_model.py:99-101)
   const int n_out = discrete ? h->num_actions : h->head_out;
-  int32_t* tokens = a.tokens + (size_t)sl.b0 * c.act_dim;
-  float* actions = a.actions + (size_t)sl.b0 * c.act_dim;
-  float* logits = a.logits ? a.logits + (size_t)sl.b0 * n_out : nullptr;
   int rc;
-  int32_t* ring = (h->tok_ring && !(a.flags & kFlagNoRing)) ? h->tok_ring + (size_t)sl.b0 * c.act_dim : nullptr;
-  const int64_t ring_stride = (int64_t)a.B * c.act_dim;
+  int32_t* ring = (h->tok_ring && !(a.flags & kFlagNoRing)) ? h->tok_ring : nullptr;
+  const int64_t ring_stride = (int64_t)B * c.act_dim;
   const bool sample = h->sampling && !(a.flags & kFlagNoRing);
   const float bw = (c.tok_max_val - c.tok_min_val) / (float)c.action_channels;
   if (discrete) {
-    rc = linear(h, ws, xa, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, ws.logits, Bk, n_out, d, impl, s,
+    rc = linear(h, ws, xa, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, ws.logits, B, n_out, d, impl, s,
                 head_only);
     if (rc) return rc;
-    if (logits) {
-      XL_CUDA(cudaMemcpyAsync(logits, ws.logits, sizeof(float) * (size_t)Bk * n_out, cudaMemcpyDeviceToDevice, s));
+    if (a.logits) {
+      XL_CUDA(cudaMemcpyAsync(a.logits, ws.logits, sizeof(float) * (size_t)B * n_out, cudaMemcpyDeviceToDevice, s));
     }
     if (sample)
-      xl::launch_sample_tokens(ws.logits, n_out, Bk, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, tokens, actions,
-                               ring, h->counters + kCntRing, h->tok_slots, ring_stride, h->counters + kCntArmed,
-                               h->counters + kCntSample, sl.b0, s);
+      xl::launch_sample_tokens(ws.logits, n_out, B, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, a.tokens,
+                               a.actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride,
+                               h->counters + kCntArmed, h->counters + kCntSample, s);
     else
-      xl::launch_argmax_tokens(ws.logits, n_out, Bk, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, tokens,
-                               actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride, s);
+      xl::launch_argmax_tokens(ws.logits, n_out, B, c.act_dim, n_out, c.discrete_actions, 1, 0.f, 0.f, a.tokens,
+                               a.actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride, s);
   } else {
-    float* lg = logits ? logits : ws.logits;
-    rc = linear(h, ws, xa, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, lg, Bk, n_out, d, impl, s, head_only);
+    float* lg = a.logits ? a.logits : ws.logits;
+    rc = linear(h, ws, xa, PW(XL_W_HEAD_W), (const float*)PW(XL_W_HEAD_B), nullptr, lg, B, n_out, d, impl, s, head_only);
     if (rc) return rc;
     if (sample)
-      xl::launch_sample_tokens(lg, h->head_out, Bk, c.act_dim, h->num_actions, c.discrete_actions, 0, bw, c.tok_min_val,
-                               tokens, actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride,
-                               h->counters + kCntArmed, h->counters + kCntSample, sl.b0, s);
+      xl::launch_sample_tokens(lg, h->head_out, B, c.act_dim, h->num_actions, c.discrete_actions, 0, bw, c.tok_min_val,
+                               a.tokens, a.actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride,
+                               h->counters + kCntArmed, h->counters + kCntSample, s);
     else
-      xl::launch_argmax_tokens(lg, h->head_out, Bk, c.act_dim, h->num_actions, c.discrete_actions, 0, bw,
-                               c.tok_min_val, tokens, actions, ring, h->counters + kCntRing, h->tok_slots, ring_stride, s);
+      xl::launch_argmax_tokens(lg, h->head_out, B, c.act_dim, h->num_actions, c.discrete_actions, 0, bw,
+                               c.tok_min_val, a.tokens, a.actions, ring, h->counters + kCntRing, h->tok_slots,
+                               ring_stride, s);
   }
   h->launches += 1;
   return XL_OK;
 }
 
-// How many env micro-batches a fused step is split into. The state stream of one micro-batch (HBM-bound)
-// overlaps the latency-bound LayerNorm / projection / conv / finalize chain of the others.
-int pick_microbatches(const xl_handle* h, int B, int mode) {
-  if (mode != XL_MODE_FUSED) return 1;
-  // Measured on B200 (profiles/r01_microbatch_pipeline.md): the chain kernels are memory-LATENCY bound and slow
-  // down under a saturated memory system by about what the overlap gains, so the default is one batch.
-  int mb = h->microbatches > 0 ? h->microbatches : 1;
-  if (mb > kMaxMicro) mb = kMaxMicro;
-  if (mb > B) mb = B;
-  return mb < 1 ? 1 : mb;
-}
-
-int run_policy(xl_handle* h, const StepArgs& a, cudaStream_t s) {
-  const xl_config& c = h->cfg;
-  const int d = c.embedding_dim, T = c.tokens_per_step;
-  const float* post_w = (const float*)h->pw[XL_W_POST_NORM - XL_W_POST_NORM];
-  const int MB = pick_microbatches(h, a.B, a.mode);
-  if (MB == 1) {
-    const Slice sl = make_slice(h, a.B, 0, a.B, s);
-    float* xt = (a.mode == XL_MODE_FUSED) ? sl.ws.x : sl.ws.xtok;
-    // launch-saving fusions of the step's head and tail (fused mode, multi-kernel stack)
-    StepArgs af = a;
-    if (h->fuse_ends && a.mode == XL_MODE_FUSED && !h->debug_skip) {
-      if (!is_slstm(h, 0) && !smallm_chunks(h, sl, T, a.flags)) af.flags |= kFlagLn0Done;
-      const int impl = (a.flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
-      const int n_out = (a.flags & XL_FLAG_DISCRETE) ? h->num_actions : h->head_out;
-      if (!a.hidden && impl != 1 && xl::gemm_tc_supported(a.B, n_out, d) && (size_t)a.B * d <= sl.ws.a_cap &&
-          d <= 4096)
-        af.flags |= kFlagHeadOnly;
-    }
-    const StepArgs& a = af;        // (shadows the parameter for the rest of this branch)
-    int rc = policy_front(h, a, sl, xt);
-    if (rc) return rc;
-    float* hid = a.hidden ? a.hidden : sl.ws.hid;
-    rc = run_encoder(h, a.state, sl, xt, hid, T, a.mode, a.flags);
-    if (rc) return rc;
-    rc = policy_back(h, a, sl, hid);
-    if (rc) return rc;
-    XL_CUDA(cudaGetLastError());
-    return XL_OK;
+int run_policy(xl_handle* h, const StepArgs& args, cudaStream_t s) {
+  const int d = h->cfg.embedding_dim, T = h->cfg.tokens_per_step;
+  const Step sl = make_step(h, args.B, s);
+  float* xt = (args.mode == XL_MODE_FUSED) ? sl.ws.x : sl.ws.xtok;
+  // launch-saving fusions of the step's head and tail (fused mode, multi-kernel stack)
+  StepArgs a = args;
+  if (h->fuse_ends && a.mode == XL_MODE_FUSED && !h->debug_skip) {
+    if (!is_slstm(h, 0) && !smallm_chunks(h, sl, T, a.flags)) a.flags |= kFlagLn0Done;
+    const int impl = (a.flags & XL_FLAG_SIMPLE_GEMM) ? 1 : h->gemm_impl;
+    const int n_out = (a.flags & XL_FLAG_DISCRETE) ? h->num_actions : h->head_out;
+    if (!a.hidden && impl != 1 && xl::gemm_tc_supported(a.B, n_out, d) && (size_t)a.B * d <= sl.ws.a_cap && d <= 4096)
+      a.flags |= kFlagHeadOnly;
   }
-  // ---- fused step, MB env micro-batches: slice 0 on the caller's stream, the others on side streams ----
-  Slice sl[kMaxMicro];
-  int b0 = 0;
-  for (int k = 0; k < MB; ++k) {
-    const int Bk = a.B / MB + (k < a.B % MB ? 1 : 0);
-    sl[k] = make_slice(h, a.B, b0, Bk, k == 0 ? s : h->side[k - 1]);
-    sl[k].ws.low_smem = 1;
-    b0 += Bk;
-  }
-  XL_CUDA(cudaEventRecord(h->ev_fork, s));
-  for (int k = 1; k < MB; ++k) XL_CUDA(cudaStreamWaitEvent(sl[k].s, h->ev_fork, 0));
-  int rc = XL_OK;
-  for (int k = 0; k < MB && !rc; ++k) rc = policy_front(h, a, sl[k], sl[k].ws.x);
-  for (int i = 0; i < c.num_blocks && !rc; ++i) {
-    if (is_slstm(h, i)) {
-      for (int k = 0; k < MB && !rc; ++k)
-        rc = slstm_block(h, a.state, sl[k].ws, a.B, sl[k].b0, sl[k].Bk, i, T, a.flags,
-                         pending_planes(h, sl[k], i, T, a.flags), sl[k].s);
-      continue;
-    }
-    for (int k = 0; k < MB && !rc; ++k) rc = block_pre(h, a.state, sl[k], i, T, a.flags);
-    for (int k = 0; k < MB && !rc; ++k) {
-      if (h->pipeline_order && !(i == 0 && k == 0)) {
-        // the HBM-bound kernels take turns: S(k, i) starts when S(k-1, i) (or S(MB-1, i-1)) has finished
-        XL_CUDA(cudaStreamWaitEvent(sl[k].s, h->ev_state[(k + MB - 1) % MB], 0));
-      }
-      rc = block_state(h, a.state, sl[k], i, T, a.flags);
-      if (!rc && h->pipeline_order) XL_CUDA(cudaEventRecord(h->ev_state[k], sl[k].s));
-    }
-    for (int k = 0; k < MB && !rc; ++k) rc = block_post(h, a.state, sl[k], i, T, a.flags);
-  }
-  for (int k = 0; k < MB && !rc; ++k) {
-    float* hid = a.hidden ? a.hidden + (size_t)sl[k].b0 * T * d : sl[k].ws.hid;
-    final_norm(h, sl[k], T, a.flags, hid, d);
-    rc = policy_back(h, a, sl[k], hid);
-  }
-  // join (also on the error path, so that a capture never ends with unjoined streams)
-  for (int k = 1; k < MB; ++k) {
-    cudaEventRecord(h->ev_join[k - 1], sl[k].s);
-    cudaStreamWaitEvent(s, h->ev_join[k - 1], 0);
-  }
+  int rc = policy_front(h, a, sl, xt);
+  if (rc) return rc;
+  float* hid = a.hidden ? a.hidden : sl.ws.hid;
+  rc = run_encoder(h, a.state, sl, xt, hid, T, a.mode, a.flags);
+  if (rc) return rc;
+  rc = policy_back(h, a, sl, hid);
   if (rc) return rc;
   XL_CUDA(cudaGetLastError());
   return XL_OK;
@@ -953,7 +884,6 @@ Ws prefill_ws(const xl_handle* h) {
   w.a_hi = h->pf_hi; w.a_lo = h->pf_lo;
   const size_t kmax = std::max(std::max((size_t)h->cfg.inner_dim, (size_t)h->cfg.embedding_dim), (size_t)h->Kpad);
   w.a_cap = (size_t)h->pf_rows * kmax;
-  w.low_smem = h->prefill_gemm_2cta;
   return w;
 }
 
@@ -986,7 +916,7 @@ int seq_cell(xl_handle* h, float* C, float* n, float* m_state, const float* q, c
   XL_CUDA(cudaGetLastError());
   if (which == 2) {
     if (int rcw = ensure_prefill_tc_ws(h, B, Sc)) return rcw;
-    const xl::CellSideStream side = {h->side[0], h->ev_fork, h->ev_join[0]};
+    const xl::CellSideStream side = {h->side, h->ev_fork, h->ev_join};
     XL_CUDA(xl::launch_cell_tc(C, n, q, k, v, h->pf_f, h->pf_i, num, qn, h->pf_tc, B, Sc, NH, DH, inner, s, &side));
     h->launches += 6;
     XL_CUDA(cudaGetLastError());
@@ -1026,7 +956,7 @@ int prefill_blocks(xl_handle* h, void* state, int Btot, int B, int Sc, unsigned 
     if (is_slstm(h, i)) {
       // no parallel form exists for the sLSTM: its cell runs token by token (Sc launches of a tiny kernel), the
       // rest of the block (conv, gate projections, GroupNorm, feed-forward) over the whole chunk
-      int rcs = slstm_block(h, state, ws, Btot, 0, B, i, Sc, flags, 1, s, len, pos);
+      int rcs = slstm_block(h, state, ws, Btot, B, i, Sc, flags, 1, s, len, pos);
       if (rcs) return rcs;
       continue;
     }
@@ -1333,6 +1263,72 @@ int seq_clear_outputs(const xl_handle* h, const SeqHead& hd, int B, cudaStream_t
   return XL_OK;
 }
 
+// encoder_only: the block stack + post_blocks_norm (what xl_encoder_step / xl_prefill read); otherwise also the
+// policy-level embeddings and the action head (xl_policy_*).
+int weights_ready(const xl_handle* h, bool encoder_only) {
+  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
+  static const int s_ids[] = {XL_W_XLSTM_NORM, XL_W_CONV_W, XL_W_CONV_B, XL_W_S_GATE_I, XL_W_S_GATE_F, XL_W_S_GATE_Z,
+                              XL_W_S_GATE_O, XL_W_S_RECURRENT, XL_W_S_BIAS, XL_W_S_GROUP_NORM, XL_W_FFN_NORM,
+                              XL_W_FFN_UP, XL_W_FFN_DOWN};
+  for (int i = 0; i < h->cfg.num_blocks; ++i) {
+    if (is_slstm(h, i)) {
+      for (int k : s_ids)
+        if (!h->blocks[i].w[k]) return fail(XL_ERR_NOT_READY, "sLSTM block %d weight id %d not bound", i, k);
+      continue;
+    }
+    for (int k = 0; k <= XL_W_PROJ_DOWN; ++k)
+      if (!h->blocks[i].w[k]) return fail(XL_ERR_NOT_READY, "block %d weight id %d not bound", i, k);
+  }
+  const int last = encoder_only ? XL_W_POST_NORM : XL_W_HEAD_B;
+  for (int id = XL_W_POST_NORM; id <= last; ++id)
+    if (!h->pw[id - XL_W_POST_NORM]) return fail(XL_ERR_NOT_READY, "policy weight id %d not bound", id);
+  return XL_OK;
+}
+
+// CUDA-graph replay of a step entry: replays the graph captured for `key`, or captures record(stream) -- which enqueues
+// the step on the stream it is given -- into a new graph on cap_stream and launches it. At most 8 graphs are kept,
+// the oldest evicted first. h->launches counts the graph's kernels on every launch; the capture itself counts none.
+template <class Record>
+int run_graph(xl_handle* h, const GraphKey& key, cudaStream_t s, Record&& record) {
+  for (auto& g : h->graphs) {
+    if (g.key == key) {
+      XL_CUDA(cudaGraphLaunch(g.exec, s));
+      h->launches += g.launches;
+      return XL_OK;
+    }
+  }
+  int rc = weights_ready(h, key.entry == GraphKey::kEncoderStep);
+  if (rc) return rc;
+  // make sure every lazy attribute (dynamic smem opt-in) is set before capture: one eager warm-up is NOT
+  // done here because it would advance the state; attributes are set inside launch paths, which is legal
+  // during capture (cudaFuncSetAttribute is not a stream operation).
+  GraphCacheEntry g;
+  g.key = key;
+  cudaGraph_t graph = nullptr;
+  const int64_t before = h->launches;
+  XL_CUDA(cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
+  rc = record(h->cap_stream);
+  cudaError_t e = cudaStreamEndCapture(h->cap_stream, &graph);
+  g.launches = h->launches - before;
+  h->launches = before;
+  if (rc) {
+    if (graph) cudaGraphDestroy(graph);
+    return rc;
+  }
+  if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
+  e = cudaGraphInstantiate(&g.exec, graph, 0);
+  cudaGraphDestroy(graph);
+  if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(e));
+  if (h->graphs.size() >= 8) {
+    cudaGraphExecDestroy(h->graphs.front().exec);
+    h->graphs.erase(h->graphs.begin());
+  }
+  h->graphs.push_back(g);
+  XL_CUDA(cudaGraphLaunch(g.exec, s));
+  h->launches += g.launches;
+  return XL_OK;
+}
+
 }  // namespace
 
 // =================================================================================================
@@ -1427,7 +1423,6 @@ int xl_create(const xl_config* cfg, xl_handle** out) {
   if (a_cap < B * (size_t)h->Kpad) a_cap = B * (size_t)h->Kpad;
   if (a_cap < (size_t)1 << 20) a_cap = (size_t)1 << 20;   // room for xl_linear unit tests
   h->a_cap = a_cap;
-  h->a_env = 4 * (inner > d ? inner : d);
   const size_t o_hi = carve(2 * a_cap), o_lo = carve(2 * a_cap);
   h->part_rows = M < kSplitRows ? M : kSplitRows;
   const size_t o_pu = carve(4 * (size_t)kSplitMax * h->part_rows * 2 * inner);
@@ -1441,12 +1436,9 @@ int xl_create(const xl_config* cfg, xl_handle** out) {
   }
   cudaMemset(h->ws, 0, h->ws_bytes);
   cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking);
-  for (int k = 0; k < kMaxMicro - 1; ++k) {
-    cudaStreamCreateWithFlags(&h->side[k], cudaStreamNonBlocking);
-    cudaEventCreateWithFlags(&h->ev_join[k], cudaEventDisableTiming);
-  }
-  for (int k = 0; k < kMaxMicro; ++k) cudaEventCreateWithFlags(&h->ev_state[k], cudaEventDisableTiming);
+  cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking);
   cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming);
+  cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
   h->x = (float*)(h->ws + o_x); h->xn = (float*)(h->ws + o_xn); h->xtok = (float*)(h->ws + o_xtok);
   h->hid = (float*)(h->ws + o_hid);
   h->u = (float*)(h->ws + o_u); h->qkv = (float*)(h->ws + o_qkv); h->act = (float*)(h->ws + o_act);
@@ -1466,8 +1458,7 @@ int xl_create(const xl_config* cfg, xl_handle** out) {
 
 void xl_destroy(xl_handle* h) {
   if (!h) return;
-  for (auto& g : h->graphs)
-    if (g.exec) cudaGraphExecDestroy(g.exec);
+  clear_graphs(h);
   if (h->ws) cudaFree(h->ws);
   if (h->pf_tc) cudaFree(h->pf_tc);
   if (h->pf_buf) cudaFree(h->pf_buf);
@@ -1475,13 +1466,9 @@ void xl_destroy(xl_handle* h) {
   if (h->rg_idx) cudaFree(h->rg_idx);
   if (h->sq_logits) cudaFree(h->sq_logits);
   if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
-  for (int k = 0; k < kMaxMicro - 1; ++k) {
-    if (h->side[k]) cudaStreamDestroy(h->side[k]);
-    if (h->ev_join[k]) cudaEventDestroy(h->ev_join[k]);
-  }
-  for (int k = 0; k < kMaxMicro; ++k)
-    if (h->ev_state[k]) cudaEventDestroy(h->ev_state[k]);
+  if (h->side) cudaStreamDestroy(h->side);
   if (h->ev_fork) cudaEventDestroy(h->ev_fork);
+  if (h->ev_join) cudaEventDestroy(h->ev_join);
   delete h;
 }
 
@@ -1538,32 +1525,7 @@ int xl_bind_weight(xl_handle* h, int layer, int which, const void* dev_ptr, int 
   if (((uintptr_t)dev_ptr) % 16) return fail(XL_ERR_INVALID_ARG, "weight pointer must be 16-byte aligned");
   if (layer >= 0) h->blocks[layer].w[which] = dev_ptr;
   else h->pw[which - XL_W_POST_NORM] = dev_ptr;
-  // bound pointers are baked into cached graphs
-  for (auto& g : h->graphs)
-    if (g.exec) cudaGraphExecDestroy(g.exec);
-  h->graphs.clear();
-  return XL_OK;
-}
-
-// encoder_only: the block stack + post_blocks_norm (what xl_encoder_step / xl_prefill read); otherwise also the
-// policy-level embeddings and the action head (xl_policy_*).
-static int weights_ready(const xl_handle* h, bool encoder_only) {
-  if (!h) return fail(XL_ERR_INVALID_ARG, "null handle");
-  static const int s_ids[] = {XL_W_XLSTM_NORM, XL_W_CONV_W, XL_W_CONV_B, XL_W_S_GATE_I, XL_W_S_GATE_F, XL_W_S_GATE_Z,
-                              XL_W_S_GATE_O, XL_W_S_RECURRENT, XL_W_S_BIAS, XL_W_S_GROUP_NORM, XL_W_FFN_NORM,
-                              XL_W_FFN_UP, XL_W_FFN_DOWN};
-  for (int i = 0; i < h->cfg.num_blocks; ++i) {
-    if (is_slstm(h, i)) {
-      for (int k : s_ids)
-        if (!h->blocks[i].w[k]) return fail(XL_ERR_NOT_READY, "sLSTM block %d weight id %d not bound", i, k);
-      continue;
-    }
-    for (int k = 0; k <= XL_W_PROJ_DOWN; ++k)
-      if (!h->blocks[i].w[k]) return fail(XL_ERR_NOT_READY, "block %d weight id %d not bound", i, k);
-  }
-  const int last = encoder_only ? XL_W_POST_NORM : XL_W_HEAD_B;
-  for (int id = XL_W_POST_NORM; id <= last; ++id)
-    if (!h->pw[id - XL_W_POST_NORM]) return fail(XL_ERR_NOT_READY, "policy weight id %d not bound", id);
+  clear_graphs(h);   // bound pointers are baked into cached graphs
   return XL_OK;
 }
 
@@ -1641,53 +1603,19 @@ int xl_encoder_step(xl_handle* h, void* state, const float* x_in, float* x_out, 
   if (rc) return rc;
   if (!state || !x_in || !x_out) return fail(XL_ERR_INVALID_ARG, "null argument");
   if (T < 1 || T > 4) return fail(XL_ERR_UNSUPPORTED, "T=%d outside [1,4]", T);
-  rc = weights_ready(h, true);
-  if (rc) return rc;
   cudaStream_t s = (cudaStream_t)stream;
+  auto record = [&](cudaStream_t rs) {
+    return run_encoder(h, state, make_step(h, B, rs), x_in, x_out, T, mode, flags & ~(unsigned)XL_FLAG_GRAPH);
+  };
   if (!(flags & XL_FLAG_GRAPH) || h->profiling) {
-    const Slice sl = make_slice(h, B, 0, B, s);
-    return run_encoder(h, state, sl, x_in, x_out, T, mode, flags & ~(unsigned)XL_FLAG_GRAPH);
+    rc = weights_ready(h, true);
+    return rc ? rc : record(s);
   }
-  // CUDA-graph replay of the encoder step (the encoder-only swap of decision_xlstm.py:188-189 at small batch is
-  // launch-bound when its ~6 kernels per block are enqueued eagerly): one graph per distinct argument tuple, in the
-  // same cache as the policy step's (keys: x_in in `states`, x_out in `hidden`, T in the upper bits of `mode`).
-  const int key_mode = mode | (T << 8) | (1 << 16);
-  for (auto& g : h->graphs) {
-    if (g.state == state && g.states == x_in && g.hidden == x_out && !g.rtg && !g.tokens && g.B == B &&
-        g.mode == key_mode && g.flags == flags) {
-      XL_CUDA(cudaGraphLaunch(g.exec, s));
-      h->launches += g.launches;
-      return XL_OK;
-    }
-  }
-  GraphCacheEntry g;
-  g.state = state; g.states = x_in; g.hidden = x_out; g.B = B; g.mode = key_mode; g.flags = flags;
-  cudaGraph_t graph = nullptr;
-  const int64_t before = h->launches;
-  XL_CUDA(cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
-  {
-    const Slice sl = make_slice(h, B, 0, B, h->cap_stream);
-    rc = run_encoder(h, state, sl, x_in, x_out, T, mode, flags & ~(unsigned)XL_FLAG_GRAPH);
-  }
-  cudaError_t e = cudaStreamEndCapture(h->cap_stream, &graph);
-  g.launches = h->launches - before;
-  h->launches = before;
-  if (rc) {
-    if (graph) cudaGraphDestroy(graph);
-    return rc;
-  }
-  if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
-  e = cudaGraphInstantiate(&g.exec, graph, 0);
-  cudaGraphDestroy(graph);
-  if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(e));
-  if (h->graphs.size() >= 8) {
-    cudaGraphExecDestroy(h->graphs.front().exec);
-    h->graphs.erase(h->graphs.begin());
-  }
-  h->graphs.push_back(g);
-  XL_CUDA(cudaGraphLaunch(g.exec, s));
-  h->launches += g.launches;
-  return XL_OK;
+  // the encoder-only swap of decision_xlstm.py:188-189 at small batch is launch-bound when its ~6 kernels per block
+  // are enqueued eagerly
+  const GraphKey key = {GraphKey::kEncoderStep, state, x_in, nullptr, nullptr, nullptr, nullptr, nullptr, x_out,
+                        B, T, mode, flags};
+  return run_graph(h, key, s, record);
 }
 
 int xl_mlstm_cell_step(xl_handle* h, float* C, float* n, float* m, const float* qkv, const float* igate,
@@ -1790,47 +1718,9 @@ int xl_policy_step(xl_handle* h, void* state, const float* states, const float* 
     }
     return rc;
   }
-  // ---- CUDA-graph replay: capture once per distinct argument tuple --------------------------------
-  for (auto& g : h->graphs) {
-    if (g.state == state && g.states == states && g.rtg == rtg && g.rewards == rewards &&
-        g.tokens == tokens && g.actions == actions && g.logits == logits && g.hidden == hidden && g.B == B &&
-        g.mode == mode && g.flags == flags) {
-      XL_CUDA(cudaGraphLaunch(g.exec, s));
-      h->launches += g.launches;
-      return XL_OK;
-    }
-  }
-  rc = xl_weights_ready(h);
-  if (rc) return rc;
-  // make sure every lazy attribute (dynamic smem opt-in) is set before capture: one eager warm-up is NOT
-  // done here because it would advance the state; attributes are set inside launch paths, which is legal
-  // during capture (cudaFuncSetAttribute is not a stream operation).
-  GraphCacheEntry g;
-  g.state = state; g.states = states; g.rtg = rtg; g.rewards = rewards; g.tokens = tokens; g.actions = actions;
-  g.logits = logits; g.hidden = hidden; g.B = B; g.mode = mode; g.flags = flags;
-  cudaGraph_t graph = nullptr;
-  const int64_t before = h->launches;
-  XL_CUDA(cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
-  rc = run_policy(h, args, h->cap_stream);
-  cudaError_t e = cudaStreamEndCapture(h->cap_stream, &graph);
-  g.launches = h->launches - before;
-  h->launches = before;
-  if (rc) {
-    if (graph) cudaGraphDestroy(graph);
-    return rc;
-  }
-  if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
-  e = cudaGraphInstantiate(&g.exec, graph, 0);
-  cudaGraphDestroy(graph);
-  if (e != cudaSuccess) return fail(XL_ERR_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(e));
-  if (h->graphs.size() >= 8) {
-    cudaGraphExecDestroy(h->graphs.front().exec);
-    h->graphs.erase(h->graphs.begin());
-  }
-  h->graphs.push_back(g);
-  XL_CUDA(cudaGraphLaunch(g.exec, s));
-  h->launches += g.launches;
-  return XL_OK;
+  const GraphKey key = {GraphKey::kPolicyStep, state, states, rtg, rewards, tokens, actions, logits, hidden,
+                        B, 0, mode, flags};
+  return run_graph(h, key, s, [&](cudaStream_t rs) { return run_policy(h, args, rs); });
 }
 
 int xl_policy_step_host(xl_handle* h, void* state, const float* h_states, const float* h_rtg,
@@ -2026,7 +1916,7 @@ static int run_seq(xl_handle* h, SeqCall c) {
   if ((rc = ragged_end(h, c.state, B, p, s))) return rc;
   // the eager tail (uniform calls only): fused encoder steps of <= 4 tokens ...
   if (enc) {
-    const Slice sl = make_slice(h, B, 0, B, s);
+    const Step sl = make_step(h, B, s);
     for (int pos = p.tail; pos < S;) {
       const SeqChunk ch = {pos, B, std::min(4, S - pos)};
       if ((rc = gather(ch, c.x, sl.ws.x, d))) return rc;
@@ -2112,7 +2002,7 @@ int xl_linear(xl_handle* h, const float* A, const void* W_bf16, const float* bia
               float* out, int M, int N, int K, int impl, void* stream) {
   if (!h || !A || !W_bf16 || !out) return fail(XL_ERR_INVALID_ARG, "null argument");
   if (M <= 0 || N <= 0 || K <= 0) return fail(XL_ERR_INVALID_ARG, "bad GEMM shape");
-  Ws w = ws_slice(h, 0, h->cfg.max_batch);
+  Ws w = step_ws(h, h->cfg.max_batch);
   w.a_cap = h->a_cap;                  // a stand-alone Linear may use the whole operand planes
   return linear(h, w, A, W_bf16, bias, residual, out, M, N, K, impl, (cudaStream_t)stream);
 }
@@ -2122,10 +2012,7 @@ int xl_set_token_ring(xl_handle* h, int32_t* ring, int slots, int next_slot, voi
   if (ring && (slots <= 0 || next_slot < 0 || next_slot >= slots))
     return fail(XL_ERR_INVALID_ARG, "token ring: slots=%d next_slot=%d", slots, next_slot);
   if (ring != h->tok_ring || (ring && slots != h->tok_slots)) {
-    // the ring pointer is baked into captured graphs
-    for (auto& g : h->graphs)
-      if (g.exec) cudaGraphExecDestroy(g.exec);
-    h->graphs.clear();
+    clear_graphs(h);   // the ring pointer is baked into captured graphs
     h->tok_ring = ring;
     h->tok_slots = ring ? slots : 0;
   }
@@ -2159,9 +2046,7 @@ int xl_set_sampling(xl_handle* h, const xl_sampling* params, uint32_t step0, voi
   }
   if (h->sampling != (params != nullptr)) {
     // the sampling kernel and the counter advance are baked into captured graphs; the parameters are not
-    for (auto& g : h->graphs)
-      if (g.exec) cudaGraphExecDestroy(g.exec);
-    h->graphs.clear();
+    clear_graphs(h);
     h->sampling = params != nullptr;
   }
   if (params) {
@@ -2186,8 +2071,7 @@ int xl_sample_actions(xl_handle* h, const float* logits, int B, unsigned flags, 
   const float bw = (c.tok_max_val - c.tok_min_val) / (float)c.action_channels;
   xl::launch_sample_tokens(logits, discrete ? h->num_actions : h->head_out, B, c.act_dim, h->num_actions,
                            c.discrete_actions, discrete ? 1 : 0, discrete ? 0.f : bw, discrete ? 0.f : c.tok_min_val,
-                           tokens, actions, nullptr, nullptr, 1, 0, h->counters + kCntUnit, h->counters + kCntUnitStep, 0,
-                           s);
+                           tokens, actions, nullptr, nullptr, 1, 0, h->counters + kCntUnit, h->counters + kCntUnitStep, s);
   h->launches += 2;
   XL_CUDA(cudaGetLastError());
   return XL_OK;
@@ -2233,25 +2117,10 @@ int xl_set_option(xl_handle* h, const char* name, int value) {
       return fail(XL_ERR_INVALID_ARG, "state_fuse must be 0 (separate finalize kernel), 1 (cluster, symmetric), "
                                       "2 (cluster, rank 0 finalizes) or 3 (unfused kernel under the cluster shape)");
     h->state_fuse = value;
-  } else if (!strcmp(name, "microbatches")) {
-    if (value < 0 || value > kMaxMicro) return fail(XL_ERR_INVALID_ARG, "microbatches must be in [0, %d]", kMaxMicro);
-#ifndef XL_DEBUG_OPTIONS
-    // The env micro-batch pipeline (round 1: measured slower, never the default) is EXPERIMENTAL: round 2 found that
-    // with >= 128 envs its concurrently running TMA state-stream and tcgen05 Linear kernels of different micro-batches
-    // give hidden states that are off by 1e-3..1e-2 from the second env step on (a race that neither pdl=0 nor eager
-    // launches remove; state_impl=0 or gemm_impl=1 do). Until that is understood the product library refuses it;
-    // -DXL_DEBUG_OPTIONS builds keep it for investigation (profiles/r02_chain_fusion.md, section 6).
-    if (value > 1)
-      return fail(XL_ERR_UNSUPPORTED, "microbatches > 1 is experimental and disabled in this build (known mismatch at "
-                                      ">= 128 envs); build with XL_DEBUG_OPTIONS=1 to enable it");
-#endif
-    h->microbatches = value;
   } else if (!strcmp(name, "prefill_cell")) {
     if (value < 0 || value > 2)
       return fail(XL_ERR_INVALID_ARG, "prefill_cell must be 0 (fp32 sequence cell), 1 (chunkwise mma.sync) or 2 (chunkwise tcgen05)");
     h->prefill_cell = (int)value;
-  } else if (!strcmp(name, "prefill_gemm_2cta")) {
-    h->prefill_gemm_2cta = value ? 1 : 0;
   } else if (!strcmp(name, "prefill_rows")) {
     if (value < 48 || value > 32768) return fail(XL_ERR_INVALID_ARG, "prefill_rows must be in [48, 32768]");
     h->prefill_rows = value;
@@ -2279,8 +2148,6 @@ int xl_set_option(xl_handle* h, const char* name, int value) {
     h->l2_prefetch_mb = value;
   } else if (!strcmp(name, "l2_prefetch_policy")) {
     h->l2_prefetch_policy = value ? 1 : 0;
-  } else if (!strcmp(name, "pipeline_order")) {
-    h->pipeline_order = value ? 1 : 0;
   } else if (!strcmp(name, "gemm_splitk")) {
     if (value < 0 || value > kSplitMax) return fail(XL_ERR_INVALID_ARG, "gemm_splitk must be in [0, %d]", kSplitMax);
     h->gemm_splitk = value;
@@ -2309,9 +2176,7 @@ int xl_set_option(xl_handle* h, const char* name, int value) {
   } else {
     return fail(XL_ERR_INVALID_ARG, "unknown option %s", name);
   }
-  for (auto& g : h->graphs)
-    if (g.exec) cudaGraphExecDestroy(g.exec);
-  h->graphs.clear();
+  clear_graphs(h);
   return XL_OK;
 }
 

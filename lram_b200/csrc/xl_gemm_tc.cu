@@ -1209,7 +1209,7 @@ cudaError_t launch_gemm_up_conv(const void* a_hi, const void* a_lo, const __nv_b
 // (bias and residual must be null; the consumer adds the planes).
 cudaError_t launch_gemm_tc(const void* a_hi, const void* a_lo, const __nv_bfloat16* W, const float* bias,
                            const float* residual, float* out, int M, int N, int K, int num_sms, int bn, int splits,
-                           long long split_stride, int low_smem, cudaStream_t s) {
+                           long long split_stride, cudaStream_t s) {
   if (!gemm_tc_supported(M, N, K)) return cudaErrorInvalidValue;
   if (splits < 1) splits = 1;
   if (splits > 1 && (bias || residual || (K / tc::BLOCK_K) % splits)) return cudaErrorInvalidValue;
@@ -1218,7 +1218,7 @@ cudaError_t launch_gemm_tc(const void* a_hi, const void* a_lo, const __nv_bfloat
     gemm_tc_plan(M, N, K, num_sms, 1, &bn, &sp);
   }
   const int two_sm = g_gemm_2cta < 0 ? (M >= 2048 ? 2 : 0) : (M >= 512 ? g_gemm_2cta : 0);
-  if (two_sm && splits == 1 && !low_smem && N >= 256 && (bn == 256 || bn == 128)) {
+  if (two_sm && splits == 1 && N >= 256 && (bn == 256 || bn == 128)) {
     CUtensorMap ma2, ml2, mw2;
     if (!tc::make_map(&ma2, a_hi, M, K, tc::BLOCK_M) || !tc::make_map(&ml2, a_lo, M, K, tc::BLOCK_M) ||
         !tc::make_map(&mw2, W, N, K, 128))
@@ -1247,15 +1247,15 @@ cudaError_t launch_gemm_tc(const void* a_hi, const void* a_lo, const __nv_bfloat
     if (persistent) return cudaLaunchKernelEx(&cfg, tc::two::gemm_tc2p_kernel, ma2, ml2, mw2, bias, residual, out, M, N, K);
     return cudaLaunchKernelEx(&cfg, tc::two::gemm_tc2_kernel, ma2, ml2, mw2, bias, residual, out, M, N, K);
   }
-  if (bn == 256 && (low_smem || N % 256 != 0)) bn = 128;
+  if (bn == 256 && N % 256 != 0) bn = 128;
   // 64-row MMA tiles (option "gemm_bm" = 64): half the A bytes per k-block and a ring twice as deep (9 stages), no
   // empty quarter tile at M = 192. Bit-identical results; measured 1.2 % SLOWER on the 48M x 64 step (3 row tiles read
   // W three times: 42 MB instead of 38 MB of L2 -> SM traffic for proj_up, and these GEMMs sit at the aggregate L2
   // read rate), equal elsewhere (profiles/r02_chain_fusion.md) -> not the default.
-  const bool bm64 = g_gemm_bm == 64 && !low_smem && bn == 64 && M > 16;
+  const bool bm64 = g_gemm_bm == 64 && bn == 64 && M > 16;
   // A-tile multicast across a cluster of 2 or 4 column-tile CTAs (option "gemm_cluster"; 128-row, 64-wide tiles only)
   const int n_tiles = (N + bn - 1) / bn;
-  int cx = (!bm64 && !low_smem && (bn == 64 || bn == 128) && N % bn == 0) ? g_gemm_cluster : 1;
+  int cx = (!bm64 && (bn == 64 || bn == 128) && N % bn == 0) ? g_gemm_cluster : 1;
   while (cx > 1 && n_tiles % cx) cx >>= 1;
   CUtensorMap ma, ml, mw;
   const int box_m = bm64 ? 64 : tc::BLOCK_M / (cx > 1 ? cx : 1);
@@ -1267,14 +1267,6 @@ cudaError_t launch_gemm_tc(const void* a_hi, const void* a_lo, const __nv_bfloat
   if (cx == 4 && bn == 64) return tc::launch<64, 4, tc::BLOCK_M, 4>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);
   if (cx == 2) return tc::launch<128, 4, tc::BLOCK_M, 2>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);
   if (cx == 4) return tc::launch<128, 4, tc::BLOCK_M, 4>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);
-  if (low_smem) {
-    // shallow rings (<= 110 KB): the CTA must fit beside a resident state-stream CTA of another micro-batch
-    switch (bn) {
-      case 128: return tc::launch<128, 2>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);
-      case 64: return tc::launch<64, 2>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);
-      default: return tc::launch<32, 3>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);
-    }
-  }
   switch (bn) {
     // 128 x 256 tiles (GEMM-sized M, e.g. the context prefill): 2/3 of the operand bytes per flop of a 128 x 128 tile
     case 256: return tc::launch<256, 3>(ma, ml, mw, bias, residual, out, M, N, K, splits, split_stride, s);

@@ -78,15 +78,14 @@ void launch_set_u32(unsigned* p, unsigned v, cudaStream_t s);
 // ---- xl_sample.cu --------------------------------------------------------------------------------
 // Stochastic action selection (xl_set_sampling; contract in include/xlstm_b200.h): drop-in for launch_argmax_tokens
 // with the same layouts. prm points at a device copy of the parameters; the step drawn for is *step_counter - 1;
-// env b's global id is prm->env_id_base + (env_offset + b) * prm->env_id_stride. num_actions <= kSampleMaxActions,
+// env b's global id is prm->env_id_base + b * prm->env_id_stride. num_actions <= kSampleMaxActions,
 // act_dim <= kSampleMaxRows.
 constexpr int kSampleMaxActions = 512;
 constexpr int kSampleMaxRows = 8;
 void launch_sample_tokens(const float* logits, int64_t row_pitch, int B, int act_dim, int num_actions,
                           int discrete_actions, int discrete, float bin_width, float min_val, int32_t* tokens,
                           float* actions, int32_t* ring, const unsigned* ring_counter, int ring_slots,
-                          int64_t ring_slot_stride, const void* prm, const unsigned* step_counter, int env_offset,
-                          cudaStream_t s);
+                          int64_t ring_slot_stride, const void* prm, const unsigned* step_counter, cudaStream_t s);
 // stream-ordered write of the parameters (an xl_sampling) to dst and of `counter_value` to *counter
 void launch_set_sampling(void* dst, const void* params, unsigned* counter, unsigned counter_value, cudaStream_t s);
 
@@ -184,7 +183,6 @@ struct StateStepParams {
   int impl;                 // 2 = persistent TMA ring (default), 1 = one-shot TMA ring, 0 = register-batched loads
   int stages;               // impl 2: ring depth (0 = default)
   int ctas_per_sm;          // impl 2: persistent CTAs per SM (0 = 1)
-  int meta_slots;           // impl 2: depth of the segment-metadata ring (0 = 3)
   // impl 2 stream-K partition (filled by the launchers): grid G, tiles per CTA q (+1 for the first r CTAs),
   // partial slots per item. sk_grid == 0 -> rows_split layout of impl 0/1.
   int sk_grid, sk_q, sk_r, sk_smax;
@@ -337,7 +335,7 @@ void launch_split_bf16(const float* in, int64_t in_stride, void* hi, void* lo, i
 // out + z*split_stride (bias/residual must be null); the consumer kernels add the planes in order.
 cudaError_t launch_gemm_tc(const void* a_hi, const void* a_lo, const __nv_bfloat16* W, const float* bias,
                            const float* residual, float* out, int M, int N, int K, int num_sms, int bn, int splits,
-                           long long split_stride, int low_smem, cudaStream_t s);
+                           long long split_stride, cudaStream_t s);
 // cost model: tile width and split-K factor (<= max_splits, dividing K/64)
 void gemm_tc_plan(int M, int N, int K, int num_sms, int max_splits, int* bn_out, int* splits_out);
 

@@ -79,7 +79,7 @@ __global__ void __launch_bounds__(32 * kSampleMaxRows) sample_tokens_kernel(
     const float* __restrict__ logits, int64_t row_pitch, int act_dim, int num_actions, int discrete_actions,
     int discrete, float bin_width, float min_val, int32_t* __restrict__ tokens, float* __restrict__ actions,
     int32_t* __restrict__ ring, const unsigned* __restrict__ ring_counter, int ring_slots, int64_t ring_slot_stride,
-    const xl_sampling* __restrict__ prm, const unsigned* __restrict__ step_counter, int env_offset) {
+    const xl_sampling* __restrict__ prm, const unsigned* __restrict__ step_counter) {
   __shared__ double s_pct[kSampleMaxRows];
   __shared__ float s_max[kSampleMaxRows];
   __shared__ int s_nan[kSampleMaxRows];
@@ -186,8 +186,7 @@ __global__ void __launch_bounds__(32 * kSampleMaxRows) sample_tokens_kernel(
       carry += __shfl_sync(0xffffffffu, s, 31);
     }
     const double Z = carry;
-    uint32_t ctr[4] = {*step_counter - 1u, (uint32_t)(p.env_id_base + (env_offset + b) * p.env_id_stride),
-                       (uint32_t)j, 0u};
+    uint32_t ctr[4] = {*step_counter - 1u, (uint32_t)(p.env_id_base + b * p.env_id_stride), (uint32_t)j, 0u};
     philox4x32_10(ctr, (uint32_t)p.seed, (uint32_t)(p.seed >> 32));
     const double u = (double)((uint64_t)(ctr[0] >> 5) * 67108864ull + (ctr[1] >> 6)) * 0x1p-53;
     const double target = u * Z;
@@ -224,12 +223,11 @@ __global__ void set_sampling_kernel(xl_sampling* dst, xl_sampling p, unsigned* c
 void launch_sample_tokens(const float* logits, int64_t row_pitch, int B, int act_dim, int num_actions,
                           int discrete_actions, int discrete, float bin_width, float min_val, int32_t* tokens,
                           float* actions, int32_t* ring, const unsigned* ring_counter, int ring_slots,
-                          int64_t ring_slot_stride, const void* prm, const unsigned* step_counter, int env_offset,
-                          cudaStream_t s) {
+                          int64_t ring_slot_stride, const void* prm, const unsigned* step_counter, cudaStream_t s) {
   const int rows = discrete ? 1 : act_dim;
   launch_k(sample_tokens_kernel, dim3(B), dim3(32 * rows), 0, s, logits, row_pitch, act_dim, num_actions,
            discrete_actions, discrete, bin_width, min_val, tokens, actions, ring, ring_counter, ring_slots,
-           ring_slot_stride, (const xl_sampling*)prm, step_counter, env_offset);
+           ring_slot_stride, (const xl_sampling*)prm, step_counter);
 }
 
 void launch_set_sampling(void* dst, const void* params, unsigned* counter, unsigned counter_value, cudaStream_t s) {

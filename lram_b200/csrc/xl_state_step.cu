@@ -848,9 +848,9 @@ static cudaError_t launch(const StateStepParams& p, cudaStream_t s) {
 //                       the gate recurrence of its (env, head) into a small ring, ahead of the consumers
 //   warps 0..7        : consumers — 128-bit shared loads, T x (2 FMA + 1 FMA) per element in registers,
 //                       128-bit streaming stores back to C, one cross-warp reduction of q^T C per segment
-// A 1-CTA/SM launch leaves shared memory and ~1700 thread slots per SM for the latency-bound kernels of OTHER
-// env micro-batches (LayerNorm, projections, conv/qkv, finalize) that the step pipeline (xl_api.cu) runs
-// concurrently on side streams.
+// A 1-CTA/SM launch leaves shared memory and ~1700 thread slots per SM for the kernels that run beside it: the L2
+// warm-up of the next block's C on the step's side stream, and the next kernel of the chain once programmatic
+// dependent launch lets it start.
 // ------------------------------------------------------------------------------------------------
 namespace pers {
 
@@ -865,6 +865,7 @@ constexpr int kStageRows = 32;
 constexpr int kW = 128;                       // column slab
 constexpr int kMaxStages = 8;
 constexpr int kMaxMetaSlots = 4;
+constexpr int kMetaSlots = 3;                 // depth of the segment-metadata ring the launcher uses
 constexpr int kConsumerWarps = kThreads / 32;
 constexpr int kBlock = kThreads + 64;         // + C-tile producer warp + metadata producer warp
 constexpr int kStageFloats = kStageRows * kW;
@@ -1112,12 +1113,11 @@ static cudaError_t launch(const StateStepParams& p, cudaStream_t s) {
   int stages = p.stages > 0 ? p.stages : 6;
   if (stages > kMaxStages) stages = kMaxStages;
   if (stages < 2) stages = 2;
-  const int meta_slots = p.meta_slots >= 2 && p.meta_slots <= kMaxMetaSlots ? p.meta_slots : 3;
-  const size_t smem = smem_bytes(T, p.DH, stages, meta_slots);
+  const size_t smem = smem_bytes(T, p.DH, stages, kMetaSlots);
   if (cudaError_t e = ensure_dyn_smem<&mlstm_state_stream_persistent_kernel<T, kStream>>(smem); e != cudaSuccess)
     return e;
   return launch_k(mlstm_state_stream_persistent_kernel<T, kStream>, dim3((unsigned)p.sk_grid), dim3(kBlock), smem,
-                  s, map, p, stages, meta_slots);
+                  s, map, p, stages, kMetaSlots);
 }
 
 }  // namespace pers

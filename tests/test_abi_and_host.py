@@ -201,16 +201,34 @@ def test_bench_dump_outputs_equal_an_independent_run(tmp_path):
     eng.close()
 
 
-def test_every_option_of_the_library_is_documented_in_the_header():
-    """xl_set_option names accepted by lram_b200/csrc/xl_api.cu must all be described in include/xlstm_b200.h (the header is
-    the boundary a maintainer reads)."""
+def _set_option_sources():
+    """(option names xl_set_option accepts in lram_b200/csrc/xl_api.cu, text of include/xlstm_b200.h)"""
     import os
     import re
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     api = open(os.path.join(root, "lram_b200", "csrc", "xl_api.cu")).read()
     hdr = open(os.path.join(root, "include", "xlstm_b200.h")).read()
     body = api[api.index("int xl_set_option"):]
-    names = sorted(set(re.findall(r'!strcmp\(name, "([a-z0-9_]+)"\)', body)))
+    return sorted(set(re.findall(r'!strcmp\(name, "([a-z0-9_]+)"\)', body))), hdr
+
+
+def test_every_option_of_the_library_is_documented_in_the_header():
+    """xl_set_option names accepted by lram_b200/csrc/xl_api.cu must all be described in include/xlstm_b200.h (the header is
+    the boundary a maintainer reads)."""
+    names, hdr = _set_option_sources()
     assert len(names) > 30
     missing = [n for n in names if f'"{n}"' not in hdr]
     assert not missing, missing
+
+
+def test_every_option_documented_in_the_header_is_accepted_by_the_library():
+    """Every '"name": [default]' entry of the header's xl_set_option comment names an option xl_set_option accepts: a
+    removed option does not stay documented."""
+    import re
+    names, hdr = _set_option_sources()
+    decl = hdr.index("int xl_set_option(")
+    block = hdr[hdr.rindex("/*", 0, decl):decl]
+    documented = sorted(set(re.findall(r'"([a-z0-9_]+)":\s*\[', block)))
+    assert len(documented) > 20
+    unknown = [n for n in documented if n not in names]
+    assert not unknown, unknown

@@ -311,54 +311,6 @@ def test_fused_equals_per_token_and_graph_replay():
     eng.close()
 
 
-def _microbatches_enabled(eng):
-    """The env micro-batch pipeline is experimental (known mismatch at >= 128 envs, see xl_set_option): the product build
-    refuses it loudly; only XL_DEBUG_OPTIONS builds run the tests below."""
-    from lram_b200._lib import XLError
-    try:
-        eng.set_option("microbatches", 2)
-    except XLError as ex:
-        assert "experimental" in str(ex)
-        return False
-    eng.set_option("microbatches", 0)
-    return True
-
-
-@pytest.mark.parametrize("name,B", [("16M", 40), ("toy128", 7)])
-def test_microbatch_pipeline_equals_single_stream(name, B):
-    """The env micro-batch pipeline (side streams, state-stream kernels taking turns) computes the same step as
-    the single-stream path: same tokens, hidden states within rounding of the partial-sum order; graph == eager."""
-    cfg, sd, eng = _engine(name, B)
-    if not _microbatches_enabled(eng):
-        eng.close()
-        pytest.skip("microbatches > 1 refused by the product build (experimental option)")
-    states, rtg, _ = make_stream(cfg, range(B), 5, domains="mixed")
-    res = {}
-    for tag, mb, order, flags in (("mb1", 1, 1, 0), ("mb4", 4, 1, 0), ("mb3_free", 3, 0, 0),
-                                  ("mb4_graph", 4, 1, L.XL_FLAG_GRAPH)):
-        eng.set_option("microbatches", mb)
-        eng.set_option("pipeline_order", order)
-        cache = eng.new_state(B)
-        s_dev = torch.empty(B, cfg.state_dim, device="cuda")
-        r_dev = torch.empty(B, device="cuda")
-        out = None
-        toks, hids = [], []
-        for t in range(5):
-            s_dev.copy_(torch.from_numpy(states[t]))
-            r_dev.copy_(torch.from_numpy(rtg[t]))
-            out = eng.policy_step(cache, s_dev, r_dev, flags=flags, want_hidden=True, want_logits=True, out=out)
-            torch.cuda.synchronize()
-            toks.append(out["action_tokens"].cpu().clone())
-            hids.append(out["last_hidden_state"].cpu().clone())
-        res[tag] = (torch.stack(toks), torch.stack(hids), cache.view(cfg.num_blocks - 1, L.XL_STATE_C).cpu().clone())
-    for tag in ("mb4", "mb3_free", "mb4_graph"):
-        assert torch.equal(res[tag][0], res["mb1"][0]), tag
-        assert _rel(res[tag][1], res["mb1"][1]) < 1e-4, tag
-        assert _rel(res[tag][2], res["mb1"][2]) < 1e-4, tag
-    assert torch.equal(res["mb4_graph"][1], res["mb4"][1])        # same kernels, same partition: bit identical
-    eng.close()
-
-
 # ------------------------------------------------------------------------------------------------------------
 # context prefill (SURVEY §8 a11 / BASELINE configs[3])
 # ------------------------------------------------------------------------------------------------------------
@@ -717,9 +669,8 @@ def test_slstm_policy_step_tokens_bit_exact(name, B, steps):
     eng.close()
 
 
-def test_slstm_prefill_reset_and_microbatches():
-    """sLSTM stacks through the other entry points: context prefill == stepping, per-env reset == fresh state,
-    env micro-batches == single stream."""
+def test_slstm_prefill_and_reset():
+    """sLSTM stacks through the other entry points: context prefill == stepping, per-env reset == fresh state."""
     from lram_b200.decision_xlstm import FusedXLSTMEncoder
     from oracle import xlstm_oracle as O
     cfg, sd, eng = _engine("toy128-ms", 4)
@@ -747,17 +698,6 @@ def test_slstm_prefill_reset_and_microbatches():
     of = eng.policy_step(eng.new_state(B), dev(states[2]), dev(rtg[2]), want_hidden=True)
     torch.cuda.synchronize()
     assert torch.equal(o1["last_hidden_state"].cpu()[[0, 3]], of["last_hidden_state"].cpu()[[0, 3]])
-    # micro-batches (experimental option: only debug builds accept it)
-    ca, cb = eng.new_state(B), eng.new_state(B)
-    for t in range(3 if _microbatches_enabled(eng) else 0):
-        eng.set_option("microbatches", 1)
-        a = eng.policy_step(ca, dev(states[t]), dev(rtg[t]), want_hidden=True)
-        eng.set_option("microbatches", 2)
-        b = eng.policy_step(cb, dev(states[t]), dev(rtg[t]), want_hidden=True)
-        torch.cuda.synchronize()
-        assert torch.equal(a["action_tokens"].cpu(), b["action_tokens"].cpu())
-        assert _rel(b["last_hidden_state"].cpu(), a["last_hidden_state"].cpu()) < 1e-5
-    eng.set_option("microbatches", 0)
     eng.close()
 
 

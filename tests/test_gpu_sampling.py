@@ -329,21 +329,6 @@ def test_policy_step_samples_its_own_logits(name, B, discrete):
 
 
 @gpu
-def test_microbatched_step_samples_the_same_tokens():
-    cfg, eng = _engine("16M", 40)
-    from test_gpu_parity import _microbatches_enabled
-    if not _microbatches_enabled(eng):
-        eng.close()
-        pytest.skip("env micro-batches are refused by this build")
-    one = _run_steps(eng, cfg, 40, 3, 0, armed=KW)
-    eng.set_option("microbatches", 2)
-    two = _run_steps(eng, cfg, 40, 3, 0, armed=KW)
-    for a, b in zip(one, two):
-        assert torch.equal(a["action_tokens"], b["action_tokens"])
-    eng.close()
-
-
-@gpu
 def test_sharded_draws_equal_single_gpu_draws():
     cfg, eng = _engine("toy128", 16)
     lg = torch.randn(16, cfg.head_out, generator=torch.Generator().manual_seed(4)).mul(3).cuda()

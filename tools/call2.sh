@@ -1,10 +1,5 @@
-# data collection: launch lists of the big configs, prefill launch list + ncu full of the mma cell, micro-batch re-test
+# data collection: launch lists of the big configs, prefill launch list + ncu full of the mma cell
 mkdir -p gpurun_out
-B="python bench.py --steps 100 --warmup 5 --no-cpu-baseline --profile-steps 0"
-for o in "microbatches=1" "microbatches=2" "microbatches=2 --opt state_rows_split=2" "microbatches=2 --opt state_rows_split=3" "microbatches=3 --opt state_rows_split=3"; do
-  echo "== $o"; timeout 120 $B --opt $o 2>/dev/null | python -c "import json,sys; d=json.loads(sys.stdin.read()); print(round(d['value']), round(d['e2e']['value']), d['ms_per_step'])"
-done > gpurun_out/ab_microbatch.txt 2>&1
-cat gpurun_out/ab_microbatch.txt
 timeout 200 ncu --metrics gpu__time_duration.sum --clock-control none -c 500 --csv --log-file gpurun_out/launches_206M_B128.csv python bench.py --model 206M --envs 128 --domains mixed --steps 2 --warmup 1 --no-cpu-baseline --profile-steps 0 > gpurun_out/ncu_206.log 2>&1
 timeout 200 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/launches_110M_B256.csv python bench.py --model 110M --envs 256 --discrete --steps 2 --warmup 1 --no-cpu-baseline --profile-steps 0 > gpurun_out/ncu_110.log 2>&1
 timeout 200 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/launches_prefill_206M_B1.csv python tools/bench_prefill.py --model 206M --envs 1 --tokens 6000 --rollout 5 --check 0 --reps 1 > gpurun_out/ncu_pf.log 2>&1

@@ -1,5 +1,5 @@
 """Times the graph-replayed policy step under xl_set_option combinations WITHOUT checking equality (use tools/ab_options.py
-for that): for experimental options whose results are under investigation.   python tools/time_options.py 206M:128 "microbatches=2" ..."""
+for that): for experimental options whose results are under investigation.   python tools/time_options.py 206M:128 "state_fuse=2" ..."""
 import json, os, sys
 import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
